@@ -1,7 +1,10 @@
 #!/usr/bin/env python
 """bench.py - GRAPE cost+gradient evaluations per second on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload NAME] [--dump-outputs DIR]
+
+`--dump-outputs DIR` writes what the last timed step returned to its caller as DIR/<name>.npy (see `dump_outputs`), so
+that two builds can be compared output for output: every input is generated from fixed seeds.
 
 A "step" is one cost+gradient evaluation of the hot path (Magnus assembly -> batched Pade-13 expm -> state /
 costate sweeps -> cost reductions -> gradient) on one batch of synthetic random controls.  Default workload =
@@ -168,6 +171,29 @@ def ncu_traffic(workload, kernel):
         return None
 
 
+DUMP_LIMIT_BYTES = 60 * 10 ** 6      # array data; with .npy headers and index files the dump stays below 64 MB
+
+
+def dump_outputs(directory, arrays):
+    """Write each array as `directory/<name>.npy`: real arrays as float64, complex ones as float64 with a trailing
+    (real, imaginary) axis.  When the arrays together exceed DUMP_LIMIT_BYTES, each keeps a fixed, seeded sample of its
+    leading-axis entries in proportion to its size, and the sampled indices go to `<name>_index.npy`."""
+    os.makedirs(directory, exist_ok=True)
+    out = {}
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        out[name] = np.stack([a.real, a.imag], axis=-1) if np.iscomplexobj(a) else a.astype(np.float64)
+    total = sum(a.nbytes for a in out.values())
+    for name, a in out.items():
+        if total > DUMP_LIMIT_BYTES and a.ndim > 0 and a.shape[0] > 1:
+            share = a.nbytes * DUMP_LIMIT_BYTES // total
+            keep = max(1, share // (a.nbytes // a.shape[0] + 8))
+            idx = np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))
+            np.save(os.path.join(directory, name + "_index.npy"), idx.astype(np.float64))
+            a = a[idx]
+        np.save(os.path.join(directory, name + ".npy"), np.ascontiguousarray(a))
+
+
 def make_problem(name):
     w = WORKLOADS[name]
     n, slices, K, S, order, cc, F = w[:7]
@@ -313,6 +339,8 @@ def run_b200(args, name):
     torch.cuda.synchronize()
     e2e_s = time.perf_counter() - t0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"cost": err, "grads": grads, "final_states": finals})
     if world > 1:
         t = torch.tensor([total_ms, e2e_s], dtype=torch.float64, device="cuda")
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -539,6 +567,8 @@ def run_lindblad(args, name):
         err, grads, finals = plan.cost_and_grad(q["controls"])
     sec = (time.perf_counter() - t0) / args.steps
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"cost": err, "grads": grads, "final_densities": finals})
     st = plan.stats()
     torch.set_num_threads(1)
     ocosts = [orc.TargetDensityInfidelity(q["targ"])]
@@ -653,6 +683,8 @@ def run_expm(args, name):
         got = expm(a)
     e2e_s = (time.perf_counter() - t0) / args.steps
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"expm": got})
     rate = batch / (ms * 1e-3)
     gbs = 32.0 * n * n * rate / 1e9
     tfl = fl * rate / 1e12
@@ -701,7 +733,14 @@ def main():
                                                                "100 scaled linearly above)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--check", action="store_true", help="kept for compatibility: every N > 1 line now carries its parity block")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (cost, gradient, final states; a seeded sample of the "
+                         "batched expm) to DIR/<name>.npy as float64, at most 64 MB")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the outputs of the CUDA path (--impl b200)")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.workload in EXPM_WORKLOADS:
         run_expm(args, args.workload)
