@@ -184,8 +184,23 @@ int qocb_expm_batched_bench(int32_t n, int64_t batch, double norm_scale, int32_t
 
 /* ---- Lindblad path: _evaluate_lindblad_discrete (qoc/core/lindbladdiscrete.py:357-441) and its jacobian (:322) -------
    Densities are [D][n][n] complex128, interleaved (NumPy C order).  H(x) = H0 + sum_r x_r A_r as above; the dissipator is
-   sum_l gamma_l (L_l rho L_l^dag - 1/2 {L_l^dag L_l, rho}) with time-independent (gamma_l, L_l).  Each of the N-1
-   intervals is a fresh adaptive Dormand-Prince 5(4) integration (qoc/core/mathmethods.py:352-480).
+   sum_l gamma_l (L_l rho L_l^dag - 1/2 {L_l^dag L_l, rho}).  Each of the N-1 intervals is a fresh adaptive Dormand-Prince
+   5(4) integration (qoc/core/mathmethods.py:352-480).
+
+   TIME DEPENDENCE.  The stage times of the adaptive integration depend on the data, so a time-dependent `hamiltonian` or
+   `lindblad_data` is given to the device as piecewise Chebyshev series of scalar functions of t, evaluated in the kernels
+   at every stage time:
+     - channel_count = KC > 0:  H(x, t) = H0 + sum_c (offset_c(t) + sum_r gain_cr(t) x_r) A_c, and a_ops of
+       qocb_lindblad_set_operators holds the KC channels A_c instead of KR control operators;
+     - time_dependent_rates = 1:  L_l(t) = f_l(t) B_l with fixed B_l (lops holds B_l, gammas is unused) and the effective
+       rate r_l(t) = gamma_l(t) |f_l(t)|^2.
+   The series table (qocb_lindblad_set_time_series, required with either) holds NS = KC (1 + KR) + (rates ? L : 0)
+   functions per row in the order [offset_c | gain_cr (c-major) | r_l], on `segments` uniform segments of width w that cover
+   [0, segments * w].  Stage times beyond the table are never extrapolated: the forward pass records the largest stage time
+   it needed (qocb_lindblad_max_stage_time), skips the reverse pass and the evaluation returns -5; the caller extends the
+   table and evaluates again (the initial-step probe t0 + h0 and the overshooting last step of an interval can reach far
+   beyond the evolution time).  The gradient maps the channel cotangents back, xbar_r = sum_c gain_cr(t) cbar_c, before
+   the interpolation weights; offsets and rates receive none.  With KC = 0 and time_dependent_rates = 0 nothing changes.
 
    CONTRACT OF THE LINDBLAD RESULTS (tolerances are asserted in tests/test_gpu_lindblad.py):
      - cost and final densities: the reference's adaptive integration at atol = 1e-12, rtol = 0.  A rounding-level change of
@@ -211,7 +226,8 @@ typedef struct {
     int32_t have_hamiltonian;    /* 0: hamiltonian = None (lindbladdiscrete.py:480-484) */
     int32_t device;
     int32_t max_rk_steps;        /* capacity of the accepted-step tape of one evaluation; 0 = automatic */
-    int32_t reserved0, reserved1;
+    int32_t channel_count;       /* KC in [0, 16]: time-dependent hamiltonian channels; 0 = time-independent H0 + x.A */
+    int32_t time_dependent_rates;/* 0 or 1 (needs lindblad_count >= 1) */
     double evolution_time;
 } qocb_lindblad_problem;
 
@@ -224,6 +240,12 @@ const char *qocb_lindblad_last_error(const qocb_lplan *plan);
 /* h0: [n][n] (NULL without hamiltonian); a_ops: [KR][n][n]; gammas: [L]; lops: [L][n][n] */
 int qocb_lindblad_set_operators(qocb_lplan *plan, const double *h0, const double *a_ops, const double *gammas,
                                 const double *lops);
+/* series: [segments][degree+1][NS] Chebyshev coefficients per segment [s w, (s+1) w] (constant term not halved);
+   degree <= 64; may be called again to replace the table */
+int qocb_lindblad_set_time_series(qocb_lplan *plan, int32_t segments, int32_t degree, double segment_width,
+                                  const double *series);
+/* largest stage time of the last forward pass (plans with a series); an evaluation returns -5 when it lies beyond the table */
+int qocb_lindblad_max_stage_time(qocb_lplan *plan, double *t);
 int qocb_lindblad_set_densities(qocb_lplan *plan, const double *rho0);
 /* mats: [D][fmax][n][n]; counts: [D] or NULL; weight = cost_multiplier / normalisation; step_cost as above */
 int qocb_lindblad_add_cost(qocb_lplan *plan, int32_t kind, int32_t step_cost, double weight, const double *mats,

@@ -29,7 +29,8 @@ EXPORTS = [
     "qocb_shard_pack_result", "qocb_state_shard_coherent_doubles", "qocb_state_shard_forward", "qocb_state_shard_finish",
     "qocb_lindblad_create", "qocb_lindblad_destroy", "qocb_lindblad_last_error",
     "qocb_lindblad_set_operators", "qocb_lindblad_set_densities", "qocb_lindblad_add_cost", "qocb_lindblad_cost",
-    "qocb_lindblad_cost_and_grad", "qocb_lindblad_stats", "qocb_lindblad_get_densities",
+    "qocb_lindblad_cost_and_grad", "qocb_lindblad_stats", "qocb_lindblad_get_densities", "qocb_lindblad_set_time_series",
+    "qocb_lindblad_max_stage_time",
 ]
 
 
@@ -48,7 +49,7 @@ class LindbladProblem(C.Structure):
     _fields_ = [("hilbert_size", C.c_int32), ("density_count", C.c_int32), ("control_count", C.c_int32),
                 ("control_eval_count", C.c_int32), ("system_eval_count", C.c_int32), ("cost_eval_step", C.c_int32),
                 ("lindblad_count", C.c_int32), ("have_hamiltonian", C.c_int32), ("device", C.c_int32),
-                ("max_rk_steps", C.c_int32), ("reserved0", C.c_int32), ("reserved1", C.c_int32),
+                ("max_rk_steps", C.c_int32), ("channel_count", C.c_int32), ("time_dependent_rates", C.c_int32),
                 ("evolution_time", C.c_double)]
 
 
@@ -146,6 +147,8 @@ def load():
     lib.qocb_lindblad_cost_and_grad.argtypes = [vp, vp, vp, vp, vp]
     lib.qocb_lindblad_stats.argtypes = [vp, vp]
     lib.qocb_lindblad_get_densities.argtypes = [vp, vp]
+    lib.qocb_lindblad_set_time_series.argtypes = [vp, i32, i32, dbl, vp]
+    lib.qocb_lindblad_max_stage_time.argtypes = [vp, vp]
     lib.qocb_flush_l2.argtypes = [vp]
     lib.qocb_shard_matrix_doubles.argtypes = [vp]
     lib.qocb_shard_vector_doubles.argtypes = [vp]

@@ -83,10 +83,36 @@ def _is_time_dependent(hamiltonian, zero, units, evolution_time, system_eval_cou
 class _RealBasis(object):
     """Streaming rank-revealing Gram-Schmidt of complex matrices over the REALS (the device coefficients are real):
     `add(m)` returns the coefficient vector of m on the basis so far, extending the basis when the residual exceeds
-    1e-12 * scale.  Earlier samples have zero weight on later basis vectors by construction."""
+    `tol` (1e-12) * scale.  Earlier samples have zero weight on later basis vectors by construction."""
 
-    def __init__(self, limit):
-        self.vecs, self.limit, self.scale = [], limit, 1.0
+    def __init__(self, limit, tol=1e-12):
+        self.vecs, self.limit, self.scale, self.tol = [], limit, 1.0, tol
+
+    def _too_many(self):
+        return NotImplementedError("the time dependence of this hamiltonian needs more than {} operator channels; not "
+                                   "supported by the CUDA path (no CPU fallback)".format(self.limit))
+
+    def seed(self, mats):
+        """starts the basis from a pool of samples by pivoted Gram-Schmidt (largest residual first), so that basis
+        directions do not come from small samples dominated by cancellation."""
+        R = np.array([np.concatenate([m.real.ravel(), m.imag.ravel()]) for m in mats])
+        if R.size == 0:
+            return
+        self.scale = max(self.scale, np.abs(R).max())
+        while True:
+            norms = np.linalg.norm(R, axis=1)
+            j = int(np.argmax(norms))
+            if norms[j] <= self.tol * self.scale * np.sqrt(R.shape[1]):
+                return
+            if len(self.vecs) >= self.limit:
+                raise self._too_many()
+            r = R[j].copy()
+            for _ in range(2):
+                for b in self.vecs:
+                    r -= np.dot(b, r) * b
+            b = r / np.linalg.norm(r)
+            self.vecs.append(b)
+            R -= np.outer(R @ b, b)
 
     def add(self, m):
         v = np.concatenate([m.real.ravel(), m.imag.ravel()])
@@ -99,11 +125,9 @@ class _RealBasis(object):
                 coef[k] += c
                 r -= c * b
         nr = np.linalg.norm(r)
-        if nr > 1e-12 * self.scale * np.sqrt(v.size):
+        if nr > self.tol * self.scale * np.sqrt(v.size):
             if len(self.vecs) >= self.limit:
-                raise NotImplementedError(
-                    "the time dependence of this hamiltonian needs more than {} operator channels; not supported by "
-                    "the CUDA path (no CPU fallback)".format(self.limit))
+                raise self._too_many()
             self.vecs.append(r / nr)
             coef[-1] = nr
             return coef
@@ -689,6 +713,244 @@ def extract_lindblad_structure(lindblad_data, evolution_time):
     return np.ascontiguousarray(g0), np.ascontiguousarray(o0)
 
 
+def _lindblad_is_time_dependent(lindblad_data, evolution_time):
+    """True when `lindblad_data(time)` returns different rates, operators or operator counts at the probe times."""
+    g0, o0 = lindblad_data(0.0)
+    g0, o0 = np.asarray(g0, dtype=np.float64), np.asarray(o0, dtype=np.complex128)
+    for t in _probe_times(evolution_time)[1:]:
+        g, o = lindblad_data(t)
+        g, o = np.asarray(g, dtype=np.float64), np.asarray(o, dtype=np.complex128)
+        if g.shape != g0.shape or o.shape != o0.shape:
+            return True
+        if not (np.allclose(g, g0, rtol=_PROBE_RTOL, atol=0) and np.allclose(o, o0, rtol=_PROBE_RTOL, atol=_PROBE_RTOL)):
+            return True
+    return False
+
+
+_SERIES_DEGREE = 24                   # highest Chebyshev degree per segment
+_SERIES_RTOL = 1e-13                  # fit check: |reconstructed - callable| <= 1e-13 * scale
+_SERIES_MAX_BYTES = 256 << 20         # table size beyond which the fit is refused
+
+
+def _cheb_coefficients(values):
+    """Chebyshev coefficients [.., deg+1, ..] (axis -2) of samples at the first-kind nodes x_k = cos(pi (k+1/2)/(deg+1)),
+    constant term not halved: f(x) = sum_j c_j T_j(x)."""
+    q = values.shape[-2]
+    k = np.arange(q) + 0.5
+    cosm = np.cos(np.pi * np.outer(np.arange(q), k) / q) * (2.0 / q)        # [j][k]
+    cosm[0] *= 0.5
+    return np.einsum("jk,...kc->...jc", cosm, values)
+
+
+def _cheb_eval(coef, u):
+    """Clenshaw for coef [deg+1][cols] at u in [-1, 1] (the same recurrence as the kernels)."""
+    b1 = np.zeros(coef.shape[1])
+    b2 = np.zeros(coef.shape[1])
+    for k in range(coef.shape[0] - 1, 0, -1):
+        b1, b2 = coef[k] + 2.0 * u * b1 - b2, b1
+    return coef[0] + u * b1 - b2
+
+
+class LindbladTimeStructure(object):
+    """Time dependence of a Lindblad problem as piecewise Chebyshev series (see `extract_lindblad_time_structure`).
+
+    g0 [n x n], channels [KC x n x n], rate_ops [L x n x n] (B_l; None without time-dependent dissipation) and
+    series [segments][degree+1][NS] with NS = KC (1 + KR) + L columns [offset_c | gain_cr (c-major) | r_l] on uniform
+    segments of width `width` that cover [0, t_max]."""
+
+    def __init__(self, g0, channels, KR, rate_ops, series, width, m):
+        self.g0, self.channels, self.KR, self.rate_ops = g0, channels, KR, rate_ops
+        self.series, self.width, self.m = np.ascontiguousarray(series), float(width), m
+        self.KC = channels.shape[0]
+        self.L = 0 if rate_ops is None else rate_ops.shape[0]
+        self.segments, self.degree = series.shape[0], series.shape[1] - 1
+        self.t_max = self.segments * self.width
+
+    def values(self, t):
+        """all NS series at time t (clamped to [0, t_max], as the kernels do)."""
+        t = min(max(float(t), 0.0), self.t_max)
+        s = min(int(t / self.width), self.segments - 1)
+        return _cheb_eval(self.series[s], 2.0 * (t - s * self.width) / self.width - 1.0)
+
+    def coefficients(self, x, t):
+        """channel coefficients offset_c(t) + sum_r gain_cr(t) x_r."""
+        v = self.values(t)
+        off, gain = v[:self.KC], v[self.KC:self.KC * (1 + self.KR)].reshape(self.KC, self.KR)
+        return off + (gain @ np.asarray(x, dtype=np.float64) if self.KR else 0.0)
+
+    def hamiltonian(self, x, t):
+        """the reconstructed H(x, t) = G0 + sum_c coef_c A_c, x = [Re u, Im u]."""
+        return self.g0 + np.tensordot(self.coefficients(x, t), self.channels, axes=(0, 0))
+
+    def rates(self, t):
+        return self.values(t)[self.KC * (1 + self.KR):]
+
+
+def _rate_directions(lindblad_data, times):
+    """fixed operator directions B_l (the largest sample of each operator, unit max-norm) of a time-dependent
+    `lindblad_data`; raises NotImplementedError when the operator count changes."""
+    best = None
+    for t in times:
+        g, o = lindblad_data(t)
+        g, o = np.asarray(g, dtype=np.float64), np.asarray(o, dtype=np.complex128)
+        if o.ndim != 3 or g.shape != (o.shape[0],):
+            raise ValueError("lindblad_data(time) must return (dissipators [L], operators [L x n x n])")
+        if best is None:
+            best = o.copy()
+        elif o.shape != best.shape:
+            raise NotImplementedError("lindblad_data(time) changes its operator count over time; not supported by the CUDA "
+                                      "Lindblad path (no CPU fallback)")
+        for l in range(o.shape[0]):
+            if np.abs(o[l]).max() > np.abs(best[l]).max():
+                best[l] = o[l]
+    for l in range(best.shape[0]):
+        s = np.abs(best[l]).max()
+        best[l] = best[l] / s if s > 0 else best[l]
+    return best
+
+
+def _rate_sample(lindblad_data, t, directions):
+    """effective rates r_l(t) = gamma_l(t) |f_l(t)|^2 with L_l(t) = f_l(t) B_l; a dissipator that leaves its direction
+    raises NotImplementedError."""
+    g, o = lindblad_data(t)
+    g, o = np.asarray(g, dtype=np.float64), np.asarray(o, dtype=np.complex128)
+    if o.shape != directions.shape:
+        raise NotImplementedError("lindblad_data(time) changes its operator count over time; not supported by the CUDA "
+                                  "Lindblad path (no CPU fallback)")
+    r = np.zeros(o.shape[0])
+    for l in range(o.shape[0]):
+        b = directions[l]
+        f = np.vdot(b, o[l]) / max(np.vdot(b, b).real, 1e-300)
+        if np.abs(o[l] - f * b).max() > _SERIES_RTOL * max(1.0, np.abs(o[l]).max()):
+            raise NotImplementedError("lindblad operator {} changes direction over time (only L_l(t) = f_l(t) B_l with a fixed "
+                                      "B_l is supported by the CUDA Lindblad path; no CPU fallback)".format(l))
+        r[l] = g[l] * abs(f) ** 2
+    return r
+
+
+def extract_lindblad_time_structure(hamiltonian, control_count, complex_controls, evolution_time, system_eval_count, t_max,
+                                    lindblad_data=None, seed=1234, min_m=1):
+    """Time dependence of a Lindblad problem for the adaptive-step kernels, which evaluate it at data-dependent stage times.
+
+    `hamiltonian(controls, time)` (time-dependent, affine in x = [Re u, Im u]; or None) becomes
+        H(x, t) = G0 + sum_c (offset_c(t) + sum_r gain_cr(t) x_r) A_c
+    over a shared real operator basis (`_RealBasis`, at most 16 channels), sampled as `extract_time_dependent_structure`
+    does (zero and unit controls); `lindblad_data(time)` (time-dependent; or None) with operators L_l(t) = f_l(t) B_l becomes
+    rates r_l(t) = gamma_l(t) |f_l(t)|^2.  Every scalar function is a Chebyshev series of degree <= 24 on uniform segments of
+    width dt/m (aligned to the system grid) covering [0, t_max], fitted from samples at each segment's Chebyshev nodes.
+
+    The fit is checked against the callables themselves at a random time in every segment, at the segment end points and at
+    the probe times, to 1e-13 x scale; m doubles until it passes.  When it stops converging, or the table would exceed
+    256 MB, NotImplementedError is raised: nothing is silently approximated.  Random controls check that the callable is
+    affine (NonlinearHamiltonian otherwise).  Returns a `LindbladTimeStructure`."""
+    T = float(evolution_time)
+    dt = T / (system_eval_count - 1)
+    rng = np.random.default_rng(seed)
+    zero, units = _unit_controls(control_count, complex_controls) if control_count else (None, [])
+    KR = len(units) if hamiltonian is not None else 0
+    g0 = None
+    if hamiltonian is not None:
+        g0 = np.array(hamiltonian(zero, 0.0), dtype=np.complex128)
+        if g0.ndim != 2 or g0.shape[0] != g0.shape[1]:
+            raise ValueError("hamiltonian(controls, time) must return a square matrix")
+    probe = [t for t in _probe_times(T) if t <= t_max]
+    directions = None
+    if lindblad_data is not None:
+        directions = _rate_directions(lindblad_data, probe + list(np.linspace(0.0, t_max, 33)))
+    L = 0 if directions is None else directions.shape[0]
+    deg = _SERIES_DEGREE
+    nodes = (np.cos(np.pi * (np.arange(deg + 1) + 0.5) / (deg + 1)) + 1.0) / 2.0          # on [0, 1] of a segment
+    m, last_err = max(1, int(min_m)), None
+    while True:
+        w = dt / m
+        segs = int(np.ceil(t_max / w - 1e-9))
+        if segs * (deg + 1) * (KR + 1 + L) * 8 > _SERIES_MAX_BYTES:           # at least one channel or one rate
+            raise NotImplementedError("the time dependence needs a Chebyshev table beyond 256 MB to reach 1e-13; not supported "
+                                      "by the CUDA Lindblad path (no CPU fallback)")
+        times = (np.arange(segs)[:, None] + nodes[None, :]) * w                              # [segs][deg+1]
+        basis = _RealBasis(_MAX_CHANNELS, tol=1e-14)
+        if hamiltonian is not None:
+            pool = []
+            for t in list(probe) + list(np.linspace(0.0, t_max, 17)):
+                d = np.asarray(hamiltonian(zero, t), dtype=np.complex128)
+                pool.append(d - g0)
+                pool += [np.asarray(hamiltonian(e, t), dtype=np.complex128) - d for e in units]
+            basis.seed(pool)
+        rows = []
+        for t in times.ravel():
+            row = []
+            if hamiltonian is not None:
+                d = np.asarray(hamiltonian(zero, t), dtype=np.complex128)
+                row.append(basis.add(d - g0))
+                for e in units:
+                    row.append(basis.add(np.asarray(hamiltonian(e, t), dtype=np.complex128) - d))
+            rows.append(row)
+        KC = len(basis.vecs)
+        samples = np.zeros((segs * (deg + 1), KC * (1 + KR) + L))
+        for k, row in enumerate(rows):
+            if row:
+                samples[k, :len(row[0])] = row[0]
+                for r in range(KR):
+                    samples[k, KC + np.arange(len(row[1 + r])) * KR + r] = row[1 + r]
+            if L:
+                samples[k, KC * (1 + KR):] = _rate_sample(lindblad_data, float(times.ravel()[k]), directions)
+        coef = _cheb_coefficients(samples.reshape(segs, deg + 1, -1))
+        # the lowest degree whose dropped tail is below rounding in every column and segment
+        amp = (np.abs(coef) / np.maximum(1.0, np.abs(samples).max(axis=0))).max(axis=(0, 2))     # [deg+1]
+        tail = np.r_[np.cumsum(amp[::-1])[::-1], 0.0]                                           # tail[j] = sum_{k >= j}
+        coef = coef[:, :int(np.argmax(tail[1:] <= 1e-15)) + 1, :]
+        if coef.nbytes > _SERIES_MAX_BYTES:
+            raise NotImplementedError("the time dependence needs a Chebyshev table beyond 256 MB to reach 1e-13; not supported "
+                                      "by the CUDA Lindblad path (no CPU fallback)")
+        channels = basis.matrices(g0.shape) if KC else np.zeros((0,) + (g0.shape if g0 is not None else (0, 0)))
+        st = LindbladTimeStructure(g0, channels, KR, directions, coef, w, m)
+        err = _series_error(st, hamiltonian, zero, units, lindblad_data, probe, rng)
+        if err <= _SERIES_RTOL:
+            break
+        if last_err is not None and m >= 16 and err > 0.25 * last_err:
+            raise NotImplementedError("the time dependence is not reproduced by piecewise Chebyshev series (fit error {:.1e} "
+                                      "relative at {} segments per system step, not converging): discontinuities inside a "
+                                      "segment are not supported by the CUDA Lindblad path (no CPU fallback)".format(err, m))
+        last_err, m = err, 2 * m
+    _check_affine(st, hamiltonian, control_count, complex_controls, zero, rng)
+    return st
+
+
+def _series_error(st, hamiltonian, zero, units, lindblad_data, probe, rng):
+    """largest relative deviation of the fitted series from the callables at off-node check times."""
+    times = list((np.arange(st.segments) + rng.uniform(0.0, 1.0, st.segments)) * st.width)
+    times += list(np.arange(st.segments + 1) * st.width) + list(probe)
+    err = 0.0
+    scale = 1.0 if hamiltonian is None else max(1.0, np.abs(st.g0).max(), np.abs(st.channels).max(initial=0.0))
+    for t in times:
+        t = min(float(t), st.t_max)
+        if hamiltonian is not None:
+            xs = [np.zeros(st.KR)] + [np.eye(st.KR)[r] for r in range(st.KR)]
+            for u, x in zip([zero] + units, xs):
+                got = np.asarray(hamiltonian(u, t), dtype=np.complex128)
+                err = max(err, np.abs(got - st.hamiltonian(x, t)).max() / max(scale, np.abs(got).max()))
+        if st.L:
+            want = _rate_sample(lindblad_data, t, st.rate_ops)
+            err = max(err, np.abs(want - st.rates(t)).max() / max(1.0, np.abs(want).max()))
+    return err
+
+
+def _check_affine(st, hamiltonian, control_count, complex_controls, zero, rng):
+    if hamiltonian is None or not st.KR:
+        return
+    scale = max(1.0, np.abs(st.g0).max(), np.abs(st.channels).max(initial=0.0))
+    for trial in range(4):
+        t = float(rng.uniform(0.0, st.t_max))
+        u = rng.standard_normal(control_count) * (1.0 + trial)
+        if complex_controls:
+            u = u + 1j * rng.standard_normal(control_count) * (1.0 + trial)
+        x = np.concatenate([u.real, u.imag]) if complex_controls else u
+        got = np.asarray(hamiltonian(u.astype(zero.dtype), t), dtype=np.complex128)
+        if not np.allclose(got, st.hamiltonian(x, t), rtol=0, atol=_PROBE_RTOL * scale * (1 + np.abs(x).sum())):
+            raise NonlinearHamiltonian("hamiltonian(controls, time) is not affine in (Re u, Im u); the CUDA Lindblad path "
+                                       "needs that form (no CPU fallback)")
+
+
 class LindbladPlan(object):
     """Device plan for `_evaluate_lindblad_discrete` and its jacobian (qoc/core/lindbladdiscrete.py:357-441, :322).
 
@@ -710,31 +972,41 @@ class LindbladPlan(object):
         self.have_h = hamiltonian is not None
         self.KR = self.K * (2 if self.complex_controls else 1) if self.have_h else 0
         self.costs = list(costs)
-        h0 = a_ops = None
-        if self.have_h:
+        self.T, self.dt = float(evolution_time), float(evolution_time) / (self.N - 1)
+        # time dependence (hamiltonian reading `time`, lindblad_data varying with time): Chebyshev series evaluated on the
+        # device at the stage times; a time-independent problem keeps the constant operators below and no series
+        td_h = td_l = False
+        if self.have_h and structure is None:
+            zero, units = _unit_controls(self.K, self.complex_controls) if self.K else (None, [])
+            td_h = _is_time_dependent(hamiltonian, zero, units, evolution_time)
+        if lindblad_data is not None:
+            td_l = _lindblad_is_time_dependent(lindblad_data, evolution_time)
+        h0 = a_ops = gammas = lops = None
+        if self.have_h and not td_h:
             if structure is None:
                 structure = extract_hamiltonian_structure(hamiltonian, self.K, self.complex_controls, evolution_time)
             h0, a_ops = structure
-            if h0.shape[0] != self.n:
-                raise ValueError("hamiltonian size {} does not match the densities' hilbert size {}".format(h0.shape[0], self.n))
-        gammas, lops = extract_lindblad_structure(lindblad_data, evolution_time)
-        self.L = 0 if gammas is None else gammas.shape[0]
-        pb = _lib.LindbladProblem(hilbert_size=self.n, density_count=self.D, control_count=self.KR,
-                                  control_eval_count=self.M if self.KR else 0, system_eval_count=self.N,
-                                  cost_eval_step=int(cost_eval_step), lindblad_count=self.L,
-                                  have_hamiltonian=int(self.have_h), device=int(device), max_rk_steps=int(max_rk_steps),
-                                  reserved0=0, reserved1=0, evolution_time=float(evolution_time))
-        handle = ctypes.c_void_p()
-        rc = self.lib.qocb_lindblad_create(ctypes.byref(pb), ctypes.byref(handle))
-        if rc != 0:
-            raise RuntimeError("qoc_b200 CUDA Lindblad path failed (rc={}): {}".format(
-                rc, self.lib.qocb_lindblad_last_error(None).decode()))
-        self.handle = handle
-        h0c = None if h0 is None else np.ascontiguousarray(h0, dtype=np.complex128)
-        aoc = None if a_ops is None or self.KR == 0 else np.ascontiguousarray(a_ops, dtype=np.complex128)
-        self._check(self.lib.qocb_lindblad_set_operators(handle, _lib.ptr(h0c), _lib.ptr(aoc), _lib.ptr(gammas), _lib.ptr(lops)))
-        self._check(self.lib.qocb_lindblad_set_densities(handle, _lib.ptr(rho0)))
+        if not td_l:
+            gammas, lops = extract_lindblad_structure(lindblad_data, evolution_time)
+        self._td = (hamiltonian if td_h else None, lindblad_data if td_l else None)
+        self.series = None
+        if td_h or td_l:
+            self.series = extract_lindblad_time_structure(self._td[0], self.K, self.complex_controls, evolution_time, self.N,
+                                                          self.T + self.dt, lindblad_data=self._td[1])
+            if td_h:
+                h0, a_ops = self.series.g0, self.series.channels
+            if td_l:
+                lops = self.series.rate_ops
+        if h0 is not None and h0.shape[0] != self.n:
+            raise ValueError("hamiltonian size {} does not match the densities' hilbert size {}".format(h0.shape[0], self.n))
+        self.L = 0 if lops is None else lops.shape[0]
+        self.range_extensions = 0
+        self._setup = dict(rho0=rho0, h0=h0, a_ops=a_ops, gammas=gammas, lops=lops, cost_eval_step=int(cost_eval_step),
+                           device=int(device), max_rk_steps=int(max_rk_steps))
+        self.handle = None
+        self._open()
         self.control_costs = []
+        self._terms = []
         from qoc_b200.models.cost import Cost
         for c in self.costs:
             terms = c.device_terms_density(self.D, self.n) if hasattr(c, "device_terms_density") else None
@@ -748,11 +1020,68 @@ class LindbladPlan(object):
                                               "`control_value_and_grad`.".format(c))
                 self.control_costs.append(c)
             for kind, step, weight, mats, counts in terms:
-                mats = np.ascontiguousarray(mats, dtype=np.complex128)
-                cnt = None if counts is None else np.ascontiguousarray(counts, dtype=np.int32)
-                self._check(self.lib.qocb_lindblad_add_cost(handle, kind, step, float(weight), _lib.ptr(mats),
-                                                            None if cnt is None else cnt.ctypes.data_as(ctypes.c_void_p),
-                                                            mats.shape[1]))
+                term = (kind, step, float(weight), np.ascontiguousarray(mats, dtype=np.complex128),
+                        None if counts is None else np.ascontiguousarray(counts, dtype=np.int32))
+                self._terms.append(term)
+                self._add_term(term)
+
+    def _open(self):
+        """creates the device plan and uploads operators, densities and (time-dependent problems) the series table."""
+        su, st = self._setup, self.series
+        KC = st.KC if st is not None and self._td[0] is not None else 0
+        tdr = int(st is not None and self._td[1] is not None)
+        pb = _lib.LindbladProblem(hilbert_size=self.n, density_count=self.D, control_count=self.KR,
+                                  control_eval_count=self.M if self.KR else 0, system_eval_count=self.N,
+                                  cost_eval_step=su["cost_eval_step"], lindblad_count=self.L,
+                                  have_hamiltonian=int(self.have_h), device=su["device"], max_rk_steps=su["max_rk_steps"],
+                                  channel_count=KC, time_dependent_rates=tdr, evolution_time=self.T)
+        handle = ctypes.c_void_p()
+        rc = self.lib.qocb_lindblad_create(ctypes.byref(pb), ctypes.byref(handle))
+        if rc != 0:
+            raise RuntimeError("qoc_b200 CUDA Lindblad path failed (rc={}): {}".format(
+                rc, self.lib.qocb_lindblad_last_error(None).decode()))
+        self.handle = handle
+        h0c = None if su["h0"] is None else np.ascontiguousarray(su["h0"], dtype=np.complex128)
+        a_ops = su["a_ops"]
+        aoc = None if a_ops is None or a_ops.shape[0] == 0 else np.ascontiguousarray(a_ops, dtype=np.complex128)
+        lops = None if su["lops"] is None else np.ascontiguousarray(su["lops"], dtype=np.complex128)
+        self._check(self.lib.qocb_lindblad_set_operators(handle, _lib.ptr(h0c), _lib.ptr(aoc), _lib.ptr(su["gammas"]),
+                                                         _lib.ptr(lops)))
+        self._check(self.lib.qocb_lindblad_set_densities(handle, _lib.ptr(su["rho0"])))
+        if st is not None:
+            self._check(self.lib.qocb_lindblad_set_time_series(handle, st.segments, st.degree, st.width, _lib.ptr(st.series)))
+
+    def _add_term(self, term):
+        kind, step, weight, mats, cnt = term
+        self._check(self.lib.qocb_lindblad_add_cost(self.handle, kind, step, weight, _lib.ptr(mats),
+                                                    None if cnt is None else cnt.ctypes.data_as(ctypes.c_void_p),
+                                                    mats.shape[1]))
+
+    _MAX_RANGE_EXTENSIONS = 4
+
+    def _evaluate(self, call):
+        """runs `call(handle)`; when a stage time left the series table (rc -5), refits the table to cover it with a margin
+        (same segment width, so the covered range keeps its values), rebuilds the plan and evaluates again."""
+        for _ in range(self._MAX_RANGE_EXTENSIONS + 1):
+            rc = call(self.handle)
+            if rc != -5 or self.series is None:
+                return self._check(rc)
+            tseen = np.zeros(1)
+            self._check(self.lib.qocb_lindblad_max_stage_time(self.handle, _lib.ptr(tseen)))
+            t_max = float(tseen[0]) + self.dt + 0.25 * max(0.0, float(tseen[0]) - self.T)
+            self.series = extract_lindblad_time_structure(self._td[0], self.K, self.complex_controls, self.T, self.N, t_max,
+                                                          lindblad_data=self._td[1], min_m=self.series.m)
+            if self._td[0] is not None:
+                self._setup.update(h0=self.series.g0, a_ops=self.series.channels)
+            if self._td[1] is not None:
+                self._setup.update(lops=self.series.rate_ops)
+            self.close()
+            self._open()
+            for term in self._terms:
+                self._add_term(term)
+            self.range_extensions += 1
+        raise RuntimeError("qoc_b200 CUDA Lindblad path: the Runge-Kutta stage times kept leaving the time series after {} "
+                           "extensions".format(self._MAX_RANGE_EXTENSIONS))
 
     def _check(self, rc):
         if rc != 0:
@@ -767,7 +1096,7 @@ class LindbladPlan(object):
         x = self._real_channels(controls) if controls is not None else None
         out = np.zeros(1)
         fd = np.empty((self.D, self.n, self.n), dtype=np.complex128)
-        self._check(self.lib.qocb_lindblad_cost(self.handle, _lib.ptr(x), _lib.ptr(out), _lib.ptr(fd)))
+        self._evaluate(lambda h: self.lib.qocb_lindblad_cost(h, _lib.ptr(x), _lib.ptr(out), _lib.ptr(fd)))
         extra, _ = self._control_costs(controls, False) if controls is not None else (0.0, None)
         return float(out[0]) + extra, fd
 
@@ -778,11 +1107,11 @@ class LindbladPlan(object):
         fd = np.empty((self.D, self.n, self.n), dtype=np.complex128)
         controls = np.asarray(controls)
         if self.KR == 0:                                   # hamiltonian = None: the state costs do not see the controls
-            self._check(self.lib.qocb_lindblad_cost(self.handle, None, _lib.ptr(out), _lib.ptr(fd)))
+            self._evaluate(lambda h: self.lib.qocb_lindblad_cost(h, None, _lib.ptr(out), _lib.ptr(fd)))
             grads = np.zeros(controls.shape, dtype=controls.dtype)
         else:
             g = np.zeros((self.M, self.KR))
-            self._check(self.lib.qocb_lindblad_cost_and_grad(self.handle, _lib.ptr(x), _lib.ptr(out), _lib.ptr(g), _lib.ptr(fd)))
+            self._evaluate(lambda h: self.lib.qocb_lindblad_cost_and_grad(h, _lib.ptr(x), _lib.ptr(out), _lib.ptr(g), _lib.ptr(fd)))
             grads = g[:, :self.K] + 1j * g[:, self.K:] if self.complex_controls else g
         extra, extra_grad = self._control_costs(controls, True)
         if extra_grad is not None:

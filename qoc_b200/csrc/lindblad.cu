@@ -69,6 +69,13 @@ struct LArgs {
     double2 *work;                              // global work arrays (used when the working set exceeds shared memory)
     int work_in_smem, ops_in_smem;
     double *grad;                               // [M][KR]
+    // time-dependent operators (0 series without them): piecewise Chebyshev series of the NS = KC*(1+KR) + L scalar
+    // functions [offset_c | gain_cr | rate_l] on `segs` uniform segments of width `seg_w` covering [0, segs * seg_w]
+    int KC, tdr, segs, deg, NS;
+    double seg_w;
+    const double *series;                       // [segs][deg+1][NS]
+    const double2 *Kops;                        // [L][n*n] 1/2 B_l^dag B_l (tdr)
+    double *tseen;                              // largest stage time of the forward pass
 };
 
 // block-wide sum, result in all threads
@@ -117,17 +124,41 @@ struct Ctx {
     double *red;            // reduction scratch
     double *coef;           // interpolated controls [KR], then slot for (i0, i1, w)
     int *loc;               // i0, i1
+    double *sv, *chan, *cbar;   // series values at t [NS], channel coefficients [KC], channel cotangents [KC] (series only)
+    double tseen = 0.;      // largest stage time evaluated (uniform over the CTA)
     // operators, rates, controls and control times: shared-memory copies when they fit (a.ops_in_smem), else global
-    const double2 *H0, *Aops, *Lops, *Khalf;
+    const double2 *H0, *Aops, *Lops, *Khalf, *Kops;
     const double *gam, *controls, *xs;
-    __device__ Ctx(const LArgs &a_) : a(a_), H0(a_.H0), Aops(a_.Aops), Lops(a_.Lops), Khalf(a_.Khalf), gam(a_.gam),
-                                      controls(a_.controls), xs(a_.xs) {}
+    __device__ Ctx(const LArgs &a_) : a(a_), H0(a_.H0), Aops(a_.Aops), Lops(a_.Lops), Khalf(a_.Khalf), Kops(a_.Kops),
+                                      gam(a_.gam), controls(a_.controls), xs(a_.xs) {}
 };
 
-// controls at time t (qoc/core/mathmethods.py:36-67 on control_eval_times) and the effective generators
-__device__ void set_time(Ctx &c, double t) {
+// the NS series at t by Clenshaw, one series per thread.  A time beyond the table is recorded in c.tseen and evaluated at
+// the table's end instead (never extrapolated); the host sees tseen, extends the table and runs the evaluation again.
+__device__ void eval_series(Ctx &c, double t) {
+    const LArgs &a = c.a;
+    c.tseen = fmax(c.tseen, t);
+    const double tc = fmin(fmax(t, 0.0), a.segs * a.seg_w);
+    const int s = min(max((int)(tc / a.seg_w), 0), a.segs - 1);
+    const double u = 2.0 * (tc - s * a.seg_w) / a.seg_w - 1.0, u2 = 2.0 * u;
+    const double *tab = a.series + (size_t)s * (a.deg + 1) * a.NS;
+    for (int j = threadIdx.x; j < a.NS; j += blockDim.x) {
+        double b1 = 0., b2 = 0.;
+        for (int k = a.deg; k >= 1; --k) {
+            const double b0 = tab[(size_t)k * a.NS + j] + u2 * b1 - b2;
+            b2 = b1; b1 = b0;
+        }
+        c.sv[j] = tab[j] + u * b1 - b2;
+    }
+    __syncthreads();
+}
+
+// controls at time t (qoc/core/mathmethods.py:36-67 on control_eval_times) and the effective generators.  TD: the plan has
+// time series (a.NS > 0); the kernels are instantiated for both, so that plans without series run the code they always ran
+template <bool TD> __device__ void set_time(Ctx &c, double t) {
     const LArgs &a = c.a;
     const int nn = a.n * a.n;
+    if constexpr (TD) eval_series(c, t);
     if (a.have_h && a.KR > 0) {
         if (threadIdx.x == 0) {
             int i0, i1;
@@ -144,14 +175,26 @@ __device__ void set_time(Ctx &c, double t) {
         }
         __syncthreads();
     }
+    if (TD && a.KC > 0) {                                  // coef_c = offset_c(t) + sum_r gain_cr(t) x_r(t)
+        for (int ch = threadIdx.x; ch < a.KC; ch += blockDim.x) {
+            double v = c.sv[ch];
+            for (int r = 0; r < a.KR; ++r) v += c.sv[a.KC + ch * a.KR + r] * c.coef[r];
+            c.chan[ch] = v;
+        }
+        __syncthreads();
+    }
+    const int nch = (TD && a.KC > 0) ? a.KC : a.KR;
+    const double *cf = (TD && a.KC > 0) ? c.chan : c.coef;
     for (int e = threadIdx.x; e < nn; e += blockDim.x) {
         double2 h = make_double2(0., 0.);
         if (a.have_h) {
             h = c.H0[e];
-            for (int r = 0; r < a.KR; ++r) { const double2 g = c.Aops[(size_t)r * nn + e]; h.x += c.coef[r] * g.x; h.y += c.coef[r] * g.y; }
+            for (int r = 0; r < nch; ++r) { const double2 g = c.Aops[(size_t)r * nn + e]; h.x += cf[r] * g.x; h.y += cf[r] * g.y; }
         }
         double2 k = make_double2(0., 0.);
-        if (a.L > 0) k = c.Khalf[e];
+        if (TD && a.tdr) {                                 // Khalf(t) = sum_l r_l(t) 1/2 B_l^dag B_l; c.gam points at r(t)
+            for (int l = 0; l < a.L; ++l) { const double2 g = c.Kops[(size_t)l * nn + e]; k.x += c.gam[l] * g.x; k.y += c.gam[l] * g.y; }
+        } else if (a.L > 0) k = c.Khalf[e];
         c.A1[e] = make_double2(h.y - k.x, -h.x - k.y);     // -i h - k
         c.A2[e] = make_double2(-h.y - k.x, h.x - k.y);     // +i h - k
     }
@@ -159,10 +202,10 @@ __device__ void set_time(Ctx &c, double t) {
 }
 
 // out = A1 rho + rho A2 + sum_l gamma_l L rho L^dag        (= get_lindbladian, mathmethods.py:187-204, regrouped)
-__device__ void rhs(Ctx &c, double t, const double2 *rho, double2 *out) {
+template <bool TD> __device__ void rhs(Ctx &c, double t, const double2 *rho, double2 *out) {
     const LArgs &a = c.a;
     const int nn = a.n * a.n;
-    set_time(c, t);
+    set_time<TD>(c, t);
     bmm<0, 0, false>(out, c.A1, 0, rho, nn, a.n, a.D, 1.0);
     bmm<0, 0, true>(out, rho, nn, c.A2, 0, a.n, a.D, 1.0);
     for (int l = 0; l < a.L; ++l) {
@@ -172,10 +215,10 @@ __device__ void rhs(Ctx &c, double t, const double2 *rho, double2 *out) {
 }
 
 // reverse of rhs at (t, rho) for the output cotangent rbar: rho_bar += ..., control gradient scattered into a.grad
-__device__ void rhs_vjp(Ctx &c, double t, const double2 *rho, const double2 *rbar, double2 *rho_bar) {
+template <bool TD> __device__ void rhs_vjp(Ctx &c, double t, const double2 *rho, const double2 *rbar, double2 *rho_bar) {
     const LArgs &a = c.a;
     const int n = a.n, nn = n * n;
-    set_time(c, t);
+    set_time<TD>(c, t);
     bmm<1, 0, true>(rho_bar, c.A1, 0, rbar, nn, n, a.D, 1.0);
     bmm<0, 1, true>(rho_bar, rbar, nn, c.A2, 0, n, a.D, 1.0);
     for (int l = 0; l < a.L; ++l) {
@@ -184,8 +227,10 @@ __device__ void rhs_vjp(Ctx &c, double t, const double2 *rho, const double2 *rba
     }
     if (a.have_h && a.KR > 0) {
         // hbar = -i sum_d (rbar_d rho_d^T - rho_d^T rbar_d);  cbar_r = Re sum_ab hbar_ab (A_r)_ab
+        // (with series the A are the KC channels, and xbar_r = sum_c gain_cr(t) cbar_c)
+        const int nch = (TD && a.KC > 0) ? a.KC : a.KR;
         double part[kMaxKRL];
-        for (int r = 0; r < a.KR; ++r) part[r] = 0.;
+        for (int r = 0; r < nch; ++r) part[r] = 0.;
         for (int e = threadIdx.x; e < nn; e += blockDim.x) {
             const int i = e / n, j = e - i * n;
             double sr = 0., si = 0.;
@@ -199,18 +244,33 @@ __device__ void rhs_vjp(Ctx &c, double t, const double2 *rho, const double2 *rba
                 }
             }
             const double hr = si, hi = -sr;                                    // -i (sr + i si)
-            for (int r = 0; r < a.KR; ++r) {
+            for (int r = 0; r < nch; ++r) {
                 const double2 g = c.Aops[(size_t)r * nn + e];
                 part[r] += hr * g.x - hi * g.y;
             }
         }
         const int i0 = c.loc[0], i1 = c.loc[1];
         const double w = (t - c.xs[i0]) / (c.xs[i1] - c.xs[i0]);
-        for (int r = 0; r < a.KR; ++r) {
-            const double cb = block_sum(part[r], c.red);
-            if (threadIdx.x == 0) {
-                a.grad[i0 * a.KR + r] += cb * (1.0 - w);
-                a.grad[i1 * a.KR + r] += cb * w;
+        if (TD && a.KC > 0) {
+            for (int ch = 0; ch < a.KC; ++ch) {
+                const double cb = block_sum(part[ch], c.red);
+                if (threadIdx.x == 0) c.cbar[ch] = cb;
+            }
+            __syncthreads();
+            if (threadIdx.x == 0)
+                for (int r = 0; r < a.KR; ++r) {
+                    double xb = 0.;
+                    for (int ch = 0; ch < a.KC; ++ch) xb += c.sv[a.KC + ch * a.KR + r] * c.cbar[ch];
+                    a.grad[i0 * a.KR + r] += xb * (1.0 - w);
+                    a.grad[i1 * a.KR + r] += xb * w;
+                }
+        } else {
+            for (int r = 0; r < a.KR; ++r) {
+                const double cb = block_sum(part[r], c.red);
+                if (threadIdx.x == 0) {
+                    a.grad[i0 * a.KR + r] += cb * (1.0 - w);
+                    a.grad[i1 * a.KR + r] += cb * w;
+                }
             }
         }
         __syncthreads();
@@ -224,7 +284,7 @@ __device__ double rms_of(const double2 *x, int count, double *red) {
 }
 
 // the six stages of one attempt from (x0, y0, k[0]); fills k[1..6], y1 and returns err
-__device__ double rk_attempt(Ctx &c, double x0, double h, const double2 *y0, double2 *const *k, double2 *ytmp, double2 *y1) {
+template <bool TD> __device__ double rk_attempt(Ctx &c, double x0, double h, const double2 *y0, double2 *const *k, double2 *ytmp, double2 *y1) {
     const int DE = c.a.D * c.a.n * c.a.n;
     for (int i = 1; i < 6; ++i) {
         for (int e = threadIdx.x; e < DE; e += blockDim.x) {
@@ -233,7 +293,7 @@ __device__ double rk_attempt(Ctx &c, double x0, double h, const double2 *y0, dou
             ytmp[e] = make_double2(y0[e].x + h * acc.x, y0[e].y + h * acc.y);
         }
         __syncthreads();
-        rhs(c, x0 + cC[i] * h, ytmp, k[i]);
+        rhs<TD>(c, x0 + cC[i] * h, ytmp, k[i]);
     }
     for (int e = threadIdx.x; e < DE; e += blockDim.x) {
         double2 acc = make_double2(0., 0.);
@@ -241,7 +301,7 @@ __device__ double rk_attempt(Ctx &c, double x0, double h, const double2 *y0, dou
         y1[e] = make_double2(y0[e].x + h * acc.x, y0[e].y + h * acc.y);
     }
     __syncthreads();
-    rhs(c, x0 + h, y1, k[6]);
+    rhs<TD>(c, x0 + h, y1, k[6]);
     double s = 0.;
     for (int e = threadIdx.x; e < DE; e += blockDim.x) {
         double2 acc = make_double2(0., 0.);
@@ -305,7 +365,7 @@ struct Work {
     double2 *p[24];
 };
 
-__device__ void carve(const LArgs &a, unsigned char *smem, Ctx &c, Work &w, int narr) {
+template <bool TD> __device__ void carve(const LArgs &a, unsigned char *smem, Ctx &c, Work &w, int narr) {
     const int nn = a.n * a.n, DE = a.D * nn;
     double *d = reinterpret_cast<double *>(smem);
     c.A1 = reinterpret_cast<double2 *>(d); d += 2 * nn;
@@ -313,6 +373,11 @@ __device__ void carve(const LArgs &a, unsigned char *smem, Ctx &c, Work &w, int 
     c.red = d; d += 32;
     c.coef = d; d += kMaxKRL;
     c.loc = reinterpret_cast<int *>(d); d += 2;
+    if (TD) {
+        c.sv = d; d += (a.NS + 1) & ~1;
+        c.chan = d; d += kMaxKRL;
+        c.cbar = d; d += kMaxKRL;
+    }
     if (a.ops_in_smem) {                           // the sequential loop re-reads these every stage: keep them on chip
         auto stage = [&](const double *src, int count) {
             double *dst = d;
@@ -322,23 +387,25 @@ __device__ void carve(const LArgs &a, unsigned char *smem, Ctx &c, Work &w, int 
         };
         c.H0 = reinterpret_cast<const double2 *>(stage(reinterpret_cast<const double *>(a.H0), 2 * nn));
         c.Khalf = reinterpret_cast<const double2 *>(stage(reinterpret_cast<const double *>(a.Khalf), 2 * nn));
-        c.Aops = reinterpret_cast<const double2 *>(stage(reinterpret_cast<const double *>(a.Aops), 2 * nn * max(a.KR, 1)));
+        c.Aops = reinterpret_cast<const double2 *>(stage(reinterpret_cast<const double *>(a.Aops), 2 * nn * max(max(a.KR, a.KC), 1)));
         c.Lops = reinterpret_cast<const double2 *>(stage(reinterpret_cast<const double *>(a.Lops), 2 * nn * max(a.L, 1)));
         c.gam = stage(a.gam, max(a.L, 1));
         c.controls = stage(a.controls, max(a.M * a.KR, 1));
         c.xs = stage(a.xs, max(a.M, 1));
+        if (TD && a.tdr) c.Kops = reinterpret_cast<const double2 *>(stage(reinterpret_cast<const double *>(a.Kops), 2 * nn * a.L));
         __syncthreads();
     }
+    if (TD && a.tdr) c.gam = c.sv + a.KC * (1 + a.KR);  // rates r_l(t), refreshed by every set_time
     double2 *base = a.work_in_smem ? reinterpret_cast<double2 *>(d) : a.work;
     c.tmp = base;
     for (int i = 0; i < narr; ++i) w.p[i] = base + (size_t)(i + 1) * DE;
 }
 
-__global__ void __launch_bounds__(LNT) k_lindblad_forward(LArgs a, int keep_tape) {
+template <bool TD> __global__ void __launch_bounds__(LNT) k_lindblad_forward(LArgs a, int keep_tape) {
     extern __shared__ __align__(16) unsigned char smem[];
     Ctx c(a);
     Work w;
-    carve(a, smem, c, w, 12);
+    carve<TD>(a, smem, c, w, 12);
     const int DE = a.D * a.n * a.n;
     double2 *y = w.p[0], *y1 = w.p[1], *ytmp = w.p[2], *out = w.p[3];
     double2 *k[7] = {w.p[4], w.p[5], w.p[6], w.p[7], w.p[8], w.p[9], w.p[10]};
@@ -356,12 +423,12 @@ __global__ void __launch_bounds__(LNT) k_lindblad_forward(LArgs a, int keep_tape
         if (fin) break;
         const double t0 = step * dt, tf = step * dt + dt;
         // initial step size (mathmethods.py:405-420)
-        rhs(c, t0, y, k[0]);
+        rhs<TD>(c, t0, y, k[0]);
         const double d0 = rms_of(y, DE, c.red), d1 = rms_of(k[0], DE, c.red);
         const double h0 = (d0 < 1e-5 || d1 < 1e-5) ? 1e-6 : 0.01 * d0 / d1;
         for (int e = threadIdx.x; e < DE; e += blockDim.x) ytmp[e] = make_double2(y[e].x + h0 * k[0][e].x, y[e].y + h0 * k[0][e].y);
         __syncthreads();
-        rhs(c, t0 + h0, ytmp, k[1]);
+        rhs<TD>(c, t0 + h0, ytmp, k[1]);
         double s = 0.;
         for (int e = threadIdx.x; e < DE; e += blockDim.x) { const double dr = k[1][e].x - k[0][e].x, di = k[1][e].y - k[0][e].y; s += dr * dr + di * di; }
         const double d2 = sqrt(block_sum(s, c.red) / DE) / h0;
@@ -374,7 +441,7 @@ __global__ void __launch_bounds__(LNT) k_lindblad_forward(LArgs a, int keep_tape
             bool rejected = false;
             double hn;
             for (;;) {
-                const double err = rk_attempt(c, xc, h, y, k, ytmp, y1);
+                const double err = rk_attempt<TD>(c, xc, h, y, k, ytmp, y1);
                 ++attempts;
                 if (err < 1.0) {
                     double fac = (err == 0.0) ? 10.0 : fmin(10.0, 0.9 * pow(err, -0.2));
@@ -420,14 +487,15 @@ __global__ void __launch_bounds__(LNT) k_lindblad_forward(LArgs a, int keep_tape
         for (int e = threadIdx.x; e < DE; e += blockDim.x) y[e] = out[e];
         __syncthreads();
     }
-    if (threadIdx.x == 0) { *a.cost = cost; a.stats[0] = attempts; a.stats[1] = accepted; }
+    if (threadIdx.x == 0) { *a.cost = cost; a.stats[0] = attempts; a.stats[1] = accepted; if (TD) *a.tseen = c.tseen; }
 }
 
-__global__ void __launch_bounds__(LNT) k_lindblad_backward(LArgs a) {
+template <bool TD> __global__ void __launch_bounds__(LNT) k_lindblad_backward(LArgs a) {
     extern __shared__ __align__(16) unsigned char smem[];
     Ctx c(a);
     Work w;
-    carve(a, smem, c, w, 22);
+    if (TD && *a.tseen > a.segs * a.seg_w) return;    // the forward pass left the table: it is run again
+    carve<TD>(a, smem, c, w, 22);
     const int DE = a.D * a.n * a.n;
     double2 *k[7] = {w.p[0], w.p[1], w.p[2], w.p[3], w.p[4], w.p[5], w.p[6]};
     double2 *kb[7] = {w.p[7], w.p[8], w.p[9], w.p[10], w.p[11], w.p[12], w.p[13]};
@@ -446,7 +514,7 @@ __global__ void __launch_bounds__(LNT) k_lindblad_backward(LArgs a) {
             const double2 *y0 = a.tape_y + (size_t)i * DE;
             for (int e = threadIdx.x; e < DE; e += blockDim.x) k[0][e] = a.tape_k1[(size_t)i * DE + e];
             __syncthreads();
-            rk_attempt(c, x0, h, y0, k, ytmp, y1);
+            rk_attempt<TD>(c, x0, h, y0, k, ytmp, y1);
             for (int e = threadIdx.x; e < DE; e += blockDim.x) {
                 for (int j = 0; j < 6; ++j) kb[j][e] = make_double2(0., 0.);
                 kb[6][e] = k1b_next[e];
@@ -470,7 +538,7 @@ __global__ void __launch_bounds__(LNT) k_lindblad_backward(LArgs a) {
             }
             __syncthreads();
             // ks[6] = rhs(x0 + h, y1)
-            rhs_vjp(c, x0 + h, y1, kb[6], y1b);
+            rhs_vjp<TD>(c, x0 + h, y1, kb[6], y1b);
             // y1 = y0 + h sum b_j k_j
             for (int e = threadIdx.x; e < DE; e += blockDim.x) {
                 y0b[e].x += y1b[e].x; y0b[e].y += y1b[e].y;
@@ -485,7 +553,7 @@ __global__ void __launch_bounds__(LNT) k_lindblad_backward(LArgs a) {
                     zb[e] = make_double2(0., 0.);
                 }
                 __syncthreads();
-                rhs_vjp(c, x0 + cC[s] * h, ytmp, kb[s], zb);
+                rhs_vjp<TD>(c, x0 + cC[s] * h, ytmp, kb[s], zb);
                 for (int e = threadIdx.x; e < DE; e += blockDim.x) {
                     y0b[e].x += zb[e].x; y0b[e].y += zb[e].y;
                     for (int j = 0; j < s; ++j) { kb[j][e].x += h * cA[s][j] * zb[e].x; kb[j][e].y += h * cA[s][j] * zb[e].y; }
@@ -496,7 +564,7 @@ __global__ void __launch_bounds__(LNT) k_lindblad_backward(LArgs a) {
             __syncthreads();
         }
         // k1 of the interval's first step = rhs(t0, y_in)
-        rhs_vjp(c, step * (a.T / (a.N - 1)), a.states + (size_t)step * DE, k1b_next, rbar);
+        rhs_vjp<TD>(c, step * (a.T / (a.N - 1)), a.states + (size_t)step * DE, k1b_next, rbar);
         if (a.nterms > 0 && is_cost_step(step, a.ces)) density_costs(c, a.states + (size_t)step * DE, true, false, rbar);
     }
 }
@@ -521,10 +589,12 @@ template <class T> struct Buf {
 struct qocb_lplan {
     qocb_lindblad_problem pb;
     int cap = 0;
-    bool ops_set = false, rho_set = false, costs_dirty = true;
+    bool ops_set = false, rho_set = false, costs_dirty = true, series_set = false;
+    int NS = 0, segs = 0, deg = 0;                 // time series: NS = KC*(1+KR) + (time_dependent_rates ? L : 0)
+    double seg_w = 0.;
     cudaStream_t stream = nullptr;
-    Buf<double2> H0, Aops, Lops, Khalf, rho0, mats, states, tape_y, tape_k1, work;
-    Buf<double> gam, controls, xs, cost, tape_x, tape_h, grad;
+    Buf<double2> H0, Aops, Lops, Khalf, Kops, rho0, mats, states, tape_y, tape_k1, work;
+    Buf<double> gam, controls, xs, cost, tape_x, tape_h, grad, series, tseen;
     Buf<int> counts, first, hit, err_flag;
     Buf<long long> stats;
     Buf<DTerm> terms;
@@ -548,6 +618,8 @@ LArgs make_largs(qocb_lplan *p) {
     a.states = p->states.p; a.cost = p->cost.p; a.tape_x = p->tape_x.p; a.tape_h = p->tape_h.p; a.tape_y = p->tape_y.p;
     a.tape_k1 = p->tape_k1.p; a.first = p->first.p; a.hit = p->hit.p; a.stats = p->stats.p; a.err_flag = p->err_flag.p;
     a.work = p->work.p; a.work_in_smem = 0; a.ops_in_smem = p->ops_in_smem; a.grad = p->grad.p;
+    a.KC = p->pb.channel_count; a.tdr = p->pb.time_dependent_rates; a.NS = p->NS; a.segs = p->segs; a.deg = p->deg;
+    a.seg_w = p->seg_w; a.series = p->series.p; a.Kops = p->Kops.p; a.tseen = p->tseen.p;
     return a;
 }
 
@@ -567,6 +639,7 @@ int upload_lcosts(qocb_lplan *p) {
 
 int run_lindblad(qocb_lplan *p, const double *controls, bool with_grad, double *cost, double *grad, double *final_densities) {
     if (!p->ops_set || !p->rho_set) return lfail(p, "operators and densities must be set before evaluation", -1);
+    if (p->NS > 0 && !p->series_set) return lfail(p, "time-dependent operators need qocb_lindblad_set_time_series before evaluation", -1);
     LTRY(p, cudaSetDevice(p->pb.device));
     if (upload_lcosts(p)) return -2;
     const size_t cnt = (size_t)p->pb.control_eval_count * p->pb.control_count;
@@ -579,10 +652,12 @@ int run_lindblad(qocb_lplan *p, const double *controls, bool with_grad, double *
     a.work_in_smem = p->in_smem_fwd;
     const int DEl = p->pb.density_count * p->pb.hilbert_size * p->pb.hilbert_size;
     const int nt = DEl <= 64 ? 32 : (DEl <= 256 ? 128 : LNT);
-    k_lindblad_forward<<<1, nt, p->smem_fwd, p->stream>>>(a, with_grad ? 1 : 0);
+    if (p->NS > 0) k_lindblad_forward<true><<<1, nt, p->smem_fwd, p->stream>>>(a, with_grad ? 1 : 0);
+    else k_lindblad_forward<false><<<1, nt, p->smem_fwd, p->stream>>>(a, with_grad ? 1 : 0);
     if (with_grad && cnt) {
         a.work_in_smem = p->in_smem_bwd;
-        k_lindblad_backward<<<1, nt, p->smem_bwd, p->stream>>>(a);
+        if (p->NS > 0) k_lindblad_backward<true><<<1, nt, p->smem_bwd, p->stream>>>(a);
+        else k_lindblad_backward<false><<<1, nt, p->smem_bwd, p->stream>>>(a);
     }
     LTRY(p, cudaGetLastError());
     int flag = 0;
@@ -593,7 +668,11 @@ int run_lindblad(qocb_lplan *p, const double *controls, bool with_grad, double *
     if (final_densities)
         LTRY(p, cudaMemcpyAsync(final_densities, p->states.p + (size_t)(p->pb.system_eval_count - 1) * DE, sizeof(double2) * DE,
                                 cudaMemcpyDeviceToHost, p->stream));
+    double tseen = 0.;
+    if (p->NS > 0) LTRY(p, cudaMemcpyAsync(&tseen, p->tseen.p, sizeof(double), cudaMemcpyDeviceToHost, p->stream));
     LTRY(p, cudaStreamSynchronize(p->stream));
+    if (p->NS > 0 && tseen > p->segs * p->seg_w)
+        return lfail(p, "a Runge-Kutta stage time lies beyond the time series: extend it (qocb_lindblad_max_stage_time)", -5);
     if (flag) return lfail(p, "the Runge-Kutta tape is full: raise max_rk_steps", -4);
     return 0;
 }
@@ -612,6 +691,10 @@ int qocb_lindblad_create(const qocb_lindblad_problem *pb, qocb_lplan **out) {
     if (pb->control_count < 0 || pb->control_count > kMaxKRL) return lfail(nullptr, "control_count (real channels) must be in [0, 16]", -1);
     if (pb->control_count > 0 && pb->control_eval_count < 2) return lfail(nullptr, "control_eval_count must be >= 2", -1);
     if (pb->lindblad_count < 0) return lfail(nullptr, "lindblad_count must be >= 0", -1);
+    if (pb->channel_count < 0 || pb->channel_count > kMaxKRL) return lfail(nullptr, "channel_count must be in [0, 16]", -1);
+    if (pb->channel_count > 0 && !pb->have_hamiltonian) return lfail(nullptr, "channel_count > 0 needs have_hamiltonian", -1);
+    if (pb->time_dependent_rates != 0 && (pb->time_dependent_rates != 1 || pb->lindblad_count < 1))
+        return lfail(nullptr, "time_dependent_rates must be 0 or 1, and 1 needs lindblad_count >= 1", -1);
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return lfail(nullptr, "no CUDA device available (this library has no CPU path)", -2);
     qocb_lplan *p = new qocb_lplan();
@@ -620,10 +703,13 @@ int qocb_lindblad_create(const qocb_lindblad_problem *pb, qocb_lplan **out) {
     CTRY(cudaSetDevice(pb->device));
     CTRY(cudaStreamCreateWithFlags(&p->stream, cudaStreamNonBlocking));
     const int n = pb->hilbert_size, nn = n * n, D = pb->density_count, KR = pb->control_count, M = pb->control_eval_count;
-    const int N = pb->system_eval_count, L = pb->lindblad_count;
+    const int N = pb->system_eval_count, L = pb->lindblad_count, KC = pb->channel_count, tdr = pb->time_dependent_rates;
     const size_t DE = (size_t)D * nn;
+    p->NS = KC * (1 + KR) + (tdr ? L : 0);
     p->cap = pb->max_rk_steps > 0 ? pb->max_rk_steps : (int)std::max<size_t>(4096, std::min<size_t>((size_t)1 << 20, ((size_t)512 << 20) / (2 * DE * sizeof(double2))));
-    CTRY(p->H0.alloc(nn)); CTRY(p->Aops.alloc((size_t)std::max(1, KR) * nn)); CTRY(p->Lops.alloc((size_t)std::max(1, L) * nn));
+    CTRY(p->H0.alloc(nn)); CTRY(p->Aops.alloc((size_t)std::max(1, std::max(KR, KC)) * nn)); CTRY(p->Lops.alloc((size_t)std::max(1, L) * nn));
+    if (tdr) CTRY(p->Kops.alloc((size_t)L * nn));
+    if (p->NS > 0) { CTRY(p->tseen.alloc(1)); CTRY(cudaMemset(p->tseen.p, 0, sizeof(double))); }
     CTRY(p->Khalf.alloc(nn)); CTRY(p->gam.alloc(std::max(1, L))); CTRY(p->controls.alloc(std::max<size_t>(1, (size_t)M * KR)));
     CTRY(p->xs.alloc(std::max(1, M))); CTRY(p->rho0.alloc(DE)); CTRY(p->states.alloc((size_t)N * DE)); CTRY(p->cost.alloc(1));
     CTRY(p->tape_x.alloc(p->cap)); CTRY(p->tape_h.alloc(p->cap)); CTRY(p->tape_y.alloc((size_t)p->cap * DE)); CTRY(p->tape_k1.alloc((size_t)p->cap * DE));
@@ -638,16 +724,20 @@ int qocb_lindblad_create(const qocb_lindblad_problem *pb, qocb_lplan **out) {
         CTRY(cudaMemcpy(p->xs.p, xs.data(), sizeof(double) * M, cudaMemcpyHostToDevice));
     }
     size_t fixed = sizeof(double) * (4 * (size_t)nn + 32 + kMaxKRL + 2);
+    if (p->NS > 0) fixed += sizeof(double) * (((size_t)p->NS + 1) / 2 * 2 + 2 * kMaxKRL);     // series values, coef_c, cbar_c
     const size_t limit = 200 * 1024;
-    const size_t ops_doubles = 2 * (size_t)nn * (2 + std::max(KR, 1) + std::max(L, 1)) + std::max(L, 1) + std::max(M * KR, 1) + std::max(M, 1) + 16;
+    const size_t ops_doubles = 2 * (size_t)nn * (2 + std::max(std::max(KR, KC), 1) + std::max(L, 1) + (tdr ? L : 0)) + std::max(L, 1) +
+                               std::max(M * KR, 1) + std::max(M, 1) + 16;
     p->ops_in_smem = ops_doubles * sizeof(double) <= 48 * 1024;
     if (p->ops_in_smem) fixed += ops_doubles * sizeof(double);
     const size_t need_f = fixed + sizeof(double2) * 13 * DE, need_b = fixed + sizeof(double2) * 23 * DE;
     p->in_smem_fwd = need_f <= limit; p->in_smem_bwd = need_b <= limit;
     p->smem_fwd = p->in_smem_fwd ? need_f : fixed; p->smem_bwd = p->in_smem_bwd ? need_b : fixed;
     if (fixed > limit) { g_lerr = "hilbert_size too large for the Lindblad kernels' shared-memory operators"; delete p; return -1; }
-    CTRY(cudaFuncSetAttribute(k_lindblad_forward, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
-    CTRY(cudaFuncSetAttribute(k_lindblad_backward, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
+    CTRY(cudaFuncSetAttribute(k_lindblad_forward<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
+    CTRY(cudaFuncSetAttribute(k_lindblad_backward<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
+    CTRY(cudaFuncSetAttribute(k_lindblad_forward<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
+    CTRY(cudaFuncSetAttribute(k_lindblad_backward<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
 #undef CTRY
     *out = p;
     return 0;
@@ -665,13 +755,32 @@ int qocb_lindblad_destroy(qocb_lplan *p) {
 int qocb_lindblad_set_operators(qocb_lplan *p, const double *h0, const double *a_ops, const double *gammas, const double *lops) {
     if (!p) return -1;
     LTRY(p, cudaSetDevice(p->pb.device));
-    const int n = p->pb.hilbert_size, nn = n * n, KR = p->pb.control_count, L = p->pb.lindblad_count;
+    const int n = p->pb.hilbert_size, nn = n * n, L = p->pb.lindblad_count;
+    const int KA = p->pb.channel_count > 0 ? p->pb.channel_count : p->pb.control_count;     // operators in a_ops
     if (p->pb.have_hamiltonian) {
-        if (!h0 || (KR > 0 && !a_ops)) return lfail(p, "h0 / a_ops missing", -1);
+        if (!h0 || (KA > 0 && !a_ops)) return lfail(p, "h0 / a_ops missing", -1);
         LTRY(p, cudaMemcpy(p->H0.p, h0, sizeof(double2) * nn, cudaMemcpyHostToDevice));
-        if (KR > 0) LTRY(p, cudaMemcpy(p->Aops.p, a_ops, sizeof(double2) * (size_t)KR * nn, cudaMemcpyHostToDevice));
+        if (KA > 0) LTRY(p, cudaMemcpy(p->Aops.p, a_ops, sizeof(double2) * (size_t)KA * nn, cudaMemcpyHostToDevice));
     }
-    if (L > 0) {
+    if (L > 0 && p->pb.time_dependent_rates) {                              // per-operator 1/2 B_l^dag B_l; rates come from the series
+        if (!lops) return lfail(p, "lops missing", -1);
+        LTRY(p, cudaMemcpy(p->Lops.p, lops, sizeof(double2) * (size_t)L * nn, cudaMemcpyHostToDevice));
+        std::vector<double> kh(2 * (size_t)L * nn, 0.0);
+        for (int l = 0; l < L; ++l) {
+            const double *Lm = lops + 2 * (size_t)l * nn;
+            double *K = kh.data() + 2 * (size_t)l * nn;
+            for (int i = 0; i < n; ++i)
+                for (int j = 0; j < n; ++j) {
+                    double sr = 0., si = 0.;
+                    for (int k = 0; k < n; ++k) {                             // conj(B[k][i]) * B[k][j]
+                        const double ar = Lm[2 * (k * n + i)], ai = -Lm[2 * (k * n + i) + 1], br = Lm[2 * (k * n + j)], bi = Lm[2 * (k * n + j) + 1];
+                        sr += ar * br - ai * bi; si += ar * bi + ai * br;
+                    }
+                    K[2 * (i * n + j)] = 0.5 * sr; K[2 * (i * n + j) + 1] = 0.5 * si;
+                }
+        }
+        LTRY(p, cudaMemcpy(p->Kops.p, kh.data(), sizeof(double2) * (size_t)L * nn, cudaMemcpyHostToDevice));
+    } else if (L > 0) {
         if (!gammas || !lops) return lfail(p, "gammas / lops missing", -1);
         LTRY(p, cudaMemcpy(p->gam.p, gammas, sizeof(double) * L, cudaMemcpyHostToDevice));
         LTRY(p, cudaMemcpy(p->Lops.p, lops, sizeof(double2) * (size_t)L * nn, cudaMemcpyHostToDevice));
@@ -691,6 +800,30 @@ int qocb_lindblad_set_operators(qocb_lplan *p, const double *h0, const double *a
         LTRY(p, cudaMemcpy(p->Khalf.p, kh.data(), sizeof(double2) * nn, cudaMemcpyHostToDevice));
     }
     p->ops_set = true;
+    return 0;
+}
+
+/* series: [segments][degree+1][NS] Chebyshev coefficients (the constant one not halved) on [s w, (s+1) w] */
+int qocb_lindblad_set_time_series(qocb_lplan *p, int32_t segments, int32_t degree, double segment_width, const double *series) {
+    if (!p || !series) return lfail(p, "null argument", -1);
+    if (p->NS == 0) return lfail(p, "this plan has neither operator channels nor time-dependent rates", -1);
+    if (segments < 1 || degree < 0 || degree > 64 || !(segment_width > 0.0)) return lfail(p, "bad time series shape", -1);
+    LTRY(p, cudaSetDevice(p->pb.device));
+    const size_t count = (size_t)segments * (degree + 1) * p->NS;
+    LTRY(p, cudaStreamSynchronize(p->stream));
+    LTRY(p, p->series.alloc(count));
+    LTRY(p, cudaMemcpy(p->series.p, series, sizeof(double) * count, cudaMemcpyHostToDevice));
+    p->segs = segments; p->deg = degree; p->seg_w = segment_width;
+    p->series_set = true;
+    return 0;
+}
+
+/* largest Runge-Kutta stage time of the last forward pass (plans with a time series) */
+int qocb_lindblad_max_stage_time(qocb_lplan *p, double *t) {
+    if (!p || !t) return lfail(p, "null argument", -1);
+    if (p->NS == 0) return lfail(p, "this plan has no time series", -1);
+    LTRY(p, cudaSetDevice(p->pb.device));
+    LTRY(p, cudaMemcpy(t, p->tseen.p, sizeof(double), cudaMemcpyDeviceToHost));
     return 0;
 }
 
