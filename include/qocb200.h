@@ -254,6 +254,22 @@ int qocb_lindblad_add_cost(qocb_lplan *plan, int32_t kind, int32_t step_cost, do
 int qocb_lindblad_cost(qocb_lplan *plan, const double *controls, double *cost, double *final_densities);
 int qocb_lindblad_cost_and_grad(qocb_lplan *plan, const double *controls, double *cost, double *grad,
                                 double *final_densities);
+/* The same evaluation in two calls, for cost terms the host evaluates itself on the densities (user-defined Cost subclasses,
+   qoc/models/cost.py:5-51, on any subset of the system steps):
+     - qocb_lindblad_forward runs the forward pass and keeps the reverse-pass tape.  `cost` is the value of the device cost
+       terms only; the densities of every step are then available through qocb_lindblad_get_densities.  Return codes as
+       qocb_lindblad_cost_and_grad, including -4 (tape full) and -5 (stage time beyond the series: extend and call again).
+     - qocb_lindblad_backward runs the reverse pass of that forward pass and returns the gradient of (device costs + host
+       terms).  seeds is NULL or [N][D][n][n] complex: row k = d c / d Re rho_k - i d c / d Im rho_k of the host terms at system
+       step k (autograd's convention, the one the device costs use).  Row N-1 is added before the reverse sweep starts, row k
+       next to the device step costs of step k; row 0 has no effect.  qocb_lindblad_forward followed by
+       qocb_lindblad_backward(seeds = NULL) gives bit-identical results to qocb_lindblad_cost_and_grad.
+   TAPE RULE: qocb_lindblad_backward needs a qocb_lindblad_forward that returned 0 as the plan's last evaluation, with no
+   setter in between (qocb_lindblad_cost and qocb_lindblad_cost_and_grad overwrite the densities without that tape);
+   otherwise it returns -1.  It may be called more than once on one tape.  With control_count = 0 it writes nothing and
+   returns 0.  The seed buffer is allocated on first use: plans that never pass seeds allocate nothing for it. */
+int qocb_lindblad_forward(qocb_lplan *plan, const double *controls, double *cost, double *final_densities);
+int qocb_lindblad_backward(qocb_lplan *plan, const double *seeds, double *grad);
 /* stats[0] = Runge-Kutta attempts, stats[1] = accepted steps of the last evaluation */
 int qocb_lindblad_stats(qocb_lplan *plan, int64_t *stats);
 /* densities at every system step of the last evaluation: [N][D][n][n] (save_intermediate_densities payload) */

@@ -30,7 +30,7 @@ EXPORTS = [
     "qocb_lindblad_create", "qocb_lindblad_destroy", "qocb_lindblad_last_error",
     "qocb_lindblad_set_operators", "qocb_lindblad_set_densities", "qocb_lindblad_add_cost", "qocb_lindblad_cost",
     "qocb_lindblad_cost_and_grad", "qocb_lindblad_stats", "qocb_lindblad_get_densities", "qocb_lindblad_set_time_series",
-    "qocb_lindblad_max_stage_time",
+    "qocb_lindblad_max_stage_time", "qocb_lindblad_forward", "qocb_lindblad_backward",
 ]
 
 
@@ -145,6 +145,8 @@ def load():
     lib.qocb_lindblad_add_cost.argtypes = [vp, i32, i32, dbl, vp, vp, i32]
     lib.qocb_lindblad_cost.argtypes = [vp, vp, vp, vp]
     lib.qocb_lindblad_cost_and_grad.argtypes = [vp, vp, vp, vp, vp]
+    lib.qocb_lindblad_forward.argtypes = [vp, vp, vp, vp]
+    lib.qocb_lindblad_backward.argtypes = [vp, vp, vp]
     lib.qocb_lindblad_stats.argtypes = [vp, vp]
     lib.qocb_lindblad_get_densities.argtypes = [vp, vp]
     lib.qocb_lindblad_set_time_series.argtypes = [vp, i32, i32, dbl, vp]

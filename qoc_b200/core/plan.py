@@ -230,6 +230,51 @@ def extract_hamiltonian_structure(hamiltonian, control_count, complex_controls, 
     return h0, a_ops
 
 
+def central_differences(f, z):
+    """4-point central differences (step 1e-3 max(1, |z_i|), error O(h^4)) of the real function `f` at every entry of the
+    array `z`, of any shape: returns (df/dRe z, df/dIm z), the second None for real `z`.  Every entry is differentiated on its
+    own, so a function that reads only one triangle of a matrix (eigvalsh and the like) gets the derivative of what it computes
+    on general matrices, not of its Hermitian restriction.  Used for the cotangents of user-defined costs."""
+    z = np.asarray(z)
+    directions = (1.0, 1j) if np.iscomplexobj(z) else (1.0,)
+    parts = [np.zeros(z.shape) for _ in directions]
+    for idx in np.ndindex(*z.shape):
+        h = 1e-3 * max(1.0, abs(z[idx]))
+        for part, direction in zip(parts, directions):
+            vals = []
+            for k in (1.0, -1.0, 2.0, -2.0):
+                q = z.copy()
+                q[idx] += k * h * direction
+                vals.append(f(q))
+            part[idx] = (8.0 * (vals[0] - vals[1]) - (vals[2] - vals[3])) / (12.0 * h)
+    return parts[0], (parts[1] if len(parts) > 1 else None)
+
+
+def explicit_control_grad(f, controls):
+    """df/dRe u + i df/dIm u (df/du for real controls) of a user-cost sum `f(controls)` whose densities or states are held
+    fixed, or None when f does not move under one random probe of the controls (most user costs never read them)."""
+    controls = np.asarray(controls)
+    base = f(controls)
+    rng = np.random.default_rng(0)
+    probe = controls + 1e-3 * (rng.standard_normal(controls.shape) + (1j * rng.standard_normal(controls.shape)
+                                                                        if np.iscomplexobj(controls) else 0))
+    if abs(f(probe) - base) <= 1e-14 * max(1.0, abs(base)):
+        return None
+    dre, dim = central_differences(f, controls)
+    g = np.zeros(controls.shape, dtype=controls.dtype)
+    g[...] = dre if dim is None else dre + 1j * dim
+    return g
+
+
+def is_user_cost(cost):
+    """a user-defined Cost subclass (qoc/models/cost.py:5-51): it overrides none of the B200 hooks (`device_terms`,
+    `device_terms_density`, `control_value_and_grad`), so `cost(controls, states_or_densities, step)` is all it has."""
+    from qoc_b200.models.cost import Cost
+    t = type(cost)
+    return (getattr(t, "device_terms", Cost.device_terms) is Cost.device_terms and getattr(t, "device_terms_density", None) is None
+            and getattr(t, "control_value_and_grad", Cost.control_value_and_grad) is Cost.control_value_and_grad)
+
+
 class SchroedingerPlan(object):
     """Device plan for `_evaluate_schroedinger_discrete` and its jacobian (schroedingerdiscrete.py:356-438,
     :318).  `cost(controls)` and `cost_and_grad(controls)` take controls in cost-function format
@@ -364,44 +409,12 @@ class SchroedingerPlan(object):
 
     def _user_seed(self, controls, finals):
         """d c / d Re psi - i d c / d Im psi of the summed user costs at the final states (autograd's cotangent convention)."""
-        seed = np.zeros((self.S, self.n), dtype=np.complex128)
-        psi = np.array(finals, dtype=np.complex128)
-        for s_ in range(self.S):
-            for a in range(self.n):
-                h = 1e-3 * max(1.0, abs(psi[s_, a, 0]))
-                d = []
-                for direction in (1.0, 1j):
-                    vals = []
-                    for k in (1.0, -1.0, 2.0, -2.0):
-                        q = psi.copy()
-                        q[s_, a, 0] += k * h * direction
-                        vals.append(self._user_value(controls, q))
-                    d.append((8.0 * (vals[0] - vals[1]) - (vals[2] - vals[3])) / (12.0 * h))
-                seed[s_, a] = d[0] - 1j * d[1]
-        return seed
+        dre, dim = central_differences(lambda q: self._user_value(controls, q), np.array(finals, dtype=np.complex128))
+        return (dre - 1j * dim).reshape(self.S, self.n)
 
     def _user_control_grad(self, controls, finals):
         """explicit dependence of the user costs on the controls (most have none: one probe decides)."""
-        controls = np.asarray(controls)
-        base = self._user_value(controls, finals)
-        rng = np.random.default_rng(0)
-        probe = controls + 1e-3 * (rng.standard_normal(controls.shape) + (1j * rng.standard_normal(controls.shape)
-                                                                            if np.iscomplexobj(controls) else 0))
-        if abs(self._user_value(probe, finals) - base) <= 1e-14 * max(1.0, abs(base)):
-            return None
-        g = np.zeros(controls.shape, dtype=controls.dtype)
-        for idx in np.ndindex(*controls.shape):
-            h = 1e-3 * max(1.0, abs(controls[idx]))
-            parts = []
-            for direction in ((1.0, 1j) if np.iscomplexobj(controls) else (1.0,)):
-                vals = []
-                for k in (1.0, -1.0, 2.0, -2.0):
-                    q = controls.copy()
-                    q[idx] += k * h * direction
-                    vals.append(self._user_value(q, finals))
-                parts.append((8.0 * (vals[0] - vals[1]) - (vals[2] - vals[3])) / (12.0 * h))
-            g[idx] = parts[0] + (1j * parts[1] if len(parts) > 1 else 0)
-        return g
+        return explicit_control_grad(lambda u: self._user_value(u, finals), controls)
 
     def _eval_with_user_costs(self, controls, want_grad):
         x = self._real_channels(controls)
@@ -1006,13 +1019,17 @@ class LindbladPlan(object):
         self.handle = None
         self._open()
         self.control_costs = []
+        self.user_costs = []
         self._terms = []
         from qoc_b200.models.cost import Cost
         for c in self.costs:
+            if is_user_cost(c):
+                self.user_costs.append(c)
+                continue
             terms = c.device_terms_density(self.D, self.n) if hasattr(c, "device_terms_density") else None
             if not terms:
                 # only genuine control-only costs (classes that override the analytic hook) may skip the device: a state
-                # cost passed by mistake or a user-defined density cost must not be dropped silently
+                # cost passed by mistake must not be dropped silently
                 hook = getattr(type(c), "control_value_and_grad", None)
                 if terms is None or hook is None or hook is Cost.control_value_and_grad:
                     raise NotImplementedError("The cost {} has no B200 device descriptor for the Lindblad path (no CPU "
@@ -1024,6 +1041,13 @@ class LindbladPlan(object):
                         None if counts is None else np.ascontiguousarray(counts, dtype=np.int32))
                 self._terms.append(term)
                 self._add_term(term)
+        # user costs by system step, where the reference evaluates them (lindbladdiscrete.py:384-441): step costs at every
+        # k % cost_eval_step == 0, k != 0, the others once on the final densities
+        ces = int(cost_eval_step)
+        self._user_at = {}
+        for c in self.user_costs:
+            for k in (range(ces, self.N, ces) if getattr(c, "requires_step_evaluation", False) else (self.N - 1,)):
+                self._user_at.setdefault(k, []).append(c)
 
     def _open(self):
         """creates the device plan and uploads operators, densities and (time-dependent problems) the series table."""
@@ -1092,31 +1116,74 @@ class LindbladPlan(object):
     _control_costs = SchroedingerPlan._control_costs
     cost_and_grad_autograd = SchroedingerPlan.cost_and_grad_autograd
 
+    # -- user-defined costs: value and density cotangents by 4-point central differences of `cost(controls, densities, step)`
+    def _user_value_at(self, controls, rho, k):
+        return float(sum(np.real(c.cost(controls, rho, k)) for c in self._user_at[k]))
+
+    def _user_densities(self, final_densities):
+        """{step: densities of the last evaluation} for the steps that carry user costs."""
+        if list(self._user_at) == [self.N - 1]:
+            return {self.N - 1: final_densities}
+        dens = self.intermediate_densities()
+        return {k: dens[k] for k in self._user_at}
+
+    def _user_value(self, controls, dens):
+        return sum(self._user_value_at(controls, dens[k], k) for k in sorted(dens))
+
+    def _user_seeds(self, controls, dens):
+        """[N][D][n][n] seed table of qocb_lindblad_backward: row k = d c / d Re rho_k - i d c / d Im rho_k of the user
+        costs evaluated at step k (each density entry differentiated on its own), zero elsewhere."""
+        seeds = np.zeros((self.N, self.D, self.n, self.n), dtype=np.complex128)
+        for k, rho in dens.items():
+            dre, dim = central_differences(lambda r: self._user_value_at(controls, r, k), rho)
+            seeds[k] = dre - 1j * dim
+        return seeds
+
     def cost(self, controls):
         x = self._real_channels(controls) if controls is not None else None
         out = np.zeros(1)
         fd = np.empty((self.D, self.n, self.n), dtype=np.complex128)
         self._evaluate(lambda h: self.lib.qocb_lindblad_cost(h, _lib.ptr(x), _lib.ptr(out), _lib.ptr(fd)))
+        value = float(out[0])
+        if self.user_costs:
+            value += self._user_value(controls, self._user_densities(fd))
         extra, _ = self._control_costs(controls, False) if controls is not None else (0.0, None)
-        return float(out[0]) + extra, fd
+        return value + extra, fd
 
     def cost_and_grad(self, controls):
-        """(error, grads, final_densities); grads = dE/dRe(u) + i dE/dIm(u) for complex controls."""
+        """(error, grads, final_densities); grads = dE/dRe(u) + i dE/dIm(u) for complex controls.  With user costs the
+        forward pass keeps its tape, the host evaluates the user costs on the densities, and the reverse pass is seeded with
+        their numeric cotangents (qocb_lindblad_forward / qocb_lindblad_backward)."""
         x = self._real_channels(controls)
         out = np.zeros(1)
         fd = np.empty((self.D, self.n, self.n), dtype=np.complex128)
         controls = np.asarray(controls)
-        if self.KR == 0:                                   # hamiltonian = None: the state costs do not see the controls
+        g = np.zeros((self.M, self.KR))
+        if self.KR == 0:                                   # hamiltonian = None: the densities do not see the controls
             self._evaluate(lambda h: self.lib.qocb_lindblad_cost(h, None, _lib.ptr(out), _lib.ptr(fd)))
+        elif self.user_costs:
+            self._evaluate(lambda h: self.lib.qocb_lindblad_forward(h, _lib.ptr(x), _lib.ptr(out), _lib.ptr(fd)))
+        else:
+            self._evaluate(lambda h: self.lib.qocb_lindblad_cost_and_grad(h, _lib.ptr(x), _lib.ptr(out), _lib.ptr(g), _lib.ptr(fd)))
+        value, user_grad = float(out[0]), None
+        if self.user_costs:
+            dens = self._user_densities(fd)
+            value += self._user_value(controls, dens)
+            if self.KR:
+                seeds = self._user_seeds(controls, dens)
+                self._check(self.lib.qocb_lindblad_backward(self.handle, _lib.ptr(seeds), _lib.ptr(g)))
+            if controls.ndim:
+                user_grad = explicit_control_grad(lambda u: self._user_value(u, dens), controls)
+        if self.KR == 0:
             grads = np.zeros(controls.shape, dtype=controls.dtype)
         else:
-            g = np.zeros((self.M, self.KR))
-            self._evaluate(lambda h: self.lib.qocb_lindblad_cost_and_grad(h, _lib.ptr(x), _lib.ptr(out), _lib.ptr(g), _lib.ptr(fd)))
             grads = g[:, :self.K] + 1j * g[:, self.K:] if self.complex_controls else g
+        if user_grad is not None:
+            grads = grads + user_grad
         extra, extra_grad = self._control_costs(controls, True)
         if extra_grad is not None:
             grads = grads + extra_grad
-        return float(out[0]) + extra, grads, fd
+        return value + extra, grads, fd
 
     def stats(self):
         s = np.zeros(2, dtype=np.int64)

@@ -76,6 +76,7 @@ struct LArgs {
     const double *series;                       // [segs][deg+1][NS]
     const double2 *Kops;                        // [L][n*n] 1/2 B_l^dag B_l (tdr)
     double *tseen;                              // largest stage time of the forward pass
+    const double2 *seeds;                       // [N][D*n*n] host-cost cotangents of the densities, or null
 };
 
 // block-wide sum, result in all threads
@@ -361,6 +362,14 @@ __device__ double density_costs(Ctx &c, const double2 *rho, bool step_state, boo
 
 __device__ __forceinline__ bool is_cost_step(int k, int ces) { return k != 0 && (k % ces) == 0; }
 
+// rbar += seeds[step]: cotangents of costs the host evaluated on the densities of this step (qocb_lindblad_backward)
+__device__ void add_seed(const LArgs &a, int step, double2 *rbar) {
+    const int DE = a.D * a.n * a.n;
+    const double2 *s = a.seeds + (size_t)step * DE;
+    for (int e = threadIdx.x; e < DE; e += blockDim.x) { rbar[e].x += s[e].x; rbar[e].y += s[e].y; }
+    __syncthreads();
+}
+
 struct Work {
     double2 *p[24];
 };
@@ -503,6 +512,7 @@ template <bool TD> __global__ void __launch_bounds__(LNT) k_lindblad_backward(LA
     for (int e = threadIdx.x; e < a.M * a.KR; e += blockDim.x) a.grad[e] = 0.;
     for (int e = threadIdx.x; e < DE; e += blockDim.x) rbar[e] = make_double2(0., 0.);
     __syncthreads();
+    if (a.seeds) add_seed(a, a.N - 1, rbar);
     if (a.nterms > 0) density_costs(c, a.states + (size_t)(a.N - 1) * DE, is_cost_step(a.N - 1, a.ces), true, rbar);
     for (int step = a.N - 2; step >= 0; --step) {
         const int first = a.first[step], last = a.hit[step];
@@ -566,6 +576,7 @@ template <bool TD> __global__ void __launch_bounds__(LNT) k_lindblad_backward(LA
         // k1 of the interval's first step = rhs(t0, y_in)
         rhs_vjp<TD>(c, step * (a.T / (a.N - 1)), a.states + (size_t)step * DE, k1b_next, rbar);
         if (a.nterms > 0 && is_cost_step(step, a.ces)) density_costs(c, a.states + (size_t)step * DE, true, false, rbar);
+        if (a.seeds && step > 0) add_seed(a, step, rbar);     // row 0: the cotangent of rho0 is not needed
     }
 }
 
@@ -593,7 +604,8 @@ struct qocb_lplan {
     int NS = 0, segs = 0, deg = 0;                 // time series: NS = KC*(1+KR) + (time_dependent_rates ? L : 0)
     double seg_w = 0.;
     cudaStream_t stream = nullptr;
-    Buf<double2> H0, Aops, Lops, Khalf, Kops, rho0, mats, states, tape_y, tape_k1, work;
+    bool tape_ok = false;                          // the last evaluation was a successful qocb_lindblad_forward
+    Buf<double2> H0, Aops, Lops, Khalf, Kops, rho0, mats, states, tape_y, tape_k1, work, seeds;
     Buf<double> gam, controls, xs, cost, tape_x, tape_h, grad, series, tseen;
     Buf<int> counts, first, hit, err_flag;
     Buf<long long> stats;
@@ -619,7 +631,7 @@ LArgs make_largs(qocb_lplan *p) {
     a.tape_k1 = p->tape_k1.p; a.first = p->first.p; a.hit = p->hit.p; a.stats = p->stats.p; a.err_flag = p->err_flag.p;
     a.work = p->work.p; a.work_in_smem = 0; a.ops_in_smem = p->ops_in_smem; a.grad = p->grad.p;
     a.KC = p->pb.channel_count; a.tdr = p->pb.time_dependent_rates; a.NS = p->NS; a.segs = p->segs; a.deg = p->deg;
-    a.seg_w = p->seg_w; a.series = p->series.p; a.Kops = p->Kops.p; a.tseen = p->tseen.p;
+    a.seg_w = p->seg_w; a.series = p->series.p; a.Kops = p->Kops.p; a.tseen = p->tseen.p; a.seeds = nullptr;
     return a;
 }
 
@@ -637,7 +649,13 @@ int upload_lcosts(qocb_lplan *p) {
     return 0;
 }
 
-int run_lindblad(qocb_lplan *p, const double *controls, bool with_grad, double *cost, double *grad, double *final_densities) {
+int lindblad_threads(const qocb_lplan *p) {
+    const int DEl = p->pb.density_count * p->pb.hilbert_size * p->pb.hilbert_size;
+    return DEl <= 64 ? 32 : (DEl <= 256 ? 128 : LNT);
+}
+
+// enqueues the forward pass (keep_tape: record the reverse-pass tape) after uploading the controls
+int launch_forward(qocb_lplan *p, const double *controls, bool keep_tape) {
     if (!p->ops_set || !p->rho_set) return lfail(p, "operators and densities must be set before evaluation", -1);
     if (p->NS > 0 && !p->series_set) return lfail(p, "time-dependent operators need qocb_lindblad_set_time_series before evaluation", -1);
     LTRY(p, cudaSetDevice(p->pb.device));
@@ -650,16 +668,27 @@ int run_lindblad(qocb_lplan *p, const double *controls, bool with_grad, double *
     LTRY(p, cudaMemsetAsync(p->err_flag.p, 0, sizeof(int), p->stream));
     LArgs a = make_largs(p);
     a.work_in_smem = p->in_smem_fwd;
-    const int DEl = p->pb.density_count * p->pb.hilbert_size * p->pb.hilbert_size;
-    const int nt = DEl <= 64 ? 32 : (DEl <= 256 ? 128 : LNT);
-    if (p->NS > 0) k_lindblad_forward<true><<<1, nt, p->smem_fwd, p->stream>>>(a, with_grad ? 1 : 0);
-    else k_lindblad_forward<false><<<1, nt, p->smem_fwd, p->stream>>>(a, with_grad ? 1 : 0);
-    if (with_grad && cnt) {
-        a.work_in_smem = p->in_smem_bwd;
-        if (p->NS > 0) k_lindblad_backward<true><<<1, nt, p->smem_bwd, p->stream>>>(a);
-        else k_lindblad_backward<false><<<1, nt, p->smem_bwd, p->stream>>>(a);
-    }
+    if (p->NS > 0) k_lindblad_forward<true><<<1, lindblad_threads(p), p->smem_fwd, p->stream>>>(a, keep_tape ? 1 : 0);
+    else k_lindblad_forward<false><<<1, lindblad_threads(p), p->smem_fwd, p->stream>>>(a, keep_tape ? 1 : 0);
     LTRY(p, cudaGetLastError());
+    return 0;
+}
+
+// enqueues the reverse pass over the tape of the last forward pass; seeds: device [N][D*n*n] or null
+int launch_backward(qocb_lplan *p, const double2 *seeds) {
+    LArgs a = make_largs(p);
+    a.work_in_smem = p->in_smem_bwd;
+    a.seeds = seeds;
+    if (p->NS > 0) k_lindblad_backward<true><<<1, lindblad_threads(p), p->smem_bwd, p->stream>>>(a);
+    else k_lindblad_backward<false><<<1, lindblad_threads(p), p->smem_bwd, p->stream>>>(a);
+    LTRY(p, cudaGetLastError());
+    return 0;
+}
+
+// copies the requested results to the host, waits for the stream and reports a stage time beyond the series (-5) or a
+// full tape (-4) of the last forward pass
+int finish_lindblad(qocb_lplan *p, double *cost, double *grad, double *final_densities) {
+    const size_t cnt = (size_t)p->pb.control_eval_count * p->pb.control_count;
     int flag = 0;
     LTRY(p, cudaMemcpyAsync(&flag, p->err_flag.p, sizeof(int), cudaMemcpyDeviceToHost, p->stream));
     if (cost) LTRY(p, cudaMemcpyAsync(cost, p->cost.p, sizeof(double), cudaMemcpyDeviceToHost, p->stream));
@@ -800,6 +829,7 @@ int qocb_lindblad_set_operators(qocb_lplan *p, const double *h0, const double *a
         LTRY(p, cudaMemcpy(p->Khalf.p, kh.data(), sizeof(double2) * nn, cudaMemcpyHostToDevice));
     }
     p->ops_set = true;
+    p->tape_ok = false;
     return 0;
 }
 
@@ -815,6 +845,7 @@ int qocb_lindblad_set_time_series(qocb_lplan *p, int32_t segments, int32_t degre
     LTRY(p, cudaMemcpy(p->series.p, series, sizeof(double) * count, cudaMemcpyHostToDevice));
     p->segs = segments; p->deg = degree; p->seg_w = segment_width;
     p->series_set = true;
+    p->tape_ok = false;
     return 0;
 }
 
@@ -833,6 +864,7 @@ int qocb_lindblad_set_densities(qocb_lplan *p, const double *rho0) {
     const size_t DE = (size_t)p->pb.density_count * p->pb.hilbert_size * p->pb.hilbert_size;
     LTRY(p, cudaMemcpy(p->rho0.p, rho0, sizeof(double2) * DE, cudaMemcpyHostToDevice));
     p->rho_set = true;
+    p->tape_ok = false;
     return 0;
 }
 
@@ -853,17 +885,49 @@ int qocb_lindblad_add_cost(qocb_lplan *p, int32_t kind, int32_t step_cost, doubl
     p->h_mats.insert(p->h_mats.end(), m, m + (size_t)D * fmax * nn);
     p->h_terms.push_back(t);
     p->costs_dirty = true;
+    p->tape_ok = false;
     return 0;
 }
 
 int qocb_lindblad_cost(qocb_lplan *p, const double *controls, double *cost, double *final_densities) {
     if (!p) return -1;
-    return run_lindblad(p, controls, false, cost, nullptr, final_densities);
+    p->tape_ok = false;
+    if (int rc = launch_forward(p, controls, false)) return rc;
+    return finish_lindblad(p, cost, nullptr, final_densities);
 }
 
 int qocb_lindblad_cost_and_grad(qocb_lplan *p, const double *controls, double *cost, double *grad, double *final_densities) {
     if (!p) return -1;
-    return run_lindblad(p, controls, true, cost, grad, final_densities);
+    p->tape_ok = false;
+    if (int rc = launch_forward(p, controls, true)) return rc;
+    if ((size_t)p->pb.control_eval_count * p->pb.control_count)
+        if (int rc = launch_backward(p, nullptr)) return rc;
+    return finish_lindblad(p, cost, grad, final_densities);
+}
+
+int qocb_lindblad_forward(qocb_lplan *p, const double *controls, double *cost, double *final_densities) {
+    if (!p) return -1;
+    p->tape_ok = false;
+    if (int rc = launch_forward(p, controls, true)) return rc;
+    const int rc = finish_lindblad(p, cost, nullptr, final_densities);
+    p->tape_ok = rc == 0;
+    return rc;
+}
+
+/* seeds: [N][D][n][n] complex or NULL; row k is added to the cotangent of the densities at system step k */
+int qocb_lindblad_backward(qocb_lplan *p, const double *seeds, double *grad) {
+    if (!p) return -1;
+    const size_t cnt = (size_t)p->pb.control_eval_count * p->pb.control_count;
+    if (!cnt) return 0;
+    if (!p->tape_ok) return lfail(p, "qocb_lindblad_backward needs a successful qocb_lindblad_forward as the last evaluation", -1);
+    LTRY(p, cudaSetDevice(p->pb.device));
+    if (seeds) {
+        const size_t count = (size_t)p->pb.system_eval_count * p->pb.density_count * p->pb.hilbert_size * p->pb.hilbert_size;
+        if (!p->seeds.p) LTRY(p, p->seeds.alloc(count));
+        LTRY(p, cudaMemcpyAsync(p->seeds.p, seeds, sizeof(double2) * count, cudaMemcpyHostToDevice, p->stream));
+    }
+    if (int rc = launch_backward(p, seeds ? p->seeds.p : nullptr)) return rc;
+    return finish_lindblad(p, nullptr, grad, nullptr);
 }
 
 /* stats[0] = Runge-Kutta attempts, stats[1] = accepted steps of the last evaluation */
