@@ -212,7 +212,15 @@ int qocb_expm_batched_bench(int32_t n, int64_t batch, double norm_scale, int32_t
        controller (qoc/core/mathmethods.py:436-462), whose inputs are error norms taken at the rounding floor; those terms are
        noise (perturbing the controls by 1e-13 moves the reference-equivalent full gradient by 1e-5 .. 1e-4).  The gradient
        returned here matches the reference-equivalent gradient with the step grid frozen within 1e-7 relative, and the full
-       one within its own reproducibility band.  It is NOT claimed at the 1e-10 of the Schroedinger path. */
+       one within its own reproducibility band.  It is NOT claimed at the 1e-10 of the Schroedinger path.
+
+   ENSEMBLES (robust control over drifts and decay rates).  ensemble_count = E > 1 runs E members, one CTA each, in one launch
+   of each kernel.  Members differ in the drift H0 and/or the rates gamma_l (qocb_lindblad_set_ensemble); rho0, control and
+   Lindblad operators, cost terms, controls and the time series are shared.  Every member runs exactly the code and the launch
+   layout of a one-member plan of the same shape, so its results are bit-identical to such a plan built with its drift and
+   rates.  The cost and gradient are the member mean: sums in member order 0..E-1 divided by E (no atomics).  Each member has
+   its own tape of max_rk_steps steps (0: max(4096, min(2^20, 8 GiB / (E * 2 * D n^2 * 16 B)))); a member whose forward
+   pass fills its tape skips its reverse pass, and the evaluation returns -4. */
 typedef struct qocb_lplan qocb_lplan;
 
 typedef struct {
@@ -228,6 +236,7 @@ typedef struct {
     int32_t max_rk_steps;        /* capacity of the accepted-step tape of one evaluation; 0 = automatic */
     int32_t channel_count;       /* KC in [0, 16]: time-dependent hamiltonian channels; 0 = time-independent H0 + x.A */
     int32_t time_dependent_rates;/* 0 or 1 (needs lindblad_count >= 1) */
+    int32_t ensemble_count;      /* E members; 0 or 1: one member (no ensemble) */
     double evolution_time;
 } qocb_lindblad_problem;
 
@@ -240,17 +249,24 @@ const char *qocb_lindblad_last_error(const qocb_lplan *plan);
 /* h0: [n][n] (NULL without hamiltonian); a_ops: [KR][n][n]; gammas: [L]; lops: [L][n][n] */
 int qocb_lindblad_set_operators(qocb_lplan *plan, const double *h0, const double *a_ops, const double *gammas,
                                 const double *lops);
+/* Members of an ensemble plan (E > 1), required before its first evaluation and again after qocb_lindblad_set_operators:
+   h0s [E][n][n] (NULL: every member takes the h0 of qocb_lindblad_set_operators; needs have_hamiltonian = 1 and
+   channel_count = 0), gammas [E][L] (NULL: every member takes the plan's; needs time_dependent_rates = 0).  Member e's
+   1/2 sum_l gamma_el L_l^dag L_l is built on the host as qocb_lindblad_set_operators builds it.  Returns -1 on E <= 1. */
+int qocb_lindblad_set_ensemble(qocb_lplan *plan, const double *h0s, const double *gammas);
 /* series: [segments][degree+1][NS] Chebyshev coefficients per segment [s w, (s+1) w] (constant term not halved);
    degree <= 64; may be called again to replace the table */
 int qocb_lindblad_set_time_series(qocb_lplan *plan, int32_t segments, int32_t degree, double segment_width,
                                   const double *series);
-/* largest stage time of the last forward pass (plans with a series); an evaluation returns -5 when it lies beyond the table */
+/* largest stage time of the last forward pass (plans with a series; the maximum over the members of an ensemble); an
+   evaluation returns -5 when it lies beyond the table */
 int qocb_lindblad_max_stage_time(qocb_lplan *plan, double *t);
 int qocb_lindblad_set_densities(qocb_lplan *plan, const double *rho0);
 /* mats: [D][fmax][n][n]; counts: [D] or NULL; weight = cost_multiplier / normalisation; step_cost as above */
 int qocb_lindblad_add_cost(qocb_lplan *plan, int32_t kind, int32_t step_cost, double weight, const double *mats,
                            const int32_t *counts, int32_t fmax);
-/* controls: [M][KR]; final_densities: [D][n][n] or NULL; grad: [M][KR] */
+/* controls: [M][KR]; final_densities: [D][n][n] or NULL; grad: [M][KR].  Ensemble: member-mean cost and gradient, and
+   final_densities [E][D][n][n] */
 int qocb_lindblad_cost(qocb_lplan *plan, const double *controls, double *cost, double *final_densities);
 int qocb_lindblad_cost_and_grad(qocb_lplan *plan, const double *controls, double *cost, double *grad,
                                 double *final_densities);
@@ -267,12 +283,16 @@ int qocb_lindblad_cost_and_grad(qocb_lplan *plan, const double *controls, double
    TAPE RULE: qocb_lindblad_backward needs a qocb_lindblad_forward that returned 0 as the plan's last evaluation, with no
    setter in between (qocb_lindblad_cost and qocb_lindblad_cost_and_grad overwrite the densities without that tape);
    otherwise it returns -1.  It may be called more than once on one tape.  With control_count = 0 it writes nothing and
-   returns 0.  The seed buffer is allocated on first use: plans that never pass seeds allocate nothing for it. */
+   returns 0.  The seed buffer is allocated on first use: plans that never pass seeds allocate nothing for it.
+   Both return -1 on an ensemble plan. */
 int qocb_lindblad_forward(qocb_lplan *plan, const double *controls, double *cost, double *final_densities);
 int qocb_lindblad_backward(qocb_lplan *plan, const double *seeds, double *grad);
-/* stats[0] = Runge-Kutta attempts, stats[1] = accepted steps of the last evaluation */
+/* stats[0] = Runge-Kutta attempts, stats[1] = accepted steps of the last evaluation (sums over the members of an ensemble) */
 int qocb_lindblad_stats(qocb_lplan *plan, int64_t *stats);
-/* densities at every system step of the last evaluation: [N][D][n][n] (save_intermediate_densities payload) */
+/* each member's results of the last evaluation: costs [E], grads [E][M][KR], stats [E][2]; any may be NULL */
+int qocb_lindblad_member_results(qocb_lplan *plan, double *costs, double *grads, int64_t *stats);
+/* densities at every system step of the last evaluation: [N][D][n][n] (save_intermediate_densities payload); [E][N][D][n][n]
+   for an ensemble */
 int qocb_lindblad_get_densities(qocb_lplan *plan, double *densities);
 
 const char *qocb_version(void);

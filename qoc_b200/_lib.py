@@ -30,7 +30,8 @@ EXPORTS = [
     "qocb_lindblad_create", "qocb_lindblad_destroy", "qocb_lindblad_last_error",
     "qocb_lindblad_set_operators", "qocb_lindblad_set_densities", "qocb_lindblad_add_cost", "qocb_lindblad_cost",
     "qocb_lindblad_cost_and_grad", "qocb_lindblad_stats", "qocb_lindblad_get_densities", "qocb_lindblad_set_time_series",
-    "qocb_lindblad_max_stage_time", "qocb_lindblad_forward", "qocb_lindblad_backward",
+    "qocb_lindblad_max_stage_time", "qocb_lindblad_forward", "qocb_lindblad_backward", "qocb_lindblad_set_ensemble",
+    "qocb_lindblad_member_results",
 ]
 
 
@@ -50,7 +51,7 @@ class LindbladProblem(C.Structure):
                 ("control_eval_count", C.c_int32), ("system_eval_count", C.c_int32), ("cost_eval_step", C.c_int32),
                 ("lindblad_count", C.c_int32), ("have_hamiltonian", C.c_int32), ("device", C.c_int32),
                 ("max_rk_steps", C.c_int32), ("channel_count", C.c_int32), ("time_dependent_rates", C.c_int32),
-                ("evolution_time", C.c_double)]
+                ("ensemble_count", C.c_int32), ("evolution_time", C.c_double)]
 
 
 def sources():
@@ -151,6 +152,8 @@ def load():
     lib.qocb_lindblad_get_densities.argtypes = [vp, vp]
     lib.qocb_lindblad_set_time_series.argtypes = [vp, i32, i32, dbl, vp]
     lib.qocb_lindblad_max_stage_time.argtypes = [vp, vp]
+    lib.qocb_lindblad_set_ensemble.argtypes = [vp, vp, vp]
+    lib.qocb_lindblad_member_results.argtypes = [vp, vp, vp, vp]
     lib.qocb_flush_l2.argtypes = [vp]
     lib.qocb_shard_matrix_doubles.argtypes = [vp]
     lib.qocb_shard_vector_doubles.argtypes = [vp]

@@ -969,11 +969,17 @@ class LindbladPlan(object):
 
     Gradient semantics: the discrete adjoint of the Dormand-Prince map on the realised (accepted) step grid.  The
     reference's autograd tape also differentiates the step-size controller; those terms are rounding noise (see
-    oracle/lindblad_adjoint_model.py and DESIGN.md section 5) and are deliberately not reproduced."""
+    oracle/lindblad_adjoint_model.py and DESIGN.md section 5) and are deliberately not reproduced.
+
+    Ensembles (robust control): `ensemble_drifts` [E][n][n] replaces the drift of `hamiltonian` and `ensemble_rates` [E][L]
+    the decay rates of `lindblad_data`, member by member.  `cost` and `cost_and_grad` then return the member mean (control
+    costs added once) with final densities [E][D][n][n], `intermediate_densities()` is [E][N][D][n][n] and `member_results()`
+    returns every member's cost, gradient and stats.  One member is the plain plan."""
 
     def __init__(self, initial_densities, costs, evolution_time, system_eval_count, hamiltonian=None,
                  lindblad_data=None, control_eval_count=0, control_count=0, complex_controls=False, cost_eval_step=1,
-                 interpolation_policy=InterpolationPolicy.LINEAR, device=0, max_rk_steps=0, structure=None):
+                 interpolation_policy=InterpolationPolicy.LINEAR, device=0, max_rk_steps=0, structure=None,
+                 ensemble_drifts=None, ensemble_rates=None):
         if interpolation_policy != InterpolationPolicy.LINEAR:
             raise ValueError("The interpolation policy {} is not implemented for this method."
                              "".format(interpolation_policy))
@@ -1013,6 +1019,14 @@ class LindbladPlan(object):
         if h0 is not None and h0.shape[0] != self.n:
             raise ValueError("hamiltonian size {} does not match the densities' hilbert size {}".format(h0.shape[0], self.n))
         self.L = 0 if lops is None else lops.shape[0]
+        h0s, rates = self._ensemble_members(ensemble_drifts, ensemble_rates, td_h, td_l)
+        self.E = 1 if h0s is None and rates is None else (h0s if h0s is not None else rates).shape[0]
+        if self.E == 1:                                  # one member: the plain plan with that member's drift and rates
+            h0 = h0 if h0s is None else h0s[0]
+            gammas = gammas if rates is None else rates[0]
+            h0s = rates = None
+        self._members = (h0s, rates)
+        self._last_extra = (0.0, None)
         self.range_extensions = 0
         self._setup = dict(rho0=rho0, h0=h0, a_ops=a_ops, gammas=gammas, lops=lops, cost_eval_step=int(cost_eval_step),
                            device=int(device), max_rk_steps=int(max_rk_steps))
@@ -1049,8 +1063,37 @@ class LindbladPlan(object):
             for k in (range(ces, self.N, ces) if getattr(c, "requires_step_evaluation", False) else (self.N - 1,)):
                 self._user_at.setdefault(k, []).append(c)
 
+    def _ensemble_members(self, drifts, rates, td_h, td_l):
+        """validated member drifts [E][n][n] and rates [E][L] (either may be None); raises before any device call."""
+        if drifts is None and rates is None:
+            return None, None
+        if any(is_user_cost(c) for c in self.costs):
+            raise NotImplementedError("user-defined costs cannot be combined with ensembles")
+        if drifts is not None:
+            if not self.have_h:
+                raise ValueError("ensemble_drifts replace the drift of `hamiltonian`, which is None")
+            if td_h:
+                raise NotImplementedError("ensemble drifts with a time-dependent hamiltonian are not supported")
+            drifts = np.ascontiguousarray(drifts, dtype=np.complex128)
+            if drifts.ndim != 3 or drifts.shape[0] < 1 or drifts.shape[1:] != (self.n, self.n):
+                raise ValueError("ensemble_drifts must have shape [E][{0}][{0}], got {1}".format(self.n, drifts.shape))
+        if rates is not None:
+            if self.L == 0:
+                raise ValueError("ensemble_rates replace the rates of `lindblad_data`, which has no operators")
+            if td_l:
+                raise NotImplementedError("ensemble rates with a time-dependent lindblad_data are not supported")
+            if np.iscomplexobj(rates):
+                raise ValueError("ensemble_rates must be real")
+            rates = np.ascontiguousarray(rates, dtype=np.float64)
+            if rates.ndim != 2 or rates.shape[0] < 1 or rates.shape[1] != self.L:
+                raise ValueError("ensemble_rates must have shape [E][{}], got {}".format(self.L, rates.shape))
+        if drifts is not None and rates is not None and drifts.shape[0] != rates.shape[0]:
+            raise ValueError("ensemble_drifts has {} members and ensemble_rates {}".format(drifts.shape[0], rates.shape[0]))
+        return drifts, rates
+
     def _open(self):
-        """creates the device plan and uploads operators, densities and (time-dependent problems) the series table."""
+        """creates the device plan and uploads operators, densities, the ensemble members and (time-dependent problems) the
+        series table."""
         su, st = self._setup, self.series
         KC = st.KC if st is not None and self._td[0] is not None else 0
         tdr = int(st is not None and self._td[1] is not None)
@@ -1058,7 +1101,8 @@ class LindbladPlan(object):
                                   control_eval_count=self.M if self.KR else 0, system_eval_count=self.N,
                                   cost_eval_step=su["cost_eval_step"], lindblad_count=self.L,
                                   have_hamiltonian=int(self.have_h), device=su["device"], max_rk_steps=su["max_rk_steps"],
-                                  channel_count=KC, time_dependent_rates=tdr, evolution_time=self.T)
+                                  channel_count=KC, time_dependent_rates=tdr,
+                                  ensemble_count=self.E if self.E > 1 else 0, evolution_time=self.T)
         handle = ctypes.c_void_p()
         rc = self.lib.qocb_lindblad_create(ctypes.byref(pb), ctypes.byref(handle))
         if rc != 0:
@@ -1071,6 +1115,8 @@ class LindbladPlan(object):
         lops = None if su["lops"] is None else np.ascontiguousarray(su["lops"], dtype=np.complex128)
         self._check(self.lib.qocb_lindblad_set_operators(handle, _lib.ptr(h0c), _lib.ptr(aoc), _lib.ptr(su["gammas"]),
                                                          _lib.ptr(lops)))
+        if self.E > 1:
+            self._check(self.lib.qocb_lindblad_set_ensemble(handle, _lib.ptr(self._members[0]), _lib.ptr(self._members[1])))
         self._check(self.lib.qocb_lindblad_set_densities(handle, _lib.ptr(su["rho0"])))
         if st is not None:
             self._check(self.lib.qocb_lindblad_set_time_series(handle, st.segments, st.degree, st.width, _lib.ptr(st.series)))
@@ -1139,15 +1185,20 @@ class LindbladPlan(object):
             seeds[k] = dre - 1j * dim
         return seeds
 
+    def _final_buffer(self):
+        shape = (self.D, self.n, self.n) if self.E == 1 else (self.E, self.D, self.n, self.n)
+        return np.empty(shape, dtype=np.complex128)
+
     def cost(self, controls):
         x = self._real_channels(controls) if controls is not None else None
         out = np.zeros(1)
-        fd = np.empty((self.D, self.n, self.n), dtype=np.complex128)
+        fd = self._final_buffer()
         self._evaluate(lambda h: self.lib.qocb_lindblad_cost(h, _lib.ptr(x), _lib.ptr(out), _lib.ptr(fd)))
         value = float(out[0])
         if self.user_costs:
             value += self._user_value(controls, self._user_densities(fd))
         extra, _ = self._control_costs(controls, False) if controls is not None else (0.0, None)
+        self._last_extra = (extra, None)
         return value + extra, fd
 
     def cost_and_grad(self, controls):
@@ -1156,7 +1207,7 @@ class LindbladPlan(object):
         their numeric cotangents (qocb_lindblad_forward / qocb_lindblad_backward)."""
         x = self._real_channels(controls)
         out = np.zeros(1)
-        fd = np.empty((self.D, self.n, self.n), dtype=np.complex128)
+        fd = self._final_buffer()
         controls = np.asarray(controls)
         g = np.zeros((self.M, self.KR))
         if self.KR == 0:                                   # hamiltonian = None: the densities do not see the controls
@@ -1174,16 +1225,43 @@ class LindbladPlan(object):
                 self._check(self.lib.qocb_lindblad_backward(self.handle, _lib.ptr(seeds), _lib.ptr(g)))
             if controls.ndim:
                 user_grad = explicit_control_grad(lambda u: self._user_value(u, dens), controls)
-        if self.KR == 0:
-            grads = np.zeros(controls.shape, dtype=controls.dtype)
-        else:
-            grads = g[:, :self.K] + 1j * g[:, self.K:] if self.complex_controls else g
+        grads = self._controls_grad(g, controls)
         if user_grad is not None:
             grads = grads + user_grad
         extra, extra_grad = self._control_costs(controls, True)
+        self._last_extra = (extra, (controls.shape, controls.dtype, extra_grad))
         if extra_grad is not None:
             grads = grads + extra_grad
         return value + extra, grads, fd
+
+    def _controls_grad(self, g, controls):
+        """dE/dRe u + i dE/dIm u in the controls' shape from the device gradient [M][KR]."""
+        if self.KR == 0:
+            return np.zeros(controls.shape, dtype=controls.dtype)
+        return g[:, :self.K] + 1j * g[:, self.K:] if self.complex_controls else g
+
+    def member_results(self):
+        """every member's (cost, gradient, stats) of the last evaluation: costs [E], gradients [E] in the controls' shape and
+        dtype (None after `cost`), stats [E] as {"attempts", "accepted"}; the control costs are included in each member's
+        cost and gradient, so member e equals a one-member plan built with its drift and rates (and the same control
+        operators)."""
+        costs = np.zeros(self.E)
+        g = np.zeros((self.E, self.M, self.KR))
+        st = np.zeros((self.E, 2), dtype=np.int64)
+        self._check(self.lib.qocb_lindblad_member_results(self.handle, _lib.ptr(costs), _lib.ptr(g),
+                                                          st.ctypes.data_as(ctypes.c_void_p)))
+        extra, grad_info = self._last_extra
+        costs = costs + extra
+        grads = None
+        if grad_info is not None:
+            shape, dtype, extra_grad = grad_info
+            zero = np.zeros(shape, dtype=dtype)
+            grads = []
+            for e in range(self.E):
+                ge = self._controls_grad(g[e], zero)
+                grads.append(ge + extra_grad if extra_grad is not None else ge)
+            grads = np.array(grads)
+        return costs, grads, [{"attempts": int(a), "accepted": int(b)} for a, b in st]
 
     def stats(self):
         s = np.zeros(2, dtype=np.int64)
@@ -1191,7 +1269,8 @@ class LindbladPlan(object):
         return {"attempts": int(s[0]), "accepted": int(s[1])}
 
     def intermediate_densities(self):
-        buf = np.empty((self.N, self.D, self.n, self.n), dtype=np.complex128)
+        shape = (self.N, self.D, self.n, self.n)
+        buf = np.empty(shape if self.E == 1 else (self.E,) + shape, dtype=np.complex128)
         self._check(self.lib.qocb_lindblad_get_densities(self.handle, _lib.ptr(buf)))
         return buf
 

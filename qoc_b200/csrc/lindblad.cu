@@ -14,6 +14,10 @@
 // hand-derived adjoint of the RK map, the dense output and the FSAL coupling on the realised grid
 // (oracle/lindblad_adjoint_model.py is the NumPy statement of the same algebra and explains, with measurements,
 // why the step-size controller itself is not differentiated).
+//
+// An ensemble plan (robust control over drifts and rates) launches E such CTAs at once: CTA e is member e and runs exactly
+// the code of a one-member plan on its own drift, rates, densities, tape and result slots (member_args); a small kernel
+// then forms the member mean in member order.
 #include <algorithm>
 #include <cmath>
 #include <cstdio>
@@ -78,6 +82,22 @@ struct LArgs {
     double *tseen;                              // largest stage time of the forward pass
     const double2 *seeds;                       // [N][D*n*n] host-cost cotangents of the densities, or null
 };
+
+// the arguments of ensemble member blockIdx.x: per-member drift, K_half, rates, densities, tape, interval indices, global
+// work, cost, gradient, stats, stage time and tape-overflow flag sit at member-major offsets; rho0, operators, cost terms,
+// controls and the time series are shared.  Member 0 is the whole plan when E = 1.
+__device__ __forceinline__ LArgs member_args(const LArgs &a0) {
+    LArgs a = a0;
+    const size_t e = blockIdx.x, nn = (size_t)a.n * a.n, DE = (size_t)a.D * nn;
+    a.H0 += e * nn; a.Khalf += e * nn; a.gam += e * (size_t)max(a.L, 1);
+    a.states += e * a.N * DE;
+    a.tape_x += e * a.cap; a.tape_h += e * a.cap; a.tape_y += e * a.cap * DE; a.tape_k1 += e * a.cap * DE;
+    a.first += e * a.N; a.hit += e * a.N;
+    if (!a.work_in_smem) a.work += e * 24 * DE;
+    a.cost += e; a.grad += e * (size_t)a.M * a.KR; a.stats += 2 * e; a.err_flag += e;
+    if (a.tseen) a.tseen += e;
+    return a;
+}
 
 // block-wide sum, result in all threads
 __device__ double block_sum(double v, double *red) {
@@ -394,11 +414,11 @@ template <bool TD> __device__ void carve(const LArgs &a, unsigned char *smem, Ct
             d += (count + 1) & ~1;
             return dst;
         };
-        c.H0 = reinterpret_cast<const double2 *>(stage(reinterpret_cast<const double *>(a.H0), 2 * nn));
-        c.Khalf = reinterpret_cast<const double2 *>(stage(reinterpret_cast<const double *>(a.Khalf), 2 * nn));
+        c.H0 = reinterpret_cast<const double2 *>(stage(reinterpret_cast<const double *>(c.H0), 2 * nn));
+        c.Khalf = reinterpret_cast<const double2 *>(stage(reinterpret_cast<const double *>(c.Khalf), 2 * nn));
         c.Aops = reinterpret_cast<const double2 *>(stage(reinterpret_cast<const double *>(a.Aops), 2 * nn * max(max(a.KR, a.KC), 1)));
         c.Lops = reinterpret_cast<const double2 *>(stage(reinterpret_cast<const double *>(a.Lops), 2 * nn * max(a.L, 1)));
-        c.gam = stage(a.gam, max(a.L, 1));
+        c.gam = stage(c.gam, max(a.L, 1));
         c.controls = stage(a.controls, max(a.M * a.KR, 1));
         c.xs = stage(a.xs, max(a.M, 1));
         if (TD && a.tdr) c.Kops = reinterpret_cast<const double2 *>(stage(reinterpret_cast<const double *>(a.Kops), 2 * nn * a.L));
@@ -410,8 +430,9 @@ template <bool TD> __device__ void carve(const LArgs &a, unsigned char *smem, Ct
     for (int i = 0; i < narr; ++i) w.p[i] = base + (size_t)(i + 1) * DE;
 }
 
-template <bool TD> __global__ void __launch_bounds__(LNT) k_lindblad_forward(LArgs a, int keep_tape) {
+template <bool TD> __global__ void __launch_bounds__(LNT) k_lindblad_forward(LArgs a0, int keep_tape) {
     extern __shared__ __align__(16) unsigned char smem[];
+    const LArgs a = member_args(a0);
     Ctx c(a);
     Work w;
     carve<TD>(a, smem, c, w, 12);
@@ -499,10 +520,12 @@ template <bool TD> __global__ void __launch_bounds__(LNT) k_lindblad_forward(LAr
     if (threadIdx.x == 0) { *a.cost = cost; a.stats[0] = attempts; a.stats[1] = accepted; if (TD) *a.tseen = c.tseen; }
 }
 
-template <bool TD> __global__ void __launch_bounds__(LNT) k_lindblad_backward(LArgs a) {
+template <bool TD> __global__ void __launch_bounds__(LNT) k_lindblad_backward(LArgs a0) {
     extern __shared__ __align__(16) unsigned char smem[];
+    const LArgs a = member_args(a0);
     Ctx c(a);
     Work w;
+    if (*a.err_flag) return;                          // the forward pass overflowed this member's tape: hit[] is not valid
     if (TD && *a.tseen > a.segs * a.seg_w) return;    // the forward pass left the table: it is run again
     carve<TD>(a, smem, c, w, 22);
     const int DE = a.D * a.n * a.n;
@@ -580,6 +603,27 @@ template <bool TD> __global__ void __launch_bounds__(LNT) k_lindblad_backward(LA
     }
 }
 
+// member mean of an ensemble: cost and gradient summed in member order 0..E-1 and divided by E, largest stage time
+// over members (deterministic: no atomics).  Thread j < cnt owns gradient entry j; thread cnt the cost and stage time.
+__global__ void k_lindblad_member_mean(int E, int cnt, const double *cost, const double *grad, const double *tseen,
+                                       double *cost_mean, double *grad_mean, double *tseen_max) {
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j < cnt) {
+        double s = 0.;
+        for (int e = 0; e < E; ++e) s += grad[(size_t)e * cnt + j];
+        grad_mean[j] = s / E;
+    } else if (j == cnt) {
+        double s = 0.;
+        for (int e = 0; e < E; ++e) s += cost[e];
+        *cost_mean = s / E;
+        if (tseen) {
+            double t = tseen[0];
+            for (int e = 1; e < E; ++e) t = fmax(t, tseen[e]);
+            *tseen_max = t;
+        }
+    }
+}
+
 thread_local std::string g_lerr;
 
 template <class T> struct Buf {
@@ -599,18 +643,21 @@ template <class T> struct Buf {
 
 struct qocb_lplan {
     qocb_lindblad_problem pb;
-    int cap = 0;
+    int E = 1;                                     // ensemble members (one CTA each)
+    bool ens_set = false;                          // qocb_lindblad_set_ensemble since the last qocb_lindblad_set_operators
+    int cap = 0;                                   // tape capacity of one member
     bool ops_set = false, rho_set = false, costs_dirty = true, series_set = false;
     int NS = 0, segs = 0, deg = 0;                 // time series: NS = KC*(1+KR) + (time_dependent_rates ? L : 0)
     double seg_w = 0.;
     cudaStream_t stream = nullptr;
     bool tape_ok = false;                          // the last evaluation was a successful qocb_lindblad_forward
     Buf<double2> H0, Aops, Lops, Khalf, Kops, rho0, mats, states, tape_y, tape_k1, work, seeds;
-    Buf<double> gam, controls, xs, cost, tape_x, tape_h, grad, series, tseen;
+    Buf<double> gam, controls, xs, cost, tape_x, tape_h, grad, series, tseen, cost_mean, grad_mean, tseen_max;
     Buf<int> counts, first, hit, err_flag;
     Buf<long long> stats;
     Buf<DTerm> terms;
     std::vector<DTerm> h_terms; std::vector<double2> h_mats; std::vector<int> h_counts;
+    std::vector<double> h_h0, h_gam, h_lops;       // the plan's operators (E > 1): members without their own take these
     size_t smem_fwd = 0, smem_bwd = 0;
     int in_smem_fwd = 0, in_smem_bwd = 0, ops_in_smem = 0;
     std::string err;
@@ -633,6 +680,25 @@ LArgs make_largs(qocb_lplan *p) {
     a.KC = p->pb.channel_count; a.tdr = p->pb.time_dependent_rates; a.NS = p->NS; a.segs = p->segs; a.deg = p->deg;
     a.seg_w = p->seg_w; a.series = p->series.p; a.Kops = p->Kops.p; a.tseen = p->tseen.p; a.seeds = nullptr;
     return a;
+}
+
+// kh += 1/2 sum_l gammas_l L_l^dag L_l, or the per-operator 1/2 L_l^dag L_l into kh + l n^2 when gammas is null
+void build_khalf(const double *lops, const double *gammas, int n, int L, double *kh) {
+    const size_t nn = (size_t)n * n;
+    for (int l = 0; l < L; ++l) {
+        const double *Lm = lops + 2 * (size_t)l * nn;
+        double *K = gammas ? kh : kh + 2 * (size_t)l * nn;
+        for (int i = 0; i < n; ++i)
+            for (int j = 0; j < n; ++j) {
+                double sr = 0., si = 0.;
+                for (int k = 0; k < n; ++k) {                             // conj(L[k][i]) * L[k][j]
+                    const double ar = Lm[2 * (k * n + i)], ai = -Lm[2 * (k * n + i) + 1], br = Lm[2 * (k * n + j)], bi = Lm[2 * (k * n + j) + 1];
+                    sr += ar * br - ai * bi; si += ar * bi + ai * br;
+                }
+                if (gammas) { K[2 * (i * n + j)] += 0.5 * gammas[l] * sr; K[2 * (i * n + j) + 1] += 0.5 * gammas[l] * si; }
+                else { K[2 * (i * n + j)] = 0.5 * sr; K[2 * (i * n + j) + 1] = 0.5 * si; }
+            }
+    }
 }
 
 int upload_lcosts(qocb_lplan *p) {
@@ -658,6 +724,7 @@ int lindblad_threads(const qocb_lplan *p) {
 int launch_forward(qocb_lplan *p, const double *controls, bool keep_tape) {
     if (!p->ops_set || !p->rho_set) return lfail(p, "operators and densities must be set before evaluation", -1);
     if (p->NS > 0 && !p->series_set) return lfail(p, "time-dependent operators need qocb_lindblad_set_time_series before evaluation", -1);
+    if (p->E > 1 && !p->ens_set) return lfail(p, "an ensemble plan needs qocb_lindblad_set_ensemble after qocb_lindblad_set_operators", -1);
     LTRY(p, cudaSetDevice(p->pb.device));
     if (upload_lcosts(p)) return -2;
     const size_t cnt = (size_t)p->pb.control_eval_count * p->pb.control_count;
@@ -665,11 +732,11 @@ int launch_forward(qocb_lplan *p, const double *controls, bool keep_tape) {
         if (!controls) return lfail(p, "controls is null", -1);
         LTRY(p, cudaMemcpyAsync(p->controls.p, controls, sizeof(double) * cnt, cudaMemcpyHostToDevice, p->stream));
     }
-    LTRY(p, cudaMemsetAsync(p->err_flag.p, 0, sizeof(int), p->stream));
+    LTRY(p, cudaMemsetAsync(p->err_flag.p, 0, sizeof(int) * p->E, p->stream));
     LArgs a = make_largs(p);
     a.work_in_smem = p->in_smem_fwd;
-    if (p->NS > 0) k_lindblad_forward<true><<<1, lindblad_threads(p), p->smem_fwd, p->stream>>>(a, keep_tape ? 1 : 0);
-    else k_lindblad_forward<false><<<1, lindblad_threads(p), p->smem_fwd, p->stream>>>(a, keep_tape ? 1 : 0);
+    if (p->NS > 0) k_lindblad_forward<true><<<p->E, lindblad_threads(p), p->smem_fwd, p->stream>>>(a, keep_tape ? 1 : 0);
+    else k_lindblad_forward<false><<<p->E, lindblad_threads(p), p->smem_fwd, p->stream>>>(a, keep_tape ? 1 : 0);
     LTRY(p, cudaGetLastError());
     return 0;
 }
@@ -679,30 +746,45 @@ int launch_backward(qocb_lplan *p, const double2 *seeds) {
     LArgs a = make_largs(p);
     a.work_in_smem = p->in_smem_bwd;
     a.seeds = seeds;
-    if (p->NS > 0) k_lindblad_backward<true><<<1, lindblad_threads(p), p->smem_bwd, p->stream>>>(a);
-    else k_lindblad_backward<false><<<1, lindblad_threads(p), p->smem_bwd, p->stream>>>(a);
+    if (p->NS > 0) k_lindblad_backward<true><<<p->E, lindblad_threads(p), p->smem_bwd, p->stream>>>(a);
+    else k_lindblad_backward<false><<<p->E, lindblad_threads(p), p->smem_bwd, p->stream>>>(a);
+    LTRY(p, cudaGetLastError());
+    return 0;
+}
+
+// enqueues the member mean of an ensemble evaluation (E > 1); with_grad: the reverse pass ran
+int launch_mean(qocb_lplan *p, bool with_grad) {
+    const int cnt = with_grad ? p->pb.control_eval_count * p->pb.control_count : 0;
+    k_lindblad_member_mean<<<cnt / 256 + 1, 256, 0, p->stream>>>(p->E, cnt, p->cost.p, p->grad.p, p->NS > 0 ? p->tseen.p : nullptr,
+                                                               p->cost_mean.p, p->grad_mean.p, p->tseen_max.p);
     LTRY(p, cudaGetLastError());
     return 0;
 }
 
 // copies the requested results to the host, waits for the stream and reports a stage time beyond the series (-5) or a
-// full tape (-4) of the last forward pass
+// full tape (-4) of the last forward pass.  An ensemble returns the member mean, every member's final densities [E][D][n][n],
+// the largest stage time over members and -4 when any member's tape overflowed.
 int finish_lindblad(qocb_lplan *p, double *cost, double *grad, double *final_densities) {
     const size_t cnt = (size_t)p->pb.control_eval_count * p->pb.control_count;
-    int flag = 0;
-    LTRY(p, cudaMemcpyAsync(&flag, p->err_flag.p, sizeof(int), cudaMemcpyDeviceToHost, p->stream));
-    if (cost) LTRY(p, cudaMemcpyAsync(cost, p->cost.p, sizeof(double), cudaMemcpyDeviceToHost, p->stream));
-    if (grad && cnt) LTRY(p, cudaMemcpyAsync(grad, p->grad.p, sizeof(double) * cnt, cudaMemcpyDeviceToHost, p->stream));
-    const size_t DE = (size_t)p->pb.density_count * p->pb.hilbert_size * p->pb.hilbert_size;
-    if (final_densities)
-        LTRY(p, cudaMemcpyAsync(final_densities, p->states.p + (size_t)(p->pb.system_eval_count - 1) * DE, sizeof(double2) * DE,
+    const bool ens = p->E > 1;
+    std::vector<int> flags(p->E, 0);
+    LTRY(p, cudaMemcpyAsync(flags.data(), p->err_flag.p, sizeof(int) * p->E, cudaMemcpyDeviceToHost, p->stream));
+    if (cost) LTRY(p, cudaMemcpyAsync(cost, ens ? p->cost_mean.p : p->cost.p, sizeof(double), cudaMemcpyDeviceToHost, p->stream));
+    if (grad && cnt) LTRY(p, cudaMemcpyAsync(grad, ens ? p->grad_mean.p : p->grad.p, sizeof(double) * cnt, cudaMemcpyDeviceToHost, p->stream));
+    const size_t DE = (size_t)p->pb.density_count * p->pb.hilbert_size * p->pb.hilbert_size, N = p->pb.system_eval_count;
+    if (final_densities && !ens)
+        LTRY(p, cudaMemcpyAsync(final_densities, p->states.p + (N - 1) * DE, sizeof(double2) * DE,
                                 cudaMemcpyDeviceToHost, p->stream));
+    if (final_densities && ens)                                  // row N-1 of every member's [N][DE] block
+        LTRY(p, cudaMemcpy2DAsync(final_densities, sizeof(double2) * DE, p->states.p + (N - 1) * DE, sizeof(double2) * N * DE,
+                                  sizeof(double2) * DE, p->E, cudaMemcpyDeviceToHost, p->stream));
     double tseen = 0.;
-    if (p->NS > 0) LTRY(p, cudaMemcpyAsync(&tseen, p->tseen.p, sizeof(double), cudaMemcpyDeviceToHost, p->stream));
+    if (p->NS > 0) LTRY(p, cudaMemcpyAsync(&tseen, ens ? p->tseen_max.p : p->tseen.p, sizeof(double), cudaMemcpyDeviceToHost, p->stream));
     LTRY(p, cudaStreamSynchronize(p->stream));
     if (p->NS > 0 && tseen > p->segs * p->seg_w)
         return lfail(p, "a Runge-Kutta stage time lies beyond the time series: extend it (qocb_lindblad_max_stage_time)", -5);
-    if (flag) return lfail(p, "the Runge-Kutta tape is full: raise max_rk_steps", -4);
+    for (int f : flags)
+        if (f) return lfail(p, "the Runge-Kutta tape is full: raise max_rk_steps", -4);
     return 0;
 }
 
@@ -724,6 +806,7 @@ int qocb_lindblad_create(const qocb_lindblad_problem *pb, qocb_lplan **out) {
     if (pb->channel_count > 0 && !pb->have_hamiltonian) return lfail(nullptr, "channel_count > 0 needs have_hamiltonian", -1);
     if (pb->time_dependent_rates != 0 && (pb->time_dependent_rates != 1 || pb->lindblad_count < 1))
         return lfail(nullptr, "time_dependent_rates must be 0 or 1, and 1 needs lindblad_count >= 1", -1);
+    if (pb->ensemble_count < 0) return lfail(nullptr, "ensemble_count must be >= 0", -1);
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return lfail(nullptr, "no CUDA device available (this library has no CPU path)", -2);
     qocb_lplan *p = new qocb_lplan();
@@ -734,17 +817,24 @@ int qocb_lindblad_create(const qocb_lindblad_problem *pb, qocb_lplan **out) {
     const int n = pb->hilbert_size, nn = n * n, D = pb->density_count, KR = pb->control_count, M = pb->control_eval_count;
     const int N = pb->system_eval_count, L = pb->lindblad_count, KC = pb->channel_count, tdr = pb->time_dependent_rates;
     const size_t DE = (size_t)D * nn;
+    const size_t E = p->E = std::max(1, pb->ensemble_count);
     p->NS = KC * (1 + KR) + (tdr ? L : 0);
-    p->cap = pb->max_rk_steps > 0 ? pb->max_rk_steps : (int)std::max<size_t>(4096, std::min<size_t>((size_t)1 << 20, ((size_t)512 << 20) / (2 * DE * sizeof(double2))));
-    CTRY(p->H0.alloc(nn)); CTRY(p->Aops.alloc((size_t)std::max(1, std::max(KR, KC)) * nn)); CTRY(p->Lops.alloc((size_t)std::max(1, L) * nn));
+    // tape of one member: 512 MiB for one member, 8 GiB shared by the members of an ensemble, within [4096, 2^20] steps
+    const size_t tape_bytes = E == 1 ? (size_t)512 << 20 : ((size_t)8 << 30) / E;
+    p->cap = pb->max_rk_steps > 0 ? pb->max_rk_steps : (int)std::max<size_t>(4096, std::min<size_t>((size_t)1 << 20, tape_bytes / (2 * DE * sizeof(double2))));
+    CTRY(p->H0.alloc(E * nn)); CTRY(p->Aops.alloc((size_t)std::max(1, std::max(KR, KC)) * nn)); CTRY(p->Lops.alloc((size_t)std::max(1, L) * nn));
     if (tdr) CTRY(p->Kops.alloc((size_t)L * nn));
-    if (p->NS > 0) { CTRY(p->tseen.alloc(1)); CTRY(cudaMemset(p->tseen.p, 0, sizeof(double))); }
-    CTRY(p->Khalf.alloc(nn)); CTRY(p->gam.alloc(std::max(1, L))); CTRY(p->controls.alloc(std::max<size_t>(1, (size_t)M * KR)));
-    CTRY(p->xs.alloc(std::max(1, M))); CTRY(p->rho0.alloc(DE)); CTRY(p->states.alloc((size_t)N * DE)); CTRY(p->cost.alloc(1));
-    CTRY(p->tape_x.alloc(p->cap)); CTRY(p->tape_h.alloc(p->cap)); CTRY(p->tape_y.alloc((size_t)p->cap * DE)); CTRY(p->tape_k1.alloc((size_t)p->cap * DE));
-    CTRY(p->first.alloc(N)); CTRY(p->hit.alloc(N)); CTRY(p->err_flag.alloc(1)); CTRY(p->stats.alloc(2));
-    CTRY(p->grad.alloc(std::max<size_t>(1, (size_t)M * KR))); CTRY(p->work.alloc(24 * DE));
-    CTRY(cudaMemset(p->H0.p, 0, sizeof(double2) * nn)); CTRY(cudaMemset(p->Khalf.p, 0, sizeof(double2) * nn));
+    if (p->NS > 0) { CTRY(p->tseen.alloc(E)); CTRY(cudaMemset(p->tseen.p, 0, sizeof(double) * E)); }
+    CTRY(p->Khalf.alloc(E * nn)); CTRY(p->gam.alloc(E * std::max(1, L))); CTRY(p->controls.alloc(std::max<size_t>(1, (size_t)M * KR)));
+    CTRY(p->xs.alloc(std::max(1, M))); CTRY(p->rho0.alloc(DE)); CTRY(p->states.alloc(E * N * DE)); CTRY(p->cost.alloc(E));
+    CTRY(p->tape_x.alloc(E * p->cap)); CTRY(p->tape_h.alloc(E * p->cap)); CTRY(p->tape_y.alloc(E * p->cap * DE)); CTRY(p->tape_k1.alloc(E * p->cap * DE));
+    CTRY(p->first.alloc(E * N)); CTRY(p->hit.alloc(E * N)); CTRY(p->err_flag.alloc(E)); CTRY(p->stats.alloc(2 * E));
+    CTRY(p->grad.alloc(E * std::max<size_t>(1, (size_t)M * KR)));
+    if (E > 1) {
+        CTRY(p->cost_mean.alloc(1)); CTRY(p->grad_mean.alloc(std::max<size_t>(1, (size_t)M * KR))); CTRY(p->tseen_max.alloc(1));
+        CTRY(cudaMemset(p->tseen_max.p, 0, sizeof(double)));
+    }
+    CTRY(cudaMemset(p->H0.p, 0, sizeof(double2) * E * nn)); CTRY(cudaMemset(p->Khalf.p, 0, sizeof(double2) * E * nn));
     // control_eval_times = numpy.linspace(0, T, M) (qoc/models/programstate.py:41)
     if (M > 0) {
         std::vector<double> xs(M);
@@ -763,6 +853,7 @@ int qocb_lindblad_create(const qocb_lindblad_problem *pb, qocb_lplan **out) {
     p->in_smem_fwd = need_f <= limit; p->in_smem_bwd = need_b <= limit;
     p->smem_fwd = p->in_smem_fwd ? need_f : fixed; p->smem_bwd = p->in_smem_bwd ? need_b : fixed;
     if (fixed > limit) { g_lerr = "hilbert_size too large for the Lindblad kernels' shared-memory operators"; delete p; return -1; }
+    CTRY(p->work.alloc((p->in_smem_fwd && p->in_smem_bwd ? 1 : E) * 24 * DE));   // one slice per member when it is used
     CTRY(cudaFuncSetAttribute(k_lindblad_forward<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
     CTRY(cudaFuncSetAttribute(k_lindblad_backward<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
     CTRY(cudaFuncSetAttribute(k_lindblad_forward<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
@@ -795,40 +886,55 @@ int qocb_lindblad_set_operators(qocb_lplan *p, const double *h0, const double *a
         if (!lops) return lfail(p, "lops missing", -1);
         LTRY(p, cudaMemcpy(p->Lops.p, lops, sizeof(double2) * (size_t)L * nn, cudaMemcpyHostToDevice));
         std::vector<double> kh(2 * (size_t)L * nn, 0.0);
-        for (int l = 0; l < L; ++l) {
-            const double *Lm = lops + 2 * (size_t)l * nn;
-            double *K = kh.data() + 2 * (size_t)l * nn;
-            for (int i = 0; i < n; ++i)
-                for (int j = 0; j < n; ++j) {
-                    double sr = 0., si = 0.;
-                    for (int k = 0; k < n; ++k) {                             // conj(B[k][i]) * B[k][j]
-                        const double ar = Lm[2 * (k * n + i)], ai = -Lm[2 * (k * n + i) + 1], br = Lm[2 * (k * n + j)], bi = Lm[2 * (k * n + j) + 1];
-                        sr += ar * br - ai * bi; si += ar * bi + ai * br;
-                    }
-                    K[2 * (i * n + j)] = 0.5 * sr; K[2 * (i * n + j) + 1] = 0.5 * si;
-                }
-        }
+        build_khalf(lops, nullptr, n, L, kh.data());
         LTRY(p, cudaMemcpy(p->Kops.p, kh.data(), sizeof(double2) * (size_t)L * nn, cudaMemcpyHostToDevice));
     } else if (L > 0) {
         if (!gammas || !lops) return lfail(p, "gammas / lops missing", -1);
         LTRY(p, cudaMemcpy(p->gam.p, gammas, sizeof(double) * L, cudaMemcpyHostToDevice));
         LTRY(p, cudaMemcpy(p->Lops.p, lops, sizeof(double2) * (size_t)L * nn, cudaMemcpyHostToDevice));
         std::vector<double> kh(2 * (size_t)nn, 0.0);                         // 1/2 sum_l gamma_l L^dag L (mathmethods.py:193-194)
-        for (int l = 0; l < L; ++l) {
-            const double *Lm = lops + 2 * (size_t)l * nn;
-            for (int i = 0; i < n; ++i)
-                for (int j = 0; j < n; ++j) {
-                    double sr = 0., si = 0.;
-                    for (int k = 0; k < n; ++k) {                             // conj(L[k][i]) * L[k][j]
-                        const double ar = Lm[2 * (k * n + i)], ai = -Lm[2 * (k * n + i) + 1], br = Lm[2 * (k * n + j)], bi = Lm[2 * (k * n + j) + 1];
-                        sr += ar * br - ai * bi; si += ar * bi + ai * br;
-                    }
-                    kh[2 * (i * n + j)] += 0.5 * gammas[l] * sr; kh[2 * (i * n + j) + 1] += 0.5 * gammas[l] * si;
-                }
-        }
+        build_khalf(lops, gammas, n, L, kh.data());
         LTRY(p, cudaMemcpy(p->Khalf.p, kh.data(), sizeof(double2) * nn, cudaMemcpyHostToDevice));
     }
+    if (p->E > 1) {                                                         // kept for the members qocb_lindblad_set_ensemble leaves alone
+        p->h_h0.assign(2 * (size_t)nn, 0.0);
+        if (p->pb.have_hamiltonian) std::copy(h0, h0 + 2 * (size_t)nn, p->h_h0.begin());
+        p->h_gam.assign(gammas && L > 0 && !p->pb.time_dependent_rates ? gammas : nullptr,
+                        gammas && L > 0 && !p->pb.time_dependent_rates ? gammas + L : nullptr);
+        p->h_lops.assign(lops ? lops : nullptr, lops ? lops + 2 * (size_t)L * nn : nullptr);
+        p->ens_set = false;
+    }
     p->ops_set = true;
+    p->tape_ok = false;
+    return 0;
+}
+
+/* h0s: [E][n][n] or NULL; gammas: [E][L] or NULL (NULL: every member takes the plan's from qocb_lindblad_set_operators) */
+int qocb_lindblad_set_ensemble(qocb_lplan *p, const double *h0s, const double *gammas) {
+    if (!p) return -1;
+    if (p->E <= 1) return lfail(p, "qocb_lindblad_set_ensemble needs ensemble_count > 1", -1);
+    if (!p->ops_set) return lfail(p, "qocb_lindblad_set_operators must come before qocb_lindblad_set_ensemble", -1);
+    if (h0s && (!p->pb.have_hamiltonian || p->pb.channel_count > 0))
+        return lfail(p, "member drifts need a time-independent hamiltonian (have_hamiltonian = 1, channel_count = 0)", -1);
+    if (gammas && p->pb.time_dependent_rates) return lfail(p, "member rates need time_dependent_rates = 0", -1);
+    LTRY(p, cudaSetDevice(p->pb.device));
+    const int n = p->pb.hilbert_size, L = p->pb.lindblad_count, E = p->E;
+    const size_t nn = (size_t)n * n, Lg = std::max(L, 1);
+    std::vector<double> H(2 * E * nn), G(E * Lg, 0.0), K(2 * E * nn, 0.0);
+    for (int e = 0; e < E; ++e) {
+        const double *h = h0s ? h0s + 2 * e * nn : p->h_h0.data();
+        std::copy(h, h + 2 * nn, H.begin() + 2 * e * nn);
+        if (L > 0 && !p->pb.time_dependent_rates) {
+            const double *g = gammas ? gammas + (size_t)e * L : p->h_gam.data();
+            std::copy(g, g + L, G.begin() + e * Lg);
+            build_khalf(p->h_lops.data(), g, n, L, K.data() + 2 * e * nn);
+        }
+    }
+    LTRY(p, cudaStreamSynchronize(p->stream));
+    LTRY(p, cudaMemcpy(p->H0.p, H.data(), sizeof(double) * H.size(), cudaMemcpyHostToDevice));
+    LTRY(p, cudaMemcpy(p->gam.p, G.data(), sizeof(double) * G.size(), cudaMemcpyHostToDevice));
+    LTRY(p, cudaMemcpy(p->Khalf.p, K.data(), sizeof(double) * K.size(), cudaMemcpyHostToDevice));
+    p->ens_set = true;
     p->tape_ok = false;
     return 0;
 }
@@ -854,7 +960,7 @@ int qocb_lindblad_max_stage_time(qocb_lplan *p, double *t) {
     if (!p || !t) return lfail(p, "null argument", -1);
     if (p->NS == 0) return lfail(p, "this plan has no time series", -1);
     LTRY(p, cudaSetDevice(p->pb.device));
-    LTRY(p, cudaMemcpy(t, p->tseen.p, sizeof(double), cudaMemcpyDeviceToHost));
+    LTRY(p, cudaMemcpy(t, p->E > 1 ? p->tseen_max.p : p->tseen.p, sizeof(double), cudaMemcpyDeviceToHost));
     return 0;
 }
 
@@ -893,6 +999,8 @@ int qocb_lindblad_cost(qocb_lplan *p, const double *controls, double *cost, doub
     if (!p) return -1;
     p->tape_ok = false;
     if (int rc = launch_forward(p, controls, false)) return rc;
+    if (p->E > 1)
+        if (int rc = launch_mean(p, false)) return rc;
     return finish_lindblad(p, cost, nullptr, final_densities);
 }
 
@@ -900,14 +1008,18 @@ int qocb_lindblad_cost_and_grad(qocb_lplan *p, const double *controls, double *c
     if (!p) return -1;
     p->tape_ok = false;
     if (int rc = launch_forward(p, controls, true)) return rc;
-    if ((size_t)p->pb.control_eval_count * p->pb.control_count)
+    const bool with_grad = (size_t)p->pb.control_eval_count * p->pb.control_count > 0;
+    if (with_grad)
         if (int rc = launch_backward(p, nullptr)) return rc;
+    if (p->E > 1)
+        if (int rc = launch_mean(p, with_grad)) return rc;
     return finish_lindblad(p, cost, grad, final_densities);
 }
 
 int qocb_lindblad_forward(qocb_lplan *p, const double *controls, double *cost, double *final_densities) {
     if (!p) return -1;
     p->tape_ok = false;
+    if (p->E > 1) return lfail(p, "qocb_lindblad_forward / qocb_lindblad_backward do not run ensemble plans", -1);
     if (int rc = launch_forward(p, controls, true)) return rc;
     const int rc = finish_lindblad(p, cost, nullptr, final_densities);
     p->tape_ok = rc == 0;
@@ -917,6 +1029,7 @@ int qocb_lindblad_forward(qocb_lplan *p, const double *controls, double *cost, d
 /* seeds: [N][D][n][n] complex or NULL; row k is added to the cotangent of the densities at system step k */
 int qocb_lindblad_backward(qocb_lplan *p, const double *seeds, double *grad) {
     if (!p) return -1;
+    if (p->E > 1) return lfail(p, "qocb_lindblad_forward / qocb_lindblad_backward do not run ensemble plans", -1);
     const size_t cnt = (size_t)p->pb.control_eval_count * p->pb.control_count;
     if (!cnt) return 0;
     if (!p->tape_ok) return lfail(p, "qocb_lindblad_backward needs a successful qocb_lindblad_forward as the last evaluation", -1);
@@ -930,22 +1043,39 @@ int qocb_lindblad_backward(qocb_lplan *p, const double *seeds, double *grad) {
     return finish_lindblad(p, nullptr, grad, nullptr);
 }
 
-/* stats[0] = Runge-Kutta attempts, stats[1] = accepted steps of the last evaluation */
+/* stats[0] = Runge-Kutta attempts, stats[1] = accepted steps of the last evaluation (sums over the members of an ensemble) */
 int qocb_lindblad_stats(qocb_lplan *p, int64_t *stats) {
     if (!p || !stats) return -1;
     LTRY(p, cudaSetDevice(p->pb.device));
-    long long s[2];
-    LTRY(p, cudaMemcpy(s, p->stats.p, sizeof(s), cudaMemcpyDeviceToHost));
-    stats[0] = s[0]; stats[1] = s[1];
+    std::vector<long long> s(2 * (size_t)p->E);
+    LTRY(p, cudaMemcpy(s.data(), p->stats.p, sizeof(long long) * s.size(), cudaMemcpyDeviceToHost));
+    stats[0] = stats[1] = 0;
+    for (int e = 0; e < p->E; ++e) { stats[0] += s[2 * e]; stats[1] += s[2 * e + 1]; }
     return 0;
 }
 
-/* densities at every system step of the last evaluation: [N][D][n][n] complex */
+/* per-member results of the last evaluation: costs [E], grads [E][M][KR], stats [E][2]; any may be NULL */
+int qocb_lindblad_member_results(qocb_lplan *p, double *costs, double *grads, int64_t *stats) {
+    if (!p) return -1;
+    LTRY(p, cudaSetDevice(p->pb.device));
+    LTRY(p, cudaStreamSynchronize(p->stream));
+    const size_t E = p->E, cnt = (size_t)p->pb.control_eval_count * p->pb.control_count;
+    if (costs) LTRY(p, cudaMemcpy(costs, p->cost.p, sizeof(double) * E, cudaMemcpyDeviceToHost));
+    if (grads && cnt) LTRY(p, cudaMemcpy(grads, p->grad.p, sizeof(double) * E * cnt, cudaMemcpyDeviceToHost));
+    if (stats) {
+        std::vector<long long> s(2 * E);
+        LTRY(p, cudaMemcpy(s.data(), p->stats.p, sizeof(long long) * s.size(), cudaMemcpyDeviceToHost));
+        for (size_t i = 0; i < 2 * E; ++i) stats[i] = s[i];
+    }
+    return 0;
+}
+
+/* densities at every system step of the last evaluation: [N][D][n][n] complex, [E][N][D][n][n] for an ensemble */
 int qocb_lindblad_get_densities(qocb_lplan *p, double *out) {
     if (!p || !out) return -1;
     LTRY(p, cudaSetDevice(p->pb.device));
     const size_t DE = (size_t)p->pb.density_count * p->pb.hilbert_size * p->pb.hilbert_size;
-    LTRY(p, cudaMemcpy(out, p->states.p, sizeof(double2) * DE * p->pb.system_eval_count, cudaMemcpyDeviceToHost));
+    LTRY(p, cudaMemcpy(out, p->states.p, sizeof(double2) * DE * p->pb.system_eval_count * p->E, cudaMemcpyDeviceToHost));
     return 0;
 }
 
