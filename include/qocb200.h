@@ -39,7 +39,8 @@ typedef struct {
     int32_t system_eval_count;   /* N  (N-1 time slices, dt = T/(N-1), programstate.py:44) */
     int32_t magnus_order;        /* 2, 4 or 6  (qoc/models/magnuspolicy.py:8-26) */
     int32_t cost_eval_step;      /* >= 1 */
-    int32_t ensemble_count;      /* E >= 1: members differ in the drift H0 only; cost = mean over members */
+    int32_t ensemble_count;      /* E >= 1: members differ in the drift H0 (and, with qocb_set_member_operators, in the
+                                    control operators); cost = mean over members */
     int32_t device;              /* CUDA device ordinal */
     int32_t store_tape;          /* 1: keep Pade intermediates of the forward pass in HBM for the reverse pass;
                                     0: recompute them in the reverse pass (less memory, ~25% more flops) */
@@ -64,6 +65,16 @@ const char *qocb_last_error(const qocb_plan *plan);           /* plan may be NUL
 
 /* H0: [E][n][n] complex (E = ensemble_count), A: [KC][n][n] complex (KC = channel_count, or control_count if that is 0) */
 int qocb_set_operators(qocb_plan *plan, const double *h0, const double *a_ops);
+/* Ensembles whose members differ in their control operators too (drive-amplitude and crosstalk errors): a_ops
+   [E][KR][n][n] complex, member e's operators in the convention of qocb_set_operators, called after it (which shares
+   a_ops over the members and takes the drifts).  G becomes [E][KR][GMAT]; with the product-free M4 the commutators
+   C0[e][r] = [G0_e, G_er] and Cs[e][s<r] = [G_es, G_er] are built from each member's own operators.  The pivot-free
+   LU stays selected only if the drift and every operator of every member are Hermitian.  The kernels run the
+   arithmetic of shared operators on the member's own matrices, so a plan given E identical copies of the shared
+   operators is bit-identical to one that never made this call.  Returns -1 for plans with a node map
+   (channel_count > 0), time-sliced, state-sharded and hilbert_size > 64 plans.  A later qocb_set_operators returns
+   the plan to shared operators.  Plans that never make this call allocate nothing for it. */
+int qocb_set_member_operators(qocb_plan *plan, const double *a_ops);
 /* Time-dependent hamiltonian(controls, time) (the callable's `time` argument, qoc/core/schroedingerdiscrete.py:483-486),
    affine in the controls: at Magnus node i of slice j
        H = H0 + sum_c coef[j][i][c] A_c,   coef[j][i][c] = offset[j][i][c] + sum_r gain[j][i][c][r] x_r(t_ji),
@@ -214,9 +225,10 @@ int qocb_expm_batched_bench(int32_t n, int64_t batch, double norm_scale, int32_t
        returned here matches the reference-equivalent gradient with the step grid frozen within 1e-7 relative, and the full
        one within its own reproducibility band.  It is NOT claimed at the 1e-10 of the Schroedinger path.
 
-   ENSEMBLES (robust control over drifts and decay rates).  ensemble_count = E > 1 runs E members, one CTA each, in one launch
-   of each kernel.  Members differ in the drift H0 and/or the rates gamma_l (qocb_lindblad_set_ensemble); rho0, control and
-   Lindblad operators, cost terms, controls and the time series are shared.  Every member runs exactly the code and the launch
+   ENSEMBLES (robust control over drifts, control operators and decay rates).  ensemble_count = E > 1 runs E members, one CTA
+   each, in one launch of each kernel.  Members differ in the drift H0 and/or the rates gamma_l (qocb_lindblad_set_ensemble)
+   and optionally in the control operators (qocb_lindblad_set_member_operators); rho0, Lindblad operators, cost terms,
+   controls and the time series are shared.  Every member runs exactly the code and the launch
    layout of a one-member plan of the same shape, so its results are bit-identical to such a plan built with its drift and
    rates.  The cost and gradient are the member mean: sums in member order 0..E-1 divided by E (no atomics).  Each member has
    its own tape of max_rk_steps steps (0: max(4096, min(2^20, 8 GiB / (E * 2 * D n^2 * 16 B)))); a member whose forward
@@ -254,6 +266,13 @@ int qocb_lindblad_set_operators(qocb_lplan *plan, const double *h0, const double
    channel_count = 0), gammas [E][L] (NULL: every member takes the plan's; needs time_dependent_rates = 0).  Member e's
    1/2 sum_l gamma_el L_l^dag L_l is built on the host as qocb_lindblad_set_operators builds it.  Returns -1 on E <= 1. */
 int qocb_lindblad_set_ensemble(qocb_lplan *plan, const double *h0s, const double *gammas);
+/* Per-member control operators of an ensemble (drive-amplitude and crosstalk errors): a_ops [E][KR][n][n], member e's
+   operators in the convention of qocb_lindblad_set_operators, called after it; member e then evolves under
+   h0_e + sum_r x_r A_er.  Every member still runs the code and the shared-memory layout of a one-member plan of the same
+   shape, so its results are bit-identical to such a plan built with its operators.  Returns -1 for plans whose
+   hamiltonian is a Chebyshev table (channel_count > 0) or that have none.  A later qocb_lindblad_set_operators returns
+   the plan to shared operators.  Plans that never make this call allocate nothing for it. */
+int qocb_lindblad_set_member_operators(qocb_lplan *plan, const double *a_ops);
 /* series: [segments][degree+1][NS] Chebyshev coefficients per segment [s w, (s+1) w] (constant term not halved);
    degree <= 64; may be called again to replace the table */
 int qocb_lindblad_set_time_series(qocb_lplan *plan, int32_t segments, int32_t degree, double segment_width,

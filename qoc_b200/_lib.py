@@ -31,7 +31,7 @@ EXPORTS = [
     "qocb_lindblad_set_operators", "qocb_lindblad_set_densities", "qocb_lindblad_add_cost", "qocb_lindblad_cost",
     "qocb_lindblad_cost_and_grad", "qocb_lindblad_stats", "qocb_lindblad_get_densities", "qocb_lindblad_set_time_series",
     "qocb_lindblad_max_stage_time", "qocb_lindblad_forward", "qocb_lindblad_backward", "qocb_lindblad_set_ensemble",
-    "qocb_lindblad_member_results",
+    "qocb_lindblad_member_results", "qocb_set_member_operators", "qocb_lindblad_set_member_operators",
 ]
 
 
@@ -112,6 +112,7 @@ def load():
     lib.qocb_last_error.argtypes = [vp]
     lib.qocb_last_error.restype = C.c_char_p
     lib.qocb_set_operators.argtypes = [vp, vp, vp]
+    lib.qocb_set_member_operators.argtypes = [vp, vp]
     lib.qocb_set_node_map.argtypes = [vp, vp, vp]
     lib.qocb_set_states.argtypes = [vp, vp]
     lib.qocb_add_cost.argtypes = [vp, i32, i32, dbl, vp, vp, i32]
@@ -153,6 +154,7 @@ def load():
     lib.qocb_lindblad_set_time_series.argtypes = [vp, i32, i32, dbl, vp]
     lib.qocb_lindblad_max_stage_time.argtypes = [vp, vp]
     lib.qocb_lindblad_set_ensemble.argtypes = [vp, vp, vp]
+    lib.qocb_lindblad_set_member_operators.argtypes = [vp, vp]
     lib.qocb_lindblad_member_results.argtypes = [vp, vp, vp, vp]
     lib.qocb_flush_l2.argtypes = [vp]
     lib.qocb_shard_matrix_doubles.argtypes = [vp]

@@ -230,6 +230,40 @@ def extract_hamiltonian_structure(hamiltonian, control_count, complex_controls, 
     return h0, a_ops
 
 
+def ensemble_member_structures(hamiltonians, hilbert_size, control_count, complex_controls, evolution_time):
+    """(h0s [E][n][n], a_ops) of the members of `ensemble_hamiltonians`, each probed as `extract_hamiltonian_structure` probes
+    the nominal hamiltonian.  a_ops is [KR][n][n] when every member's operators equal member 0's exactly (the members differ
+    in the drift only: the plan takes the drift-only route of `ensemble_drifts`), else [E][KR][n][n].  Raises before any
+    device call: ValueError for no members, a member of another hilbert size or one that does not take the plan's controls,
+    NotImplementedError for a member that reads `time`, NonlinearHamiltonian for one that is not affine in the controls."""
+    members = list(hamiltonians)
+    if not members:
+        raise ValueError("ensemble_hamiltonians needs at least one member")
+    zero, units = _unit_controls(control_count, complex_controls) if control_count else (None, [])
+    h0s, ops = [], []
+    for e, h in enumerate(members):
+        if not callable(h):
+            raise ValueError("ensemble_hamiltonians[{}] is not a callable hamiltonian(controls, time)".format(e))
+        try:
+            time_dependent = _is_time_dependent(h, zero, units, evolution_time)
+            if not time_dependent:
+                h0, a_ops = extract_hamiltonian_structure(h, control_count, complex_controls, evolution_time)
+        except (IndexError, TypeError, ValueError) as err:
+            raise ValueError("ensemble_hamiltonians[{}] does not take the plan's {} {} controls: {}".format(
+                e, control_count, "complex" if complex_controls else "real", err)) from err
+        if time_dependent:
+            raise NotImplementedError("ensemble hamiltonians that read `time` are not supported (member {})".format(e))
+        if h0.shape != (hilbert_size, hilbert_size):
+            raise ValueError("ensemble_hamiltonians[{}] has shape {}, the plan's hilbert size is {}".format(
+                e, h0.shape, hilbert_size))
+        h0s.append(h0)
+        ops.append(a_ops)
+    h0s = np.ascontiguousarray(h0s, dtype=np.complex128)
+    ops = np.ascontiguousarray(ops, dtype=np.complex128)
+    shared = all(np.array_equal(a, ops[0]) for a in ops[1:])
+    return h0s, np.ascontiguousarray(ops[0]) if shared else ops
+
+
 def central_differences(f, z):
     """4-point central differences (step 1e-3 max(1, |z_i|), error O(h^4)) of the real function `f` at every entry of the
     array `z`, of any shape: returns (df/dRe z, df/dIm z), the second None for real `z`.  Every entry is differentiated on its
@@ -284,7 +318,14 @@ class SchroedingerPlan(object):
                  control_eval_count=0, control_count=0, complex_controls=False,
                  magnus_policy=MagnusPolicy.M2, cost_eval_step=1,
                  interpolation_policy=InterpolationPolicy.LINEAR, device=0, store_tape=True,
-                 chunks_per_member=0, ensemble_drifts=None, structure=None, slice_range=None, state_slice=None):
+                 chunks_per_member=0, ensemble_drifts=None, structure=None, slice_range=None, state_slice=None,
+                 ensemble_hamiltonians=None):
+        """`ensemble_drifts` [E][n][n] (members differ in the drift) or `ensemble_hamiltonians` [h_0 .. h_{E-1}] (callables
+        like `hamiltonian`: members differ in the drift and the control operators, e.g. drive-amplitude or crosstalk errors)
+        make a robust-control ensemble: cost and gradient are the member mean, final and intermediate states per member."""
+        if ensemble_drifts is not None and ensemble_hamiltonians is not None:
+            raise ValueError("pass ensemble_drifts or ensemble_hamiltonians, not both")
+        ensemble = ensemble_drifts is not None or ensemble_hamiltonians is not None
         if interpolation_policy != InterpolationPolicy.LINEAR:
             raise NotImplementedError("The interpolation policy {} is not yet supported for this method."
                                       "".format(interpolation_policy))
@@ -300,7 +341,7 @@ class SchroedingerPlan(object):
             s0, s1 = int(state_slice[0]), int(state_slice[1])
             if not 0 <= s0 < s1 <= self.S_total:
                 raise ValueError("bad state slice {} of {} states".format(state_slice, self.S_total))
-            if ensemble_drifts is not None or slice_range is not None:
+            if ensemble or slice_range is not None:
                 raise NotImplementedError("state sharding cannot be combined with ensembles or time-slice sharding")
             initial_states = initial_states[s0:s1]
             self.state_first = s0
@@ -311,6 +352,12 @@ class SchroedingerPlan(object):
         self.complex_controls = bool(complex_controls)
         self.KR = self.K * (2 if self.complex_controls else 1)
         self.costs = list(costs)
+        from qoc_b200.models.cost import Cost
+        user_cost = lambda c: (getattr(type(c), "device_terms", Cost.device_terms) is Cost.device_terms and
+                               getattr(type(c), "control_value_and_grad", Cost.control_value_and_grad) is
+                               Cost.control_value_and_grad)
+        if ensemble_hamiltonians is not None and any(user_cost(c) for c in self.costs):
+            raise NotImplementedError("user-defined costs cannot be combined with ensembles or sharded plans")
         if structure is None:
             structure = extract_hamiltonian_structure(hamiltonian, self.K, self.complex_controls, evolution_time,
                                                       system_eval_count=self.N, magnus_order=magnus_policy.order)
@@ -319,10 +366,18 @@ class SchroedingerPlan(object):
         node_map = structure[2:] if len(structure) == 4 else None
         if node_map is not None and ensemble_drifts is not None:
             raise NotImplementedError("ensemble drifts with a time-dependent hamiltonian are not supported")
+        if node_map is not None and ensemble_hamiltonians is not None:
+            raise NotImplementedError("ensemble hamiltonians with a time-dependent hamiltonian are not supported")
         if h0.shape[0] != self.n:
             raise ValueError("hamiltonian size {} does not match the states' hilbert size {}".format(h0.shape[0], self.n))
-        if ensemble_drifts is not None:          # build-side extension: members differ in the drift only
+        member_ops = None                        # [E][KR][n][n] when the members' control operators differ
+        if ensemble_drifts is not None:
             h0s = np.ascontiguousarray(ensemble_drifts, dtype=np.complex128)
+        elif ensemble_hamiltonians is not None:
+            h0s, a_ops = ensemble_member_structures(ensemble_hamiltonians, self.n, self.K, self.complex_controls,
+                                                    evolution_time)
+            if a_ops.ndim == 4:
+                member_ops, a_ops = a_ops, a_ops[0]
         else:
             h0s = np.ascontiguousarray(h0[None], dtype=np.complex128)
         self.E = h0s.shape[0]
@@ -341,6 +396,8 @@ class SchroedingerPlan(object):
         self.handle = handle
         a_ops = np.ascontiguousarray(a_ops, dtype=np.complex128)
         _lib.check(self.lib.qocb_set_operators(handle, _lib.ptr(h0s), _lib.ptr(a_ops) if a_ops.shape[0] else None), handle)
+        if member_ops is not None:
+            _lib.check(self.lib.qocb_set_member_operators(handle, _lib.ptr(member_ops)), handle)
         if node_map is not None:
             offset = np.ascontiguousarray(node_map[0], dtype=np.float64)
             gain = np.ascontiguousarray(node_map[1], dtype=np.float64)
@@ -349,10 +406,8 @@ class SchroedingerPlan(object):
         _lib.check(self.lib.qocb_set_states(handle, _lib.ptr(psi0)), handle)
         self.control_costs = []
         self.user_costs = []
-        from qoc_b200.models.cost import Cost
         for c in self.costs:
-            if (getattr(type(c), "device_terms", Cost.device_terms) is Cost.device_terms and
-                    getattr(type(c), "control_value_and_grad", Cost.control_value_and_grad) is Cost.control_value_and_grad):
+            if user_cost(c):
                 # a user-defined Cost subclass (qoc/models/cost.py:5-51): only `cost(controls, states, step)` exists.  Its value and
                 # a numeric cotangent of the final states are computed on the host around qocb_forward / qocb_backward.
                 if getattr(c, "requires_step_evaluation", False):
@@ -971,15 +1026,16 @@ class LindbladPlan(object):
     reference's autograd tape also differentiates the step-size controller; those terms are rounding noise (see
     oracle/lindblad_adjoint_model.py and DESIGN.md section 5) and are deliberately not reproduced.
 
-    Ensembles (robust control): `ensemble_drifts` [E][n][n] replaces the drift of `hamiltonian` and `ensemble_rates` [E][L]
-    the decay rates of `lindblad_data`, member by member.  `cost` and `cost_and_grad` then return the member mean (control
+    Ensembles (robust control): `ensemble_drifts` [E][n][n] replaces the drift of `hamiltonian`, or `ensemble_hamiltonians`
+    [h_0 .. h_{E-1}] (callables like `hamiltonian`) its drift and control operators, and `ensemble_rates` [E][L] the decay
+    rates of `lindblad_data`, member by member.  `cost` and `cost_and_grad` then return the member mean (control
     costs added once) with final densities [E][D][n][n], `intermediate_densities()` is [E][N][D][n][n] and `member_results()`
     returns every member's cost, gradient and stats.  One member is the plain plan."""
 
     def __init__(self, initial_densities, costs, evolution_time, system_eval_count, hamiltonian=None,
                  lindblad_data=None, control_eval_count=0, control_count=0, complex_controls=False, cost_eval_step=1,
                  interpolation_policy=InterpolationPolicy.LINEAR, device=0, max_rk_steps=0, structure=None,
-                 ensemble_drifts=None, ensemble_rates=None):
+                 ensemble_drifts=None, ensemble_rates=None, ensemble_hamiltonians=None):
         if interpolation_policy != InterpolationPolicy.LINEAR:
             raise ValueError("The interpolation policy {} is not implemented for this method."
                              "".format(interpolation_policy))
@@ -1019,13 +1075,16 @@ class LindbladPlan(object):
         if h0 is not None and h0.shape[0] != self.n:
             raise ValueError("hamiltonian size {} does not match the densities' hilbert size {}".format(h0.shape[0], self.n))
         self.L = 0 if lops is None else lops.shape[0]
-        h0s, rates = self._ensemble_members(ensemble_drifts, ensemble_rates, td_h, td_l)
+        h0s, rates, ops = self._ensemble_members(ensemble_drifts, ensemble_rates, ensemble_hamiltonians, td_h, td_l)
         self.E = 1 if h0s is None and rates is None else (h0s if h0s is not None else rates).shape[0]
+        member_ops = None                                # [E][KR][n][n] when the members' control operators differ
+        if ops is not None:
+            a_ops, member_ops = (ops[0], ops) if ops.ndim == 4 else (ops, None)
         if self.E == 1:                                  # one member: the plain plan with that member's drift and rates
             h0 = h0 if h0s is None else h0s[0]
             gammas = gammas if rates is None else rates[0]
             h0s = rates = None
-        self._members = (h0s, rates)
+        self._members = (h0s, rates, member_ops)
         self._last_extra = (0.0, None)
         self.range_extensions = 0
         self._setup = dict(rho0=rho0, h0=h0, a_ops=a_ops, gammas=gammas, lops=lops, cost_eval_step=int(cost_eval_step),
@@ -1063,13 +1122,23 @@ class LindbladPlan(object):
             for k in (range(ces, self.N, ces) if getattr(c, "requires_step_evaluation", False) else (self.N - 1,)):
                 self._user_at.setdefault(k, []).append(c)
 
-    def _ensemble_members(self, drifts, rates, td_h, td_l):
-        """validated member drifts [E][n][n] and rates [E][L] (either may be None); raises before any device call."""
-        if drifts is None and rates is None:
-            return None, None
+    def _ensemble_members(self, drifts, rates, hamiltonians, td_h, td_l):
+        """validated member drifts [E][n][n], rates [E][L] and, from `ensemble_hamiltonians`, control operators ([KR][n][n]
+        when shared, else [E][KR][n][n]); any may be None.  Raises before any device call."""
+        if drifts is None and rates is None and hamiltonians is None:
+            return None, None, None
         if any(is_user_cost(c) for c in self.costs):
             raise NotImplementedError("user-defined costs cannot be combined with ensembles")
-        if drifts is not None:
+        ops = None
+        if hamiltonians is not None:
+            if drifts is not None:
+                raise ValueError("pass ensemble_drifts or ensemble_hamiltonians, not both")
+            if not self.have_h:
+                raise ValueError("ensemble_hamiltonians replace `hamiltonian`, which is None")
+            if td_h:
+                raise NotImplementedError("ensemble hamiltonians with a time-dependent hamiltonian are not supported")
+            drifts, ops = ensemble_member_structures(hamiltonians, self.n, self.K, self.complex_controls, self.T)
+        elif drifts is not None:
             if not self.have_h:
                 raise ValueError("ensemble_drifts replace the drift of `hamiltonian`, which is None")
             if td_h:
@@ -1088,8 +1157,9 @@ class LindbladPlan(object):
             if rates.ndim != 2 or rates.shape[0] < 1 or rates.shape[1] != self.L:
                 raise ValueError("ensemble_rates must have shape [E][{}], got {}".format(self.L, rates.shape))
         if drifts is not None and rates is not None and drifts.shape[0] != rates.shape[0]:
-            raise ValueError("ensemble_drifts has {} members and ensemble_rates {}".format(drifts.shape[0], rates.shape[0]))
-        return drifts, rates
+            raise ValueError("{} has {} members and ensemble_rates {}".format(
+                "ensemble_drifts" if hamiltonians is None else "ensemble_hamiltonians", drifts.shape[0], rates.shape[0]))
+        return drifts, rates, ops
 
     def _open(self):
         """creates the device plan and uploads operators, densities, the ensemble members and (time-dependent problems) the
@@ -1117,6 +1187,8 @@ class LindbladPlan(object):
                                                          _lib.ptr(lops)))
         if self.E > 1:
             self._check(self.lib.qocb_lindblad_set_ensemble(handle, _lib.ptr(self._members[0]), _lib.ptr(self._members[1])))
+            if self._members[2] is not None:
+                self._check(self.lib.qocb_lindblad_set_member_operators(handle, _lib.ptr(self._members[2])))
         self._check(self.lib.qocb_lindblad_set_densities(handle, _lib.ptr(su["rho0"])))
         if st is not None:
             self._check(self.lib.qocb_lindblad_set_time_series(handle, st.segments, st.degree, st.width, _lib.ptr(st.series)))

@@ -434,23 +434,28 @@ class StateShardedPlan(object):
 
 
 class EnsembleShardedPlan(object):
-    """robust-control ensembles (cfg5): members that differ in the drift are independent units, block-partitioned across the
+    """robust-control ensembles (cfg5): members that differ in the drift (`ensemble_drifts`) or in drift and control
+    operators (`ensemble_hamiltonians`, callables like `hamiltonian`) are independent units, block-partitioned across the
     ranks; one NCCL all-reduce of [gradient | cost] on the plan stream ends the evaluation - inside the device-timed region,
     no host bounce.  Cost = mean over members.  `cost_and_grad` returns the final states of the LOCAL members."""
 
-    def __init__(self, hamiltonian, initial_states, costs, evolution_time, system_eval_count, ensemble_drifts, device=0,
-                 group=None, **kw):
+    def __init__(self, hamiltonian, initial_states, costs, evolution_time, system_eval_count, ensemble_drifts=None, device=0,
+                 group=None, ensemble_hamiltonians=None, **kw):
+        if (ensemble_drifts is None) == (ensemble_hamiltonians is None):
+            raise ValueError("EnsembleShardedPlan needs exactly one of ensemble_drifts and ensemble_hamiltonians")
         import torch
         import torch.distributed as dist
         self.torch, self.dist, self.group = torch, dist, group
         self.rank, self.world = dist.get_rank(group), dist.get_world_size(group)
         self.comm = TorchDistComm(group)
-        drifts = np.asarray(ensemble_drifts)
-        self.E_total = drifts.shape[0]
+        members = np.asarray(ensemble_drifts) if ensemble_hamiltonians is None else list(ensemble_hamiltonians)
+        self.E_total = len(members)
         b = slice_bounds(self.E_total, self.world)
         self.member_range = (b[self.rank], b[self.rank + 1])
-        self.plan = SchroedingerPlan(hamiltonian, initial_states, costs, evolution_time, system_eval_count,
-                                     ensemble_drifts=drifts[b[self.rank]:b[self.rank + 1]], device=device, **kw)
+        local = members[b[self.rank]:b[self.rank + 1]]
+        self.plan = SchroedingerPlan(hamiltonian, initial_states, costs, evolution_time, system_eval_count, device=device,
+                                     **(dict(ensemble_drifts=local) if ensemble_hamiltonians is None
+                                        else dict(ensemble_hamiltonians=local)), **kw)
         p = self.plan
         self.KR, self.K, self.M, self.S, self.n, self.E = p.KR, p.K, p.M, p.S, p.n, p.E
         self.complex_controls = p.complex_controls

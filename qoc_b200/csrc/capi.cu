@@ -73,6 +73,15 @@ struct FeedMaps {
     int premagnus;      // 1: U[w] holds M_w (magnus.cuh); 0: assemble the Magnus matrix in this kernel
 };
 
+// member e's control operators and their commutators (per-member operators only: the strides are 0 when they are
+// shared).  Applied where the operators are read rather than once per slice, so that the pointers are not held in
+// registers across the Pade passes (k_backward<64> sits at the register limit).
+__device__ __forceinline__ GenArgs member_ops(GenArgs ga, int e) {
+    ga.G += e * ga.g_stride;
+    ga.Cs += e * ga.cs_stride;
+    return ga;
+}
+
 template <class C>
 __global__ void __launch_bounds__(C::NT) k_forward(KArgs a, const __grid_constant__ FeedMaps fm) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -109,10 +118,10 @@ __global__ void __launch_bounds__(C::NT) k_forward(KArgs a, const __grid_constan
             load_coefs<C>(sm, ga, j);
             if (magnus_pair_ok<C>(ga) && w + 1 < we) {
                 load_coefs_to<C>(sm.red, ga, j + 1);
-                magnus_forward_pair<C>(sm, ga, sm.coef, sm.red, gMnext);
+                magnus_forward_pair<C>(sm, member_ops(ga, e), sm.coef, sm.red, gMnext);
                 parked = true;
             } else {
-                magnus_forward<C>(sm, ga, scratch);
+                magnus_forward<C>(sm, member_ops(ga, e), scratch);
             }
         }
         PROF_MARK(1);
@@ -183,7 +192,7 @@ __global__ void __launch_bounds__(C::NT) k_backward(KArgs a, const __grid_consta
             piv = a.tape_piv + (size_t)w * C::NP;
             s = a.meta[w];
         } else {
-            magnus_forward<C>(sm, ga, scratch);
+            magnus_forward<C>(sm, member_ops(ga, e), scratch);
             s = pade_forward<C>(sm, ctape, cpiv, scratch + (size_t)S_T0 * C::GMAT, scratch + (size_t)S_T1 * C::GMAT, kCtaTapeR,
                                 nullptr, nullptr, a.herm, a.tape_min);
             if (s > kCtaTapeR && threadIdx.x == 0) *a.err_flag = 1;
@@ -232,7 +241,7 @@ __global__ void __launch_bounds__(C::NT) k_backward(KArgs a, const __grid_consta
             for_owned<C>([&](int, int, int row, int col) { stg2<C>(gM, row, col, lds2<C>(sm.X0, row, col)); });
             __syncthreads();
         } else {
-            magnus_backward<C>(sm, ga, scratch, a.node_grad + (size_t)w * ga.q * ga.KR);
+            magnus_backward<C>(sm, member_ops(ga, e), scratch, a.node_grad + (size_t)w * ga.q * ga.KR);
         }
         PROF_MARK(13);
     }
@@ -409,6 +418,42 @@ void from_planar(const double *src, double *dst, int n, int NP) {
         }
 }
 
+// host-side commutators of the product-free M4 (qocb_set_operators, qocb_set_member_operators); interleaved complex n x n
+typedef std::vector<double> HostMat;
+HostMat host_generator(const double *h, int n) {             // G = -1j H
+    HostMat g(2 * (size_t)n * n);
+    for (size_t i = 0; i < (size_t)n * n; ++i) { g[2 * i] = h[2 * i + 1]; g[2 * i + 1] = -h[2 * i]; }
+    return g;
+}
+HostMat host_commutator(const HostMat &x, const HostMat &y, int n) {   // [x, y]
+    HostMat c(2 * (size_t)n * n, 0.0);
+    for (int i = 0; i < n; ++i)
+        for (int k = 0; k < n; ++k) {
+            const double xr = x[2 * ((size_t)i * n + k)], xi = x[2 * ((size_t)i * n + k) + 1];
+            const double yr = y[2 * ((size_t)i * n + k)], yi = y[2 * ((size_t)i * n + k) + 1];
+            for (int j = 0; j < n; ++j) {
+                const double br = y[2 * ((size_t)k * n + j)], bi = y[2 * ((size_t)k * n + j) + 1];
+                const double ar = x[2 * ((size_t)k * n + j)], ai = x[2 * ((size_t)k * n + j) + 1];
+                c[2 * ((size_t)i * n + j)] += (xr * br - xi * bi) - (yr * ar - yi * ai);
+                c[2 * ((size_t)i * n + j) + 1] += (xr * bi + xi * br) - (yr * ai + yi * ar);
+            }
+        }
+    return c;
+}
+// Hermitian to 1e-13 of the largest entry: selects the pivot-free LU where it is safe (tile.cuh)
+bool host_is_hermitian(const double *h, int n) {
+    double mx = 0., dev = 0.;
+    for (int r = 0; r < n; ++r)
+        for (int c = 0; c <= r; ++c) {
+            const double ar = h[2 * ((size_t)r * n + c)], ai = h[2 * ((size_t)r * n + c) + 1];
+            const double br = h[2 * ((size_t)c * n + r)], bi = h[2 * ((size_t)c * n + r) + 1];
+            mx = std::max(mx, std::max(std::fabs(ar) + std::fabs(ai), std::fabs(br) + std::fabs(bi)));
+            dev = std::max(dev, std::fabs(ar - br) + std::fabs(ai + bi));
+        }
+    return dev <= 1e-13 * mx;
+}
+bool no_nopiv() { const char *np_ = getenv("QOCB_NO_NOPIV"); return np_ && np_[0] == '1'; }
+
 template <class T> struct DevBuf {
     T *p = nullptr; size_t n = 0;
     cudaError_t alloc(size_t count) {
@@ -510,6 +555,8 @@ struct qocb_plan {
     int lowrank_mode = 2;               // 0 dense reverse pass, 1 re-associated rank-S form, 2 Krylov basis of A2 (QOCB_LOWRANK=0/1/2)
     bool premagnus_ok = true;           // QOCB_NO_PREMAGNUS=1: assemble the Magnus matrices inside k_forward (A/B comparison)
     bool hermitian = false;             // H0 (every member) and every operator channel are Hermitian (QOCB_NO_NOPIV=1 clears it)
+    bool drift_hermitian = false;       // H0 of every member is Hermitian (qocb_set_member_operators recomputes `hermitian`)
+    bool member_ops = false;            // G, C0 and Cs hold every member's own control operators (qocb_set_member_operators)
     double *h_pinned = nullptr;         // [M*KR controls | M*KR grad | 1 cost]
     // CUDA graph of one whole host-facing evaluation (H2D controls, all kernels, D2H of gradient, cost, final states and the
     // error flag): replayed by qocb_cost / qocb_cost_and_grad from the third call on - launch-bound small problems gain 2x
@@ -626,6 +673,9 @@ KArgs make_kargs(qocb_plan *p) {
     a.ga.KR = p->KC; a.ga.q = p->q; a.ga.order = p->pb.magnus_order;
     a.ga.nodecoef = p->mapped ? p->nodecoef.p : nullptr;
     a.ga.C0 = p->C0.p; a.ga.Cs = p->Cs.p; a.ga.comm = p->comm_ok ? 1 : 0;
+    const long long GM = 2LL * p->NP * p->NP;
+    a.ga.g_stride = p->member_ops ? p->KC * GM : 0;
+    a.ga.cs_stride = p->member_ops && p->comm_ok ? p->KC * (p->KC - 1) / 2 * GM : 0;
     a.ga.dt = p->pb.evolution_time / (p->pb.system_eval_count - 1);
     a.N = p->Nloc; a.E = p->pb.ensemble_count;
     a.s_cap = kStoredTapeR; a.tape_mats = p->tape_mats;
@@ -1778,17 +1828,7 @@ int qocb_set_operators(qocb_plan *p, const double *h0, const double *a_ops) {
     CU_TRY(p, cudaSetDevice(p->pb.device));
     const int n = p->pb.hilbert_size, NP = p->NP, E = p->pb.ensemble_count, KR = p->KC;   // operator channels
     const size_t GM = 2 * (size_t)NP * NP;
-    auto is_hermitian = [&](const double *h) {
-        double mx = 0., dev = 0.;
-        for (int r = 0; r < n; ++r)
-            for (int c = 0; c <= r; ++c) {
-                const double ar = h[2 * ((size_t)r * n + c)], ai = h[2 * ((size_t)r * n + c) + 1];
-                const double br = h[2 * ((size_t)c * n + r)], bi = h[2 * ((size_t)c * n + r) + 1];
-                mx = std::max(mx, std::max(std::fabs(ar) + std::fabs(ai), std::fabs(br) + std::fabs(bi)));
-                dev = std::max(dev, std::fabs(ar - br) + std::fabs(ai + bi));
-            }
-        return dev <= 1e-13 * mx;
-    };
+    auto is_hermitian = [&](const double *h) { return host_is_hermitian(h, n); };
     if (p->large) {                                    // interleaved generators G = -1j * H
         {   // Hermitian operators: the Pade denominator may be factored by the own block LU (large.cuh) while ||A||_1 < 2.5
             bool herm = is_hermitian(h0);
@@ -1832,10 +1872,11 @@ int qocb_set_operators(qocb_plan *p, const double *h0, const double *a_ops) {
         auto is_herm = is_hermitian;
         bool herm = true;
         for (int e = 0; e < E && herm; ++e) herm = is_herm(h0 + (size_t)e * 2 * n * n);
+        p->drift_hermitian = herm;
         for (int r = 0; r < KR && herm && a_ops; ++r) herm = is_herm(a_ops + (size_t)r * 2 * n * n);
-        const char *np_ = getenv("QOCB_NO_NOPIV");
-        p->hermitian = herm && !(np_ && np_[0] == '1');
+        p->hermitian = herm && !no_nopiv();
     }
+    p->member_ops = false;
     std::vector<double> buf((size_t)std::max(E, KR) * GM);
     for (int e = 0; e < E; ++e) to_planar(h0 + (size_t)e * 2 * n * n, buf.data() + (size_t)e * GM, n, NP, true);
     CU_TRY(p, cudaMemcpy(p->G0.p, buf.data(), sizeof(double) * E * GM, cudaMemcpyHostToDevice));
@@ -1848,44 +1889,71 @@ int qocb_set_operators(qocb_plan *p, const double *h0, const double *a_ops) {
     p->comm_ok = false;
     { const char *nc = getenv("QOCB_NO_COMM"); if (p->pb.magnus_order == 4 && KR <= kMaxCommKR && !(nc && nc[0] == '1')) p->comm_ok = true; }
     if (p->comm_ok) {
-        typedef std::vector<double> Mat;                           // interleaved complex n x n
-        auto gen = [&](const double *h) { Mat g(2 * (size_t)n * n); for (size_t i = 0; i < (size_t)n * n; ++i) { g[2 * i] = h[2 * i + 1]; g[2 * i + 1] = -h[2 * i]; } return g; };
-        auto comm = [&](const Mat &x, const Mat &y) {
-            Mat c(2 * (size_t)n * n, 0.0);
-            for (int i = 0; i < n; ++i)
-                for (int k = 0; k < n; ++k) {
-                    const double xr = x[2 * ((size_t)i * n + k)], xi = x[2 * ((size_t)i * n + k) + 1];
-                    const double yr = y[2 * ((size_t)i * n + k)], yi = y[2 * ((size_t)i * n + k) + 1];
-                    for (int j = 0; j < n; ++j) {
-                        const double br = y[2 * ((size_t)k * n + j)], bi = y[2 * ((size_t)k * n + j) + 1];
-                        const double ar = x[2 * ((size_t)k * n + j)], ai = x[2 * ((size_t)k * n + j) + 1];
-                        c[2 * ((size_t)i * n + j)] += (xr * br - xi * bi) - (yr * ar - yi * ai);
-                        c[2 * ((size_t)i * n + j) + 1] += (xr * bi + xi * br) - (yr * ai + yi * ar);
-                    }
-                }
-            return c;
-        };
-        std::vector<Mat> g(KR);
-        for (int r = 0; r < KR; ++r) g[r] = gen(a_ops + (size_t)r * 2 * n * n);
+        std::vector<HostMat> g(KR);
+        for (int r = 0; r < KR; ++r) g[r] = host_generator(a_ops + (size_t)r * 2 * n * n, n);
         const int npair = KR * (KR - 1) / 2;
         CU_TRY(p, p->C0.alloc(std::max<size_t>(1, (size_t)E * KR) * GM)); CU_TRY(p, p->Cs.alloc(std::max<size_t>(1, (size_t)npair) * GM));
         std::vector<double> pl(GM);
         for (int e = 0; e < E; ++e) {
-            const Mat g0 = gen(h0 + (size_t)e * 2 * n * n);
+            const HostMat g0 = host_generator(h0 + (size_t)e * 2 * n * n, n);
             for (int r = 0; r < KR; ++r) {
-                const Mat c = comm(g0, g[r]);
+                const HostMat c = host_commutator(g0, g[r], n);
                 to_planar(c.data(), pl.data(), n, NP, false);
                 CU_TRY(p, cudaMemcpy(p->C0.p + ((size_t)e * KR + r) * GM, pl.data(), sizeof(double) * GM, cudaMemcpyHostToDevice));
             }
         }
         for (int s_ = 0; s_ < KR; ++s_)
             for (int r = s_ + 1; r < KR; ++r) {
-                const Mat c = comm(g[s_], g[r]);
+                const HostMat c = host_commutator(g[s_], g[r], n);
                 to_planar(c.data(), pl.data(), n, NP, false);
                 CU_TRY(p, cudaMemcpy(p->Cs.p + (size_t)comm_pair(s_, r, KR) * GM, pl.data(), sizeof(double) * GM, cudaMemcpyHostToDevice));
             }
     }
     p->ops_set = true;
+    return 0;
+}
+
+int qocb_set_member_operators(qocb_plan *p, const double *a_ops) {
+    if (!p || !a_ops) { set_error(p, "null argument"); return -1; }
+    if (!p->ops_set) { set_error(p, "qocb_set_member_operators needs qocb_set_operators first"); return -1; }
+    if (p->mapped) { set_error(p, "per-member operators need a plan without a node map (time-dependent or non-linear structure)"); return -1; }
+    if (p->large || p->sharded || p->state_sharded) { set_error(p, "per-member operators are not implemented for time-sharded, state-sharded or hilbert_size > 64 plans"); return -1; }
+    drop_graphs(p);
+    CU_TRY(p, cudaSetDevice(p->pb.device));
+    CU_TRY(p, cudaStreamSynchronize(p->stream));                          // no evaluation in flight reads G, C0 or Cs
+    const int n = p->pb.hilbert_size, NP = p->NP, E = p->pb.ensemble_count, KR = p->KC;
+    const size_t GM = 2 * (size_t)NP * NP, nn2 = 2 * (size_t)n * n;
+    bool herm = p->drift_hermitian;
+    for (size_t m = 0; m < (size_t)E * KR && herm; ++m) herm = host_is_hermitian(a_ops + m * nn2, n);
+    p->hermitian = herm && !no_nopiv();
+    std::vector<double> buf(std::max<size_t>(1, (size_t)E * KR) * GM);
+    for (size_t m = 0; m < (size_t)E * KR; ++m) to_planar(a_ops + m * nn2, buf.data() + m * GM, n, NP, true);
+    CU_TRY(p, p->G.alloc(buf.size()));
+    CU_TRY(p, cudaMemcpy(p->G.p, buf.data(), sizeof(double) * buf.size(), cudaMemcpyHostToDevice));
+    // product-free M4: C0[e][r] = [G0_e, G_{e,r}], Cs[e][s<r] = [G_{e,s}, G_{e,r}] from each member's own operators
+    if (p->comm_ok) {
+        const int npair = KR * (KR - 1) / 2;
+        CU_TRY(p, p->Cs.alloc(std::max<size_t>(1, (size_t)E * npair) * GM));
+        std::vector<double> g0p(GM), pl(GM), g0(nn2);
+        for (int e = 0; e < E; ++e) {
+            CU_TRY(p, cudaMemcpy(g0p.data(), p->G0.p + (size_t)e * GM, sizeof(double) * GM, cudaMemcpyDeviceToHost));
+            from_planar(g0p.data(), g0.data(), n, NP);                     // G0_e = -1j H0_e, as qocb_set_operators stored it
+            std::vector<HostMat> g(KR);
+            for (int r = 0; r < KR; ++r) g[r] = host_generator(a_ops + ((size_t)e * KR + r) * nn2, n);
+            for (int r = 0; r < KR; ++r) {
+                const HostMat c = host_commutator(g0, g[r], n);
+                to_planar(c.data(), pl.data(), n, NP, false);
+                CU_TRY(p, cudaMemcpy(p->C0.p + ((size_t)e * KR + r) * GM, pl.data(), sizeof(double) * GM, cudaMemcpyHostToDevice));
+            }
+            for (int s_ = 0; s_ < KR; ++s_)
+                for (int r = s_ + 1; r < KR; ++r) {
+                    const HostMat c = host_commutator(g[s_], g[r], n);
+                    to_planar(c.data(), pl.data(), n, NP, false);
+                    CU_TRY(p, cudaMemcpy(p->Cs.p + ((size_t)e * npair + comm_pair(s_, r, KR)) * GM, pl.data(), sizeof(double) * GM, cudaMemcpyHostToDevice));
+                }
+        }
+    }
+    p->member_ops = true;
     return 0;
 }
 

@@ -55,7 +55,7 @@ struct Smem {
 
 struct GenArgs {
     const double *G0;           // this member's drift generator, planar padded
-    const double *G;            // [KR][GMAT] control generators
+    const double *G;            // [KR][GMAT] control generators (per member: [E][KR][GMAT], this member's after the offset)
     const double *controls;     // [M][KR]
     const int *itab_idx;        // [N-1][q][2]
     const double *itab_w;       // [N-1][q][2]
@@ -65,6 +65,9 @@ struct GenArgs {
     // C0[r] = [G0, G_r] (per member) and Cs[(s<r)] = [G_s, G_r]; enabled for KR <= kMaxCommKR
     const double *C0, *Cs;
     int comm;
+    // member strides (doubles) of G and Cs: KR GMAT and npair GMAT when every member has its own control operators
+    // (qocb_set_member_operators), 0 when the members share them
+    long long g_stride, cs_stride;
     // time-dependent operators: channel coefficients of every local node, [slice][q][KR], precomputed by k_node_coefs
     // (KR then counts operator channels); nullptr = interpolate the controls here
     const double *nodecoef;

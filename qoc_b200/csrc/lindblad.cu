@@ -60,6 +60,7 @@ struct LArgs {
     int n, D, KR, M, N, L, ces, have_h, nterms, cap;
     double T;
     const double2 *H0, *Aops, *Lops, *Khalf;   // [n*n], [KR][n*n], [L][n*n], 1/2 sum_l gamma_l L^dag L
+    long long ops_stride;                       // member stride of Aops: KR n^2 with per-member operators, else 0
     const double *gam, *controls, *xs;
     const double2 *rho0;
     const DTerm *terms; const double2 *mats; const int *counts;
@@ -84,12 +85,14 @@ struct LArgs {
 };
 
 // the arguments of ensemble member blockIdx.x: per-member drift, K_half, rates, densities, tape, interval indices, global
-// work, cost, gradient, stats, stage time and tape-overflow flag sit at member-major offsets; rho0, operators, cost terms,
-// controls and the time series are shared.  Member 0 is the whole plan when E = 1.
+// work, cost, gradient, stats, stage time and tape-overflow flag sit at member-major offsets, and so do the control
+// operators when the members have their own (ops_stride > 0); rho0, Lindblad operators, cost terms, controls and the time
+// series are shared.  Member 0 is the whole plan when E = 1.
 __device__ __forceinline__ LArgs member_args(const LArgs &a0) {
     LArgs a = a0;
     const size_t e = blockIdx.x, nn = (size_t)a.n * a.n, DE = (size_t)a.D * nn;
     a.H0 += e * nn; a.Khalf += e * nn; a.gam += e * (size_t)max(a.L, 1);
+    a.Aops += e * a.ops_stride;
     a.states += e * a.N * DE;
     a.tape_x += e * a.cap; a.tape_h += e * a.cap; a.tape_y += e * a.cap * DE; a.tape_k1 += e * a.cap * DE;
     a.first += e * a.N; a.hit += e * a.N;
@@ -645,6 +648,7 @@ struct qocb_lplan {
     qocb_lindblad_problem pb;
     int E = 1;                                     // ensemble members (one CTA each)
     bool ens_set = false;                          // qocb_lindblad_set_ensemble since the last qocb_lindblad_set_operators
+    bool member_ops = false;                       // Aops holds [E][KR][n*n] (qocb_lindblad_set_member_operators)
     int cap = 0;                                   // tape capacity of one member
     bool ops_set = false, rho_set = false, costs_dirty = true, series_set = false;
     int NS = 0, segs = 0, deg = 0;                 // time series: NS = KC*(1+KR) + (time_dependent_rates ? L : 0)
@@ -669,10 +673,11 @@ int lfail(qocb_lplan *p, const char *msg, int rc) { if (p) p->err = msg; g_lerr 
 
 LArgs make_largs(qocb_lplan *p) {
     LArgs a;
+    const int n = p->pb.hilbert_size;
     a.n = p->pb.hilbert_size; a.D = p->pb.density_count; a.KR = p->pb.control_count; a.M = p->pb.control_eval_count;
     a.N = p->pb.system_eval_count; a.L = p->pb.lindblad_count; a.ces = p->pb.cost_eval_step; a.have_h = p->pb.have_hamiltonian;
     a.nterms = (int)p->h_terms.size(); a.cap = p->cap; a.T = p->pb.evolution_time;
-    a.H0 = p->H0.p; a.Aops = p->Aops.p; a.Lops = p->Lops.p; a.Khalf = p->Khalf.p; a.gam = p->gam.p; a.controls = p->controls.p;
+    a.H0 = p->H0.p; a.Aops = p->Aops.p; a.ops_stride = p->member_ops ? (long long)p->pb.control_count * n * n : 0; a.Lops = p->Lops.p; a.Khalf = p->Khalf.p; a.gam = p->gam.p; a.controls = p->controls.p;
     a.xs = p->xs.p; a.rho0 = p->rho0.p; a.terms = p->terms.p; a.mats = p->mats.p; a.counts = p->counts.p;
     a.states = p->states.p; a.cost = p->cost.p; a.tape_x = p->tape_x.p; a.tape_h = p->tape_h.p; a.tape_y = p->tape_y.p;
     a.tape_k1 = p->tape_k1.p; a.first = p->first.p; a.hit = p->hit.p; a.stats = p->stats.p; a.err_flag = p->err_flag.p;
@@ -882,6 +887,7 @@ int qocb_lindblad_set_operators(qocb_lplan *p, const double *h0, const double *a
         LTRY(p, cudaMemcpy(p->H0.p, h0, sizeof(double2) * nn, cudaMemcpyHostToDevice));
         if (KA > 0) LTRY(p, cudaMemcpy(p->Aops.p, a_ops, sizeof(double2) * (size_t)KA * nn, cudaMemcpyHostToDevice));
     }
+    p->member_ops = false;
     if (L > 0 && p->pb.time_dependent_rates) {                              // per-operator 1/2 B_l^dag B_l; rates come from the series
         if (!lops) return lfail(p, "lops missing", -1);
         LTRY(p, cudaMemcpy(p->Lops.p, lops, sizeof(double2) * (size_t)L * nn, cudaMemcpyHostToDevice));
@@ -935,6 +941,22 @@ int qocb_lindblad_set_ensemble(qocb_lplan *p, const double *h0s, const double *g
     LTRY(p, cudaMemcpy(p->gam.p, G.data(), sizeof(double) * G.size(), cudaMemcpyHostToDevice));
     LTRY(p, cudaMemcpy(p->Khalf.p, K.data(), sizeof(double) * K.size(), cudaMemcpyHostToDevice));
     p->ens_set = true;
+    p->tape_ok = false;
+    return 0;
+}
+
+/* a_ops: [E][KR][n][n], member e's control operators */
+int qocb_lindblad_set_member_operators(qocb_lplan *p, const double *a_ops) {
+    if (!p || !a_ops) return lfail(p, "null argument", -1);
+    if (!p->ops_set) return lfail(p, "qocb_lindblad_set_operators must come before qocb_lindblad_set_member_operators", -1);
+    if (!p->pb.have_hamiltonian || p->pb.channel_count > 0)
+        return lfail(p, "member operators need a time-independent hamiltonian (have_hamiltonian = 1, channel_count = 0)", -1);
+    LTRY(p, cudaSetDevice(p->pb.device));
+    const size_t count = (size_t)p->E * p->pb.control_count * p->pb.hilbert_size * p->pb.hilbert_size;
+    LTRY(p, cudaStreamSynchronize(p->stream));
+    LTRY(p, p->Aops.alloc(std::max<size_t>(1, count)));
+    if (count) LTRY(p, cudaMemcpy(p->Aops.p, a_ops, sizeof(double2) * count, cudaMemcpyHostToDevice));
+    p->member_ops = true;
     p->tape_ok = false;
     return 0;
 }

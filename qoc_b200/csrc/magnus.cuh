@@ -49,9 +49,10 @@ __global__ void __launch_bounds__(kMagThreads) k_magnus(GenArgs ga, int GMAT, in
         if (e != member) {                                  // operator slabs: drift-dependent ones per member, the rest once
             load_slab(0, ga.G0 + (size_t)e * GMAT);
             if (m4) for (int r = 0; r < KR; ++r) load_slab(1 + KR + r, ga.C0 + ((size_t)e * KR + r) * GMAT);
-            if (member < 0) {
-                for (int r = 0; r < KR; ++r) load_slab(1 + r, ga.G + (size_t)r * GMAT);
-                if (m4) for (int pr = 0; pr < KR * (KR - 1) / 2; ++pr) load_slab(1 + 2 * KR + pr, ga.Cs + (size_t)pr * GMAT);
+            if (member < 0 || ga.g_stride) {                // per-member control operators (g_stride > 0): also per member
+                const double *G = ga.G + e * ga.g_stride, *Cs = ga.Cs + e * ga.cs_stride;
+                for (int r = 0; r < KR; ++r) load_slab(1 + r, G + (size_t)r * GMAT);
+                if (m4) for (int pr = 0; pr < KR * (KR - 1) / 2; ++pr) load_slab(1 + 2 * KR + pr, Cs + (size_t)pr * GMAT);
             }
             member = e;
         }
