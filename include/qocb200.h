@@ -75,6 +75,25 @@ int qocb_set_operators(qocb_plan *plan, const double *h0, const double *a_ops);
    (channel_count > 0), time-sliced, state-sharded and hilbert_size > 64 plans.  A later qocb_set_operators returns
    the plan to shared operators.  Plans that never make this call allocate nothing for it. */
 int qocb_set_member_operators(qocb_plan *plan, const double *a_ops);
+/* CONTROL BATCHES (multi-start optimisation): B independent control sets [B][M][KR] of ONE problem - one hamiltonian,
+   one set of initial states and cost terms - evaluated in one launch sequence, each with its own cost and gradient.
+   Create the plan with ensemble_count = B and call qocb_set_control_batch before qocb_set_operators, which then takes
+   h0 [1][n][n]: the drift, the control operators and the commutators of the product-free M4 are stored once, so the
+   operator memory does not grow with B (the propagators, the tape, the states and the control / gradient buffers do).
+   Start b runs exactly the code of member b of an ensemble with start b's controls; its cost, gradient and final states
+   match a one-member plan given controls[b] to rounding (the split of the slices into chunks differs with B), and B = 1
+   is bit-identical to an ordinary plan.  Returns -1 once operators are set (so also for per-member operators), for
+   plans with a node map (channel_count > 0, time-dependent or non-linear hamiltonians), and for time-sliced,
+   state-sharded and hilbert_size > 64 plans; qocb_set_member_operators refuses a control batch.  On a control batch
+   qocb_cost, qocb_cost_and_grad, qocb_forward and qocb_backward return -1; qocb_upload_controls takes [B][M][KR] and
+   qocb_download_result returns costs [B] and grads [B][M][KR]; qocb_get_states / qocb_get_final_states are per start. */
+int qocb_set_control_batch(qocb_plan *plan);
+/* controls: [B][M][KR] real, costs: [B], final_states: [B][S][n] complex or NULL.  Like qocb_cost, the evaluation is
+   replayed as a CUDA graph from the third call on. */
+int qocb_batch_cost(qocb_plan *plan, const double *controls, double *costs, double *final_states);
+/* grads: [B][M][KR] real, start b's gradient only (no mean over starts) */
+int qocb_batch_cost_and_grad(qocb_plan *plan, const double *controls, double *costs, double *grads,
+                             double *final_states);
 /* Time-dependent hamiltonian(controls, time) (the callable's `time` argument, qoc/core/schroedingerdiscrete.py:483-486),
    affine in the controls: at Magnus node i of slice j
        H = H0 + sum_c coef[j][i][c] A_c,   coef[j][i][c] = offset[j][i][c] + sum_r gain[j][i][c][r] x_r(t_ji),

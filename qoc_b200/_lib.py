@@ -32,6 +32,7 @@ EXPORTS = [
     "qocb_lindblad_cost_and_grad", "qocb_lindblad_stats", "qocb_lindblad_get_densities", "qocb_lindblad_set_time_series",
     "qocb_lindblad_max_stage_time", "qocb_lindblad_forward", "qocb_lindblad_backward", "qocb_lindblad_set_ensemble",
     "qocb_lindblad_member_results", "qocb_set_member_operators", "qocb_lindblad_set_member_operators",
+    "qocb_set_control_batch", "qocb_batch_cost", "qocb_batch_cost_and_grad",
 ]
 
 
@@ -113,6 +114,9 @@ def load():
     lib.qocb_last_error.restype = C.c_char_p
     lib.qocb_set_operators.argtypes = [vp, vp, vp]
     lib.qocb_set_member_operators.argtypes = [vp, vp]
+    lib.qocb_set_control_batch.argtypes = [vp]
+    lib.qocb_batch_cost.argtypes = [vp, vp, vp, vp]
+    lib.qocb_batch_cost_and_grad.argtypes = [vp, vp, vp, vp, vp]
     lib.qocb_set_node_map.argtypes = [vp, vp, vp]
     lib.qocb_set_states.argtypes = [vp, vp]
     lib.qocb_add_cost.argtypes = [vp, i32, i32, dbl, vp, vp, i32]

@@ -319,13 +319,28 @@ class SchroedingerPlan(object):
                  magnus_policy=MagnusPolicy.M2, cost_eval_step=1,
                  interpolation_policy=InterpolationPolicy.LINEAR, device=0, store_tape=True,
                  chunks_per_member=0, ensemble_drifts=None, structure=None, slice_range=None, state_slice=None,
-                 ensemble_hamiltonians=None):
+                 ensemble_hamiltonians=None, control_batch=None):
         """`ensemble_drifts` [E][n][n] (members differ in the drift) or `ensemble_hamiltonians` [h_0 .. h_{E-1}] (callables
         like `hamiltonian`: members differ in the drift and the control operators, e.g. drive-amplitude or crosstalk errors)
-        make a robust-control ensemble: cost and gradient are the member mean, final and intermediate states per member."""
+        make a robust-control ensemble: cost and gradient are the member mean, final and intermediate states per member.
+
+        `control_batch=B` evaluates B independent control sets of this one problem per call (multi-start optimisation):
+        `cost(controls [B][M][K])` returns (errors [B], final states [B][S][n][1]), `cost_and_grad` also grads [B][M][K],
+        each start exactly what a one-member plan returns for its controls.  Not combinable with ensembles, sharding,
+        user-defined costs, time-dependent or non-linear hamiltonians, or n > 64 (NotImplementedError, before any device
+        call)."""
         if ensemble_drifts is not None and ensemble_hamiltonians is not None:
             raise ValueError("pass ensemble_drifts or ensemble_hamiltonians, not both")
         ensemble = ensemble_drifts is not None or ensemble_hamiltonians is not None
+        self.B = None
+        if control_batch is not None:
+            if isinstance(control_batch, bool) or not isinstance(control_batch, (int, np.integer)) or control_batch < 1:
+                raise ValueError("control_batch must be a positive integer, got {!r}".format(control_batch))
+            if ensemble:
+                raise NotImplementedError("control batches cannot be combined with ensemble_drifts / ensemble_hamiltonians")
+            if slice_range is not None or state_slice is not None:
+                raise NotImplementedError("control batches cannot be combined with time-slice or state sharding")
+            self.B = int(control_batch)
         if interpolation_policy != InterpolationPolicy.LINEAR:
             raise NotImplementedError("The interpolation policy {} is not yet supported for this method."
                                       "".format(interpolation_policy))
@@ -358,12 +373,25 @@ class SchroedingerPlan(object):
                                Cost.control_value_and_grad)
         if ensemble_hamiltonians is not None and any(user_cost(c) for c in self.costs):
             raise NotImplementedError("user-defined costs cannot be combined with ensembles or sharded plans")
+        if self.B is not None:
+            if any(user_cost(c) for c in self.costs):
+                raise NotImplementedError("user-defined costs cannot be combined with control batches")
+            if self.n > 64:
+                raise NotImplementedError("control batches are not implemented for hilbert_size > 64")
         if structure is None:
-            structure = extract_hamiltonian_structure(hamiltonian, self.K, self.complex_controls, evolution_time,
-                                                      system_eval_count=self.N, magnus_order=magnus_policy.order)
+            try:
+                structure = extract_hamiltonian_structure(hamiltonian, self.K, self.complex_controls, evolution_time,
+                                                          system_eval_count=self.N, magnus_order=magnus_policy.order)
+            except NonlinearHamiltonian as err:
+                if self.B is None:
+                    raise
+                # a plain NotImplementedError: make_schroedinger_plan must not route a batch to NonlinearSchroedingerPlan
+                raise NotImplementedError("control batches need a hamiltonian affine in the controls: {}".format(err)) from err
         self.structure = structure
         h0, a_ops = structure[0], structure[1]
         node_map = structure[2:] if len(structure) == 4 else None
+        if node_map is not None and self.B is not None:
+            raise NotImplementedError("control batches with a time-dependent hamiltonian are not supported")
         if node_map is not None and ensemble_drifts is not None:
             raise NotImplementedError("ensemble drifts with a time-dependent hamiltonian are not supported")
         if node_map is not None and ensemble_hamiltonians is not None:
@@ -380,7 +408,7 @@ class SchroedingerPlan(object):
                 member_ops, a_ops = a_ops, a_ops[0]
         else:
             h0s = np.ascontiguousarray(h0[None], dtype=np.complex128)
-        self.E = h0s.shape[0]
+        self.E = h0s.shape[0] if self.B is None else self.B
         pb = _lib.Problem(hilbert_size=self.n, state_count=self.S, control_count=self.KR,
                           control_eval_count=self.M, system_eval_count=self.N,
                           magnus_order=magnus_policy.order, cost_eval_step=int(cost_eval_step),
@@ -394,6 +422,8 @@ class SchroedingerPlan(object):
         handle = ctypes.c_void_p()
         _lib.check(self.lib.qocb_plan_create(ctypes.byref(pb), ctypes.byref(handle)))
         self.handle = handle
+        if self.B is not None:
+            _lib.check(self.lib.qocb_set_control_batch(handle), handle)
         a_ops = np.ascontiguousarray(a_ops, dtype=np.complex128)
         _lib.check(self.lib.qocb_set_operators(handle, _lib.ptr(h0s), _lib.ptr(a_ops) if a_ops.shape[0] else None), handle)
         if member_ops is not None:
@@ -456,7 +486,38 @@ class SchroedingerPlan(object):
 
     def _final_states(self, buf):
         fs = buf.reshape(self.E, self.S, self.n, 1)
-        return fs[0] if self.E == 1 else fs
+        return fs[0] if self.E == 1 and self.B is None else fs
+
+    def _batch_channels(self, controls):
+        """[B][M][K] controls -> [B][M][KR] real channels (complex: [Re u | Im u] per control step, as `_real_channels`)."""
+        controls = np.asarray(controls)
+        if controls.shape != (self.B, self.M, self.K):
+            raise ValueError("controls of a control batch must have shape {}".format((self.B, self.M, self.K)))
+        if self.complex_controls:
+            return np.ascontiguousarray(np.concatenate([controls.real, controls.imag], axis=2), dtype=np.float64)
+        return np.ascontiguousarray(controls, dtype=np.float64)
+
+    def _batch_eval(self, controls, want_grad):
+        """(errors [B], grads [B][M][K] or None, finals [B][S][n][1]); host control costs are added per start."""
+        x = self._batch_channels(controls)
+        controls = np.asarray(controls)
+        out = np.zeros(self.B)
+        fs = np.empty((self.B, self.S, self.n), dtype=np.complex128)
+        grads = None
+        if want_grad:
+            g = np.zeros((self.B, self.M, self.KR))
+            _lib.check(self.lib.qocb_batch_cost_and_grad(self.handle, _lib.ptr(x), _lib.ptr(out), _lib.ptr(g), _lib.ptr(fs)),
+                       self.handle)
+            grads = g[..., :self.K] + 1j * g[..., self.K:] if self.complex_controls else g
+        else:
+            _lib.check(self.lib.qocb_batch_cost(self.handle, _lib.ptr(x), _lib.ptr(out), _lib.ptr(fs)), self.handle)
+        errors = np.empty(self.B)
+        for b in range(self.B):
+            extra, extra_grad = self._control_costs(controls[b], want_grad)
+            errors[b] = float(out[b]) + extra
+            if extra_grad is not None:
+                grads[b] = grads[b] + extra_grad
+        return errors, grads, self._final_states(fs)
 
     # -- user-defined costs: value and cotangents by 4-point central differences of `cost(controls, states, step)` ---------
     def _user_value(self, controls, finals):
@@ -494,6 +555,9 @@ class SchroedingerPlan(object):
 
     # -- the seam ---------------------------------------------------------------------------------------
     def cost(self, controls):
+        if self.B is not None:
+            errors, _, finals = self._batch_eval(controls, False)
+            return errors, finals
         if self.user_costs:
             err, _, finals = self._eval_with_user_costs(controls, False)
             return err, finals
@@ -507,7 +571,9 @@ class SchroedingerPlan(object):
     def cost_and_grad(self, controls):
         """returns (error, grads, final_states); grads has controls' shape and dtype and is
         dE/dRe(u) + i dE/dIm(u) for complex controls (the value after the wrapper's conjugate,
-        schroedingerdiscrete.py:323-324)."""
+        schroedingerdiscrete.py:323-324).  A control batch returns (errors [B], grads [B][M][K], final_states)."""
+        if self.B is not None:
+            return self._batch_eval(controls, True)
         if self.user_costs:
             return self._eval_with_user_costs(controls, True)
         x = self._real_channels(controls)
@@ -554,20 +620,22 @@ class SchroedingerPlan(object):
         return buf
 
     def intermediate_states(self):
-        """[N][S][n][1] states of the last evaluation (member 0 unless E > 1: then [E][N][S][n][1])."""
+        """[N][S][n][1] states of the last evaluation (member 0 unless E > 1: then [E][N][S][n][1]; a control batch:
+        [B][N][S][n][1])."""
         buf = np.empty((self.E, self.N, self.S, self.n), dtype=np.complex128)
         _lib.check(self.lib.qocb_get_states(self.handle, _lib.ptr(buf)), self.handle)
         buf = buf[..., None]
-        return buf[0] if self.E == 1 else buf
+        return buf[0] if self.E == 1 and self.B is None else buf
 
     def propagators(self):
         buf = np.empty((self.E, self.N - 1, self.n, self.n), dtype=np.complex128)
         _lib.check(self.lib.qocb_get_propagators(self.handle, _lib.ptr(buf)), self.handle)
-        return buf[0] if self.E == 1 else buf
+        return buf[0] if self.E == 1 and self.B is None else buf
 
     # -- device-resident benchmarking hooks --------------------------------------------------------------
     def upload(self, controls):
-        _lib.check(self.lib.qocb_upload_controls(self.handle, _lib.ptr(self._real_channels(controls))), self.handle)
+        x = self._real_channels(controls) if self.B is None else self._batch_channels(controls)
+        _lib.check(self.lib.qocb_upload_controls(self.handle, _lib.ptr(x)), self.handle)
 
     def time_resident(self, with_grad=True, warmup=3, iters=10, flush_l2=True):
         total = np.zeros(1)

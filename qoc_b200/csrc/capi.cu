@@ -102,8 +102,8 @@ __global__ void __launch_bounds__(C::NT) k_forward(KArgs a, const __grid_constan
     for (int w = wb; w < we; ++w) {
         const int e = w / (a.N - 1), j = w - e * (a.N - 1);
         GenArgs ga = a.ga;
-        ga.G0 += (size_t)e * C::GMAT;
-        ga.C0 += (size_t)e * ga.KR * C::GMAT;
+        ga.G0 += e * ga.drift_stride;
+        ga.C0 += e * ga.KR * ga.drift_stride;
         PROF_DECL
         double *gU = a.U + (size_t)w * C::GMAT;
         double *gMnext = scratch + (size_t)S_E * C::GMAT;            // parked Magnus matrix (slot unused by the forward of M2 / M4)
@@ -115,9 +115,9 @@ __global__ void __launch_bounds__(C::NT) k_forward(KArgs a, const __grid_constan
             __syncthreads();
             parked = false;
         } else {
-            load_coefs<C>(sm, ga, j);
+            load_coefs<C>(sm, ga, j, e);
             if (magnus_pair_ok<C>(ga) && w + 1 < we) {
-                load_coefs_to<C>(sm.red, ga, j + 1);
+                load_coefs_to<C>(sm.red, ga, j + 1, e);                 // chunks never straddle members
                 magnus_forward_pair<C>(sm, member_ops(ga, e), sm.coef, sm.red, gMnext);
                 parked = true;
             } else {
@@ -183,9 +183,9 @@ __global__ void __launch_bounds__(C::NT) k_backward(KArgs a, const __grid_consta
         PROF_DECL
         const int e = w / (a.N - 1), j = w - e * (a.N - 1);
         GenArgs ga = a.ga;
-        ga.G0 += (size_t)e * C::GMAT;
-        ga.C0 += (size_t)e * ga.KR * C::GMAT;
-        load_coefs<C>(sm, ga, j);
+        ga.G0 += e * ga.drift_stride;
+        ga.C0 += e * ga.KR * ga.drift_stride;
+        load_coefs<C>(sm, ga, j, e);
         const double *tape; const int *piv; int s;
         if (a.tape && a.meta[w] <= a.s_cap) {
             tape = a.tape + (size_t)w * a.tape_mats * C::GMAT;
@@ -264,6 +264,19 @@ __global__ void k_gather_grad(const int *csr_ptr, const int *csr_idx, const doub
     grad[t] = sum / E;
 }
 
+// control batches: grad[b][m][r] = sum_{(j,i) using control point m} weight * node_grad[b][j][i][r], one thread per entry, the
+// CSR order of k_gather_grad and no member mean (E = 1 gives k_gather_grad's bits)
+__global__ void k_gather_grad_members(const int *csr_ptr, const int *csr_idx, const double *csr_w, const double *node_grad,
+                                      double *grad, int M, int KR, int q, int Nm1, int E) {
+    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= (long long)E * M * KR) return;
+    const int b = (int)(t / ((long long)M * KR)), mr = (int)(t - (long long)b * M * KR), m = mr / KR, r = mr % KR;
+    const double *ng = node_grad + (size_t)b * Nm1 * q * KR;
+    double sum = 0.;
+    for (int p = csr_ptr[m]; p < csr_ptr[m + 1]; ++p) sum += csr_w[p] * ng[(size_t)csr_idx[p] * KR + r];
+    grad[t] = sum;
+}
+
 // time-dependent operators: channel coefficients of every local node from the interpolated controls,
 // coef[ji][c] = off[ji][c] + sum_r gain[ji][c][r] x_r(t_ji)
 __global__ void k_node_coefs(const double *controls, const int *itab_idx, const double *itab_w, const double *off, const double *gain,
@@ -294,6 +307,15 @@ __global__ void k_finalize_cost(const double *cost_part, int nchunks, int E, dou
         for (int c = 0; c < nchunks; ++c) s += cost_part[c];
         *cost = s / E;
     }
+}
+
+// control batches: cost[e] = sum of member e's chunk costs in chunk order (E = 1 gives k_finalize_cost's bits)
+__global__ void k_member_cost(const double *cost_part, const int *member_chunk0, int E, double *cost) {
+    const int e = blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= E) return;
+    double s = 0.;
+    for (int c = member_chunk0[e]; c < member_chunk0[e + 1]; ++c) s += cost_part[c];
+    cost[e] = s;
 }
 
 template <class C>
@@ -557,7 +579,8 @@ struct qocb_plan {
     bool hermitian = false;             // H0 (every member) and every operator channel are Hermitian (QOCB_NO_NOPIV=1 clears it)
     bool drift_hermitian = false;       // H0 of every member is Hermitian (qocb_set_member_operators recomputes `hermitian`)
     bool member_ops = false;            // G, C0 and Cs hold every member's own control operators (qocb_set_member_operators)
-    double *h_pinned = nullptr;         // [M*KR controls | M*KR grad | 1 cost]
+    bool batch = false;                 // control batch (qocb_set_control_batch): member b has its own controls, cost and gradient
+    double *h_pinned = nullptr;         // [ctl_doubles controls | ctl_doubles grad | cost_count costs]
     // CUDA graph of one whole host-facing evaluation (H2D controls, all kernels, D2H of gradient, cost, final states and the
     // error flag): replayed by qocb_cost / qocb_cost_and_grad from the third call on - launch-bound small problems gain 2x
     cudaGraphExec_t gexec[2] = {nullptr, nullptr};
@@ -676,6 +699,8 @@ KArgs make_kargs(qocb_plan *p) {
     const long long GM = 2LL * p->NP * p->NP;
     a.ga.g_stride = p->member_ops ? p->KC * GM : 0;
     a.ga.cs_stride = p->member_ops && p->comm_ok ? p->KC * (p->KC - 1) / 2 * GM : 0;
+    a.ga.ctl_stride = p->batch ? (long long)p->pb.control_eval_count * p->pb.control_count : 0;
+    a.ga.drift_stride = p->batch ? 0 : GM;
     a.ga.dt = p->pb.evolution_time / (p->pb.system_eval_count - 1);
     a.N = p->Nloc; a.E = p->pb.ensemble_count;
     a.s_cap = kStoredTapeR; a.tape_mats = p->tape_mats;
@@ -1491,16 +1516,28 @@ int enqueue_expm_backward(qocb_plan *p, cudaEvent_t mid) {
     const int tot = p->pb.control_eval_count * p->pb.control_count;
     const double *ng = nullptr;
     rc = node_grad_for_gather(p, &ng); if (rc) return rc;
-    if (tot > 0)
+    if (tot > 0 && p->batch) {
+        const long long bt = (long long)tot * p->pb.ensemble_count;
+        k_gather_grad_members<<<(unsigned)((bt + 127) / 128), 128, 0, p->stream>>>(p->csr_ptr.p, p->csr_idx.p, p->csr_w.p, ng,
+                                                                              p->grad.p, p->pb.control_eval_count,
+                                                                              p->pb.control_count, p->q, p->Nloc - 1,
+                                                                              p->pb.ensemble_count);
+    } else if (tot > 0) {
         k_gather_grad<<<(tot + 127) / 128, 128, 0, p->stream>>>(p->csr_ptr.p, p->csr_idx.p, p->csr_w.p, ng,
                                                               p->grad.p, p->pb.control_eval_count, p->pb.control_count,
                                                               p->q, p->Nloc - 1, p->pb.ensemble_count);
+    }
     CU_TRY(p, cudaGetLastError());
     return 0;
 }
 
 int enqueue_finalize(qocb_plan *p) {
-    k_finalize_cost<<<1, 32, 0, p->stream>>>(p->cost_part.p, p->lvl_count[p->levels], p->pb.ensemble_count, p->cost.p);
+    if (p->batch) {
+        const int E = p->pb.ensemble_count;
+        k_member_cost<<<(E + 127) / 128, 128, 0, p->stream>>>(p->cost_part.p, make_sargs(p).member_chunk0, E, p->cost.p);
+    } else {
+        k_finalize_cost<<<1, 32, 0, p->stream>>>(p->cost_part.p, p->lvl_count[p->levels], p->pb.ensemble_count, p->cost.p);
+    }
     CU_TRY(p, cudaGetLastError());
     return 0;
 }
@@ -1531,6 +1568,13 @@ int enqueue_eval(qocb_plan *p, bool with_grad, cudaEvent_t *ev) {
     rec(7);
     return 0;
 }
+
+// doubles of the controls (and of the gradient) crossing the ABI, and the number of costs: [B][M][KR] and B for a control
+// batch, [M][KR] and 1 otherwise
+size_t ctl_doubles(const qocb_plan *p) {
+    return (size_t)(p->batch ? p->pb.ensemble_count : 1) * p->pb.control_eval_count * p->pb.control_count;
+}
+int cost_count(const qocb_plan *p) { return p->batch ? p->pb.ensemble_count : 1; }
 
 int check_device_flag(qocb_plan *p) {
     int flag = 0;
@@ -1826,7 +1870,8 @@ int qocb_set_operators(qocb_plan *p, const double *h0, const double *a_ops) {
     if (!p || !h0) { set_error(p, "null argument"); return -1; }
     drop_graphs(p);
     CU_TRY(p, cudaSetDevice(p->pb.device));
-    const int n = p->pb.hilbert_size, NP = p->NP, E = p->pb.ensemble_count, KR = p->KC;   // operator channels
+    const int n = p->pb.hilbert_size, NP = p->NP, KR = p->KC;   // operator channels
+    const int E = p->batch ? 1 : p->pb.ensemble_count;           // drifts: the members of a control batch share one
     const size_t GM = 2 * (size_t)NP * NP;
     auto is_hermitian = [&](const double *h) { return host_is_hermitian(h, n); };
     if (p->large) {                                    // interleaved generators G = -1j * H
@@ -1918,6 +1963,7 @@ int qocb_set_member_operators(qocb_plan *p, const double *a_ops) {
     if (!p->ops_set) { set_error(p, "qocb_set_member_operators needs qocb_set_operators first"); return -1; }
     if (p->mapped) { set_error(p, "per-member operators need a plan without a node map (time-dependent or non-linear structure)"); return -1; }
     if (p->large || p->sharded || p->state_sharded) { set_error(p, "per-member operators are not implemented for time-sharded, state-sharded or hilbert_size > 64 plans"); return -1; }
+    if (p->batch) { set_error(p, "the members of a control batch share their operators"); return -1; }
     drop_graphs(p);
     CU_TRY(p, cudaSetDevice(p->pb.device));
     CU_TRY(p, cudaStreamSynchronize(p->stream));                          // no evaluation in flight reads G, C0 or Cs
@@ -1954,6 +2000,30 @@ int qocb_set_member_operators(qocb_plan *p, const double *a_ops) {
         }
     }
     p->member_ops = true;
+    return 0;
+}
+
+int qocb_set_control_batch(qocb_plan *p) {
+    if (!p) { set_error(p, "null argument"); return -1; }
+    if (p->batch) return 0;
+    if (p->ops_set) { set_error(p, "qocb_set_control_batch must be called before qocb_set_operators"); return -1; }
+    if (p->mapped) { set_error(p, "control batches need a plan without a node map (time-dependent or non-linear structure)"); return -1; }
+    if (p->large || p->sharded || p->state_sharded) { set_error(p, "control batches are not implemented for time-sliced, state-sharded or hilbert_size > 64 plans"); return -1; }
+    drop_graphs(p);
+    CU_TRY(p, cudaSetDevice(p->pb.device));
+    CU_TRY(p, cudaStreamSynchronize(p->stream));
+    const int B = p->pb.ensemble_count;
+    const size_t GM = 2 * (size_t)p->NP * p->NP, cnt = std::max<size_t>(1, (size_t)B * p->pb.control_eval_count * p->pb.control_count);
+    // one shared drift (qocb_set_operators then takes h0 [1][n][n] and builds KR commutators); per start: controls, gradient, cost
+    CU_TRY(p, p->G0.alloc(GM));
+    CU_TRY(p, p->controls.alloc(cnt)); CU_TRY(p, p->grad.alloc(cnt)); CU_TRY(p, p->cost.alloc(B));
+    CU_TRY(p, cudaMemset(p->controls.p, 0, sizeof(double) * cnt));
+    CU_TRY(p, cudaMemset(p->grad.p, 0, sizeof(double) * cnt));
+    double *hp = nullptr;
+    CU_TRY(p, cudaMallocHost(&hp, sizeof(double) * (2 * cnt + B + 8)));
+    cudaFreeHost(p->h_pinned);
+    p->h_pinned = hp;
+    p->batch = true;
     return 0;
 }
 
@@ -2035,7 +2105,7 @@ int qocb_add_cost(qocb_plan *p, int32_t kind, int32_t step_cost, double weight, 
 int qocb_upload_controls(qocb_plan *p, const double *controls) {
     if (!p) return -1;
     CU_TRY(p, cudaSetDevice(p->pb.device));
-    const size_t cnt = (size_t)p->pb.control_eval_count * p->pb.control_count;
+    const size_t cnt = ctl_doubles(p);
     if (cnt == 0) return 0;
     if (!controls) { set_error(p, "controls is null"); return -1; }
     std::memcpy(p->h_pinned, controls, sizeof(double) * cnt);
@@ -2058,13 +2128,14 @@ int qocb_sync(qocb_plan *p) {
 int qocb_download_result(qocb_plan *p, double *cost, double *grad) {
     if (!p) return -1;
     CU_TRY(p, cudaSetDevice(p->pb.device));
-    const size_t cnt = (size_t)p->pb.control_eval_count * p->pb.control_count;
+    const size_t cnt = ctl_doubles(p);
+    const int nc = cost_count(p);
     double *hg = p->h_pinned + std::max<size_t>(1, cnt), *hc = hg + std::max<size_t>(1, cnt);
     if (grad && cnt) CU_TRY(p, cudaMemcpyAsync(hg, p->grad.p, sizeof(double) * cnt, cudaMemcpyDeviceToHost, p->stream));
-    CU_TRY(p, cudaMemcpyAsync(hc, p->cost.p, sizeof(double), cudaMemcpyDeviceToHost, p->stream));
+    CU_TRY(p, cudaMemcpyAsync(hc, p->cost.p, sizeof(double) * nc, cudaMemcpyDeviceToHost, p->stream));
     CU_TRY(p, cudaStreamSynchronize(p->stream));
     if (grad && cnt) std::memcpy(grad, hg, sizeof(double) * cnt);
-    if (cost) *cost = *hc;
+    if (cost) std::memcpy(cost, hc, sizeof(double) * nc);
     return check_device_flag(p);
 }
 
@@ -2086,14 +2157,14 @@ static int fetch_final_states(qocb_plan *p, double *final_states) {
 
 // everything one host-facing evaluation puts on the stream, in capture-safe form (async copies through pinned buffers)
 static int enqueue_host_eval(qocb_plan *p, bool with_grad) {
-    const size_t cnt = (size_t)p->pb.control_eval_count * p->pb.control_count;
+    const size_t cnt = ctl_doubles(p);
     const size_t VS = (size_t)p->pb.state_count * 2 * p->NP;
     const int N = p->Nloc, E = p->pb.ensemble_count;
     double *hg = p->h_pinned + std::max<size_t>(1, cnt), *hc = hg + std::max<size_t>(1, cnt);
     if (cnt) CU_TRY(p, cudaMemcpyAsync(p->controls.p, p->h_pinned, sizeof(double) * cnt, cudaMemcpyHostToDevice, p->stream));
     int rc = enqueue_eval(p, with_grad, nullptr); if (rc) return rc;
     if (with_grad && cnt) CU_TRY(p, cudaMemcpyAsync(hg, p->grad.p, sizeof(double) * cnt, cudaMemcpyDeviceToHost, p->stream));
-    CU_TRY(p, cudaMemcpyAsync(hc, p->cost.p, sizeof(double), cudaMemcpyDeviceToHost, p->stream));
+    CU_TRY(p, cudaMemcpyAsync(hc, p->cost.p, sizeof(double) * cost_count(p), cudaMemcpyDeviceToHost, p->stream));
     CU_TRY(p, cudaMemcpy2DAsync(p->h_fin, sizeof(double) * VS, p->psi.p + (size_t)(N - 1) * VS, sizeof(double) * N * VS,
                                 sizeof(double) * VS, E, cudaMemcpyDeviceToHost, p->stream));
     CU_TRY(p, cudaMemcpyAsync(p->h_flag, p->err_flag.p, sizeof(int), cudaMemcpyDeviceToHost, p->stream));
@@ -2110,7 +2181,7 @@ static int host_eval(qocb_plan *p, bool with_grad, const double *controls, doubl
         return fetch_final_states(p, final_states);
     }
     int rc = ready(p); if (rc) return rc;                          // synchronous uploads of changed cost tables: never captured
-    const size_t cnt = (size_t)p->pb.control_eval_count * p->pb.control_count;
+    const size_t cnt = ctl_doubles(p);
     if (cnt) {
         if (!controls) { set_error(p, "controls is null"); return -1; }
         std::memcpy(p->h_pinned, controls, sizeof(double) * cnt);
@@ -2139,7 +2210,7 @@ static int host_eval(qocb_plan *p, bool with_grad, const double *controls, doubl
     CU_TRY(p, cudaStreamSynchronize(p->stream));
     double *hg = p->h_pinned + std::max<size_t>(1, cnt), *hc = hg + std::max<size_t>(1, cnt);
     if (with_grad && grad && cnt) std::memcpy(grad, hg, sizeof(double) * cnt);
-    if (cost) *cost = *hc;
+    if (cost) std::memcpy(cost, hc, sizeof(double) * cost_count(p));
     if (*p->h_flag) { set_error(p, "device error flag set: scaling count exceeded the recompute tape capacity"); return -4; }
     if (final_states) {
         const int n = p->pb.hilbert_size, NP = p->NP, S = p->pb.state_count, E = p->pb.ensemble_count;
@@ -2154,17 +2225,36 @@ static int host_eval(qocb_plan *p, bool with_grad, const double *controls, doubl
     return 0;
 }
 
+static bool refuse_batch(qocb_plan *p, const char *call) {
+    if (!p || !p->batch) return false;
+    set_error(p, (std::string(call) + " serves [M][KR] controls and one cost: a control batch takes qocb_batch_cost / "
+                  "qocb_batch_cost_and_grad").c_str());
+    return true;
+}
+
 int qocb_cost(qocb_plan *p, const double *controls, double *cost, double *final_states) {
+    if (refuse_batch(p, "qocb_cost")) return -1;
     return host_eval(p, false, controls, cost, nullptr, final_states);
 }
 
 int qocb_cost_and_grad(qocb_plan *p, const double *controls, double *cost, double *grad, double *final_states) {
+    if (refuse_batch(p, "qocb_cost_and_grad")) return -1;
     return host_eval(p, true, controls, cost, grad, final_states);
+}
+
+int qocb_batch_cost(qocb_plan *p, const double *controls, double *costs, double *final_states) {
+    if (p && !p->batch) { set_error(p, "qocb_batch_cost needs a control batch (qocb_set_control_batch)"); return -1; }
+    return host_eval(p, false, controls, costs, nullptr, final_states);
+}
+
+int qocb_batch_cost_and_grad(qocb_plan *p, const double *controls, double *costs, double *grads, double *final_states) {
+    if (p && !p->batch) { set_error(p, "qocb_batch_cost_and_grad needs a control batch (qocb_set_control_batch)"); return -1; }
+    return host_eval(p, true, controls, costs, grads, final_states);
 }
 
 // ---- split evaluation: forward pass now, reverse pass later with an extra cotangent of the final states -------------------
 int qocb_forward(qocb_plan *p, const double *controls, double *cost, double *final_states) {
-    if (!p) return -1;
+    if (!p || refuse_batch(p, "qocb_forward")) return -1;
     if (p->sharded || p->state_sharded || p->pb.ensemble_count != 1) { set_error(p, "qocb_forward / qocb_backward need an unsharded single-member plan"); return -1; }
     CU_TRY(p, cudaSetDevice(p->pb.device));
     int rc = qocb_upload_controls(p, controls); if (rc) return rc;
@@ -2182,7 +2272,7 @@ int qocb_forward(qocb_plan *p, const double *controls, double *cost, double *fin
 }
 
 int qocb_backward(qocb_plan *p, const double *final_seed, double *grad) {
-    if (!p) return -1;
+    if (!p || refuse_batch(p, "qocb_backward")) return -1;
     if (p->sharded || p->state_sharded || p->pb.ensemble_count != 1) { set_error(p, "qocb_forward / qocb_backward need an unsharded single-member plan"); return -1; }
     CU_TRY(p, cudaSetDevice(p->pb.device));
     const int n = p->pb.hilbert_size, NP = p->large ? n : p->NP, S = p->pb.state_count;

@@ -68,6 +68,10 @@ struct GenArgs {
     // member strides (doubles) of G and Cs: KR GMAT and npair GMAT when every member has its own control operators
     // (qocb_set_member_operators), 0 when the members share them
     long long g_stride, cs_stride;
+    // member strides (doubles) of the controls and of the drift: a control batch (qocb_set_control_batch) gives every
+    // member its own [M][KR] controls (ctl_stride = M KR) and shares G0 / C0 (drift_stride = 0); otherwise ctl_stride = 0
+    // and drift_stride = GMAT (C0: KR drift_stride)
+    long long ctl_stride, drift_stride;
     // time-dependent operators: channel coefficients of every local node, [slice][q][KR], precomputed by k_node_coefs
     // (KR then counts operator channels); nullptr = interpolate the controls here
     const double *nodecoef;
@@ -75,20 +79,23 @@ struct GenArgs {
 constexpr int kMaxCommKR = 6;
 __host__ __device__ inline int comm_pair(int s, int r, int KR) { return s * KR - s * (s + 1) / 2 + (r - s - 1); }   // s < r
 
-// interpolated control coefficients of slice j at the Magnus nodes -> sm.coef[i*kMaxKR + r]
+// interpolated control coefficients of slice j of member `member` at the Magnus nodes -> sm.coef[i*kMaxKR + r]
 template <class C>
-__device__ __forceinline__ void load_coefs_to(double *dst, const GenArgs &ga, int j) {
+__device__ __forceinline__ void load_coefs_to(double *dst, const GenArgs &ga, int j, int member) {
+    const double *ctl = ga.controls + member * ga.ctl_stride;
     for (int e = threadIdx.x; e < ga.q * ga.KR; e += C::NT) {
         const int i = e / ga.KR, r = e % ga.KR;
         if (ga.nodecoef) { dst[i * kMaxKR + r] = ga.nodecoef[(size_t)(j * ga.q + i) * ga.KR + r]; continue; }
         const int *id = ga.itab_idx + (j * ga.q + i) * 2;
         const double *w = ga.itab_w + (j * ga.q + i) * 2;
-        dst[i * kMaxKR + r] = ga.controls[id[0] * ga.KR + r] * w[0] + ga.controls[id[1] * ga.KR + r] * w[1];
+        dst[i * kMaxKR + r] = ctl[id[0] * ga.KR + r] * w[0] + ctl[id[1] * ga.KR + r] * w[1];
     }
     __syncthreads();
 }
 template <class C>
-__device__ __forceinline__ void load_coefs(const Smem<C> &sm, const GenArgs &ga, int j) { load_coefs_to<C>(sm.coef, ga, j); }
+__device__ __forceinline__ void load_coefs(const Smem<C> &sm, const GenArgs &ga, int j, int member) {
+    load_coefs_to<C>(sm.coef, ga, j, member);
+}
 
 // owned pair of  alpha0 * G0 + sum_r cf[r] * G_r
 template <class C>

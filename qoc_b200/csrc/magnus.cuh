@@ -47,8 +47,11 @@ __global__ void __launch_bounds__(kMagThreads) k_magnus(GenArgs ga, int GMAT, in
         const int cnt = (int)min((long long)kMagTile, min(wend - w0, (long long)(Nm1 - j0)));
         __syncthreads();                                    // the previous tile is done with ops / wts
         if (e != member) {                                  // operator slabs: drift-dependent ones per member, the rest once
-            load_slab(0, ga.G0 + (size_t)e * GMAT);
-            if (m4) for (int r = 0; r < KR; ++r) load_slab(1 + KR + r, ga.C0 + ((size_t)e * KR + r) * GMAT);
+            if (member < 0 || ga.drift_stride) {            // a control batch (drift_stride = 0) shares the drift too
+                const double *G0 = ga.G0 + e * ga.drift_stride, *C0 = ga.C0 + e * KR * ga.drift_stride;
+                load_slab(0, G0);
+                if (m4) for (int r = 0; r < KR; ++r) load_slab(1 + KR + r, C0 + (size_t)r * GMAT);
+            }
             if (member < 0 || ga.g_stride) {                // per-member control operators (g_stride > 0): also per member
                 const double *G = ga.G + e * ga.g_stride, *Cs = ga.Cs + e * ga.cs_stride;
                 for (int r = 0; r < KR; ++r) load_slab(1 + r, G + (size_t)r * GMAT);
@@ -57,13 +60,14 @@ __global__ void __launch_bounds__(kMagThreads) k_magnus(GenArgs ga, int GMAT, in
             member = e;
         }
         // weights of the tile: wts[c][jj]
+        const double *ctl = ga.controls + e * ga.ctl_stride;
         for (int idx = tid; idx < cnt * nops; idx += kMagThreads) {
             const int jj = idx / nops, c = idx - jj * nops, j = j0 + jj;
             auto coef = [&](int node, int r) -> double {
                 if (ga.nodecoef) return ga.nodecoef[(size_t)(j * q + node) * KR + r];
                 const int *id = ga.itab_idx + (j * q + node) * 2;
                 const double *iw = ga.itab_w + (j * q + node) * 2;
-                return ga.controls[id[0] * KR + r] * iw[0] + ga.controls[id[1] * KR + r] * iw[1];
+                return ctl[id[0] * KR + r] * iw[0] + ctl[id[1] * KR + r] * iw[1];
             };
             double wv;
             if (c == 0) wv = dt;
