@@ -58,7 +58,7 @@ struct KArgs {
     double *node_grad;          // [E*(N-1)][q][KR]
     int S;
     int lowrank;                // 1: use the rank-S reverse pass where it applies (QOCB_NO_LOWRANK=1 disables it)
-    int herm;                   // 1: every operator is Hermitian => anti-Hermitian Magnus matrices (pivot-free LU where safe)
+    int herm;                   // 1: every operator is Hermitian => anti-Hermitian Magnus matrices (pivot-free Pade inverse where safe)
     int tape_min;               // 1: slices without squarings keep {A, A2, LU} only (Krylov reverse pass, lowrank == 2)
     int post_adj;               // 1: slices replayed from the stored tape leave mbar in their A slot; k_magnus_adj does the Magnus adjoint
     int *err_flag;
@@ -462,7 +462,7 @@ HostMat host_commutator(const HostMat &x, const HostMat &y, int n) {   // [x, y]
         }
     return c;
 }
-// Hermitian to 1e-13 of the largest entry: selects the pivot-free LU where it is safe (tile.cuh)
+// Hermitian to 1e-13 of the largest entry: selects the pivot-free Pade inverse where it is safe (tile.cuh)
 bool host_is_hermitian(const double *h, int n) {
     double mx = 0., dev = 0.;
     for (int r = 0; r < n; ++r)
@@ -1913,7 +1913,7 @@ int qocb_set_operators(qocb_plan *p, const double *h0, const double *a_ops) {
         p->ops_set = true;
         return 0;
     }
-    {   // Hermitian operators => anti-Hermitian generators: selects the pivot-free LU where it is safe (tile.cuh)
+    {   // Hermitian operators => anti-Hermitian generators: selects the pivot-free Pade inverse where it is safe (tile.cuh)
         auto is_herm = is_hermitian;
         bool herm = true;
         for (int e = 0; e < E && herm; ++e) herm = is_herm(h0 + (size_t)e * 2 * n * n);

@@ -27,6 +27,10 @@ __device__ __constant__ double kB[14] = {
 
 // tape slots (each GMAT doubles)
 enum { T_A = 0, T_A2, T_A4, T_A6, T_W1, T_X1, T_Y, T_LU, T_R = 8 };
+// The T_LU slot holds the inverse of the Pade denominator (pivot-free slices, tile.cuh: gj_invert_nopiv) or its LUi factors;
+// the slice's permutation row says which: kTapeInverse in every entry for Q^-1, the row permutation of the LU otherwise.
+constexpr int kTapeInverse = -1;
+__device__ __forceinline__ bool tape_holds_inverse(const int *tpiv) { return tpiv[0] == kTapeInverse; }
 // CTA scratch slots
 enum { S_A = 0, S_A2, S_A4, S_A6, S_B3, S_C12, S_E, S_P, S_QM, S_T0, S_T1, S_T2, S_T3, S_COUNT };
 
@@ -278,10 +282,11 @@ __device__ void magnus_forward_pair(const Smem<C> &sm, const GenArgs &ga, const 
 // ---------------------------------------------------------------------------------------------------------
 // Pade-13 forward.  In: M in X2.  Out: U = expm(M) in X1 (all threads past a barrier); returns s.
 // tape: 8 + s matrices are written when tape != nullptr (T_R + i holds R_i for i < s); piv_out: int[NP].
-// Asynchronous feed of k_forward (tma.cuh).  While the substitutions and squarings of this slice run, pade_forward starts
-//   * the chunk propagator (matrix idxP of mapP) into X1 as soon as the solve has consumed its right-hand side - only when
-//     the slice needs no squarings, because then U stays in X0 and X1 is free until the chunk product;
-//   * the next slice's Magnus matrix (matrix idxM of mapM) into X2 once the LU factors have gone to the tape.
+// Asynchronous feed of k_forward (tma.cuh).  While the end of this slice runs, pade_forward starts
+//   * the chunk propagator (matrix idxP of mapP) into X1 as soon as R0 = Q^-1 P no longer reads P (after the product with
+//     Q^-1, or after the solve's permuted copy of its right-hand side) - only when the slice needs no squarings, because
+//     then U stays in X0 and X1 is free until the chunk product;
+//   * the next slice's Magnus matrix (matrix idxM of mapM) into X2 once Q^-1 or the LU factors have gone to the tape.
 // Negative indices skip a fetch.  fetchedP reports whether the propagator fetch was issued.
 struct Feed {
     const CUtensorMap *mapM, *mapP;
@@ -291,8 +296,8 @@ struct Feed {
 };
 
 // u_out != nullptr: the caller accepts U in X0 when no squarings are needed (*u_out = X0 or X1); otherwise U is in X1.
-// herm != 0: the argument is anti-Hermitian (Hermitian operators): slices with ||A||_1 < QOCB_NOPIV_NORM factor the Pade
-// denominator without pivoting (tile.cuh: lu_factor_blocked_nopiv).
+// herm != 0: the argument is anti-Hermitian (Hermitian operators): slices with ||A||_1 < QOCB_NOPIV_NORM and no squarings
+// invert the Pade denominator without pivoting (tile.cuh: gj_invert_nopiv) and form R0 = Q^-1 P as one product.
 #define QOCB_NOPIV_NORM 2.5
 template <class C>
 __device__ int pade_forward(const Smem<C> &sm, double *tape, int *piv_out, double *tmpY, double *tmpV, int s_cap,
@@ -494,21 +499,31 @@ __device__ int pade_forward(const Smem<C> &sm, double *tape, int *piv_out, doubl
         __syncthreads();
     }
     PROF_MARK(3);
-    if (herm && s == 0 && norm < QOCB_NOPIV_NORM) lu_factor_blocked_nopiv<C>(sm.X2, sm.piv);
-    else lu_factor_blocked<C>(sm.X2, sm.piv, sm.piv + C::NP);
-    PROF_MARK(4);
+    const bool inverse = herm && s == 0 && norm < QOCB_NOPIV_NORM;
     {
         const bool feedP = feed != nullptr && feed->idxP >= 0 && s == 0;
         if (feed) feed->fetchedP = feedP;
         auto b_free = [&]() {
             if (feedP && threadIdx.x == 0) tma_fetch_matrix<C::NP>(sm.X1, feed->mapP, feed->idxP, feed->barP);
         };
-        lu_solve_blocked<C, false>(sm.X2, sm.piv, sm.X1, sm.X0, b_free);   // R0 = Q^-1 P in X0 (Y is dead)
+        if (inverse) {
+            gj_invert_nopiv<C>(sm.X2, sm.X0);                           // Q^-1 in X2 (X0: scratch, Y is dead)
+            PROF_MARK(19);
+            acc.zero(); mma_smem<C, false, false, false>(acc, sm.X2, sm.X1);   // R0 = Q^-1 P
+            for_owned<C>([&](int i, int j, int row, int col) { sts2<C>(sm.X0, row, col, accv<C>(acc, i, j)); });
+            __syncthreads();
+            b_free();
+            PROF_MARK(25);
+        } else {
+            lu_factor_blocked<C>(sm.X2, sm.piv, sm.piv + C::NP);
+            PROF_MARK(4);
+            lu_solve_blocked<C, false>(sm.X2, sm.piv, sm.X1, sm.X0, b_free);   // R0 = Q^-1 P in X0 (Y is dead)
+            PROF_MARK(5);
+        }
     }
-    PROF_MARK(5);
     if (keep) {
-        s2g<C>(tape + (size_t)T_LU * C::GMAT, sm.X2);                   // LUi format (tile.cuh) + row permutation
-        for (int c = threadIdx.x; c < C::NP; c += C::NT) piv_out[c] = sm.piv[c];
+        s2g<C>(tape + (size_t)T_LU * C::GMAT, sm.X2);                   // Q^-1, or the LUi factors (tile.cuh) + row permutation
+        for (int c = threadIdx.x; c < C::NP; c += C::NT) piv_out[c] = inverse ? kTapeInverse : sm.piv[c];
     }
     if (feed != nullptr && feed->idxM >= 0) {                           // X2 is dead from here on
         __syncthreads();
@@ -559,7 +574,14 @@ __device__ void pade_backward(const Smem<C> &sm, const double *tape, const int *
     g2s<C>(sm.X1, s > 0 ? tape + (size_t)T_R * C::GMAT : gU);
     __syncthreads();
     PROF_MARK(10);
-    lu_solve_blocked<C, true>(sm.X2, sm.piv, sm.X0, sm.X2);             // X2 = pbar = Q^-T rbar (over the dead LU)
+    if (tape_holds_inverse(tpiv)) {
+        acc.zero(); mma_smem<C, true, false, false>(acc, sm.X2, sm.X0);  // pbar = (Q^-1)^T rbar
+        __syncthreads();
+        for_owned<C>([&](int i, int j, int row, int col) { sts2<C>(sm.X2, row, col, accv<C>(acc, i, j)); });
+        __syncthreads();
+    } else {
+        lu_solve_blocked<C, true>(sm.X2, sm.piv, sm.X0, sm.X2);         // X2 = pbar = Q^-T rbar (over the dead LU)
+    }
     PROF_MARK(11);
     acc.zero(); mma_smem<C, false, true, false>(acc, sm.X2, sm.X1);      // pbar R0^T = -qbar
     __syncthreads();
@@ -688,18 +710,30 @@ __device__ void pade_backward_lowrank(const Smem<C> &sm, const double *tape, con
     for (int c = threadIdx.x; c < NP; c += C::NT) sm.piv[c] = tperm[c];
     pf_load(tape + (size_t)T_Y * C::GMAT);
     __syncthreads();
-    // ---- stage 1: l = Q^-T lam (thin solve), row un-permutation through RIGHT
-    lu_solve_thin_T<C>(X0, LEFT);
-    for (int e = threadIdx.x; e < NP * 4; e += C::NT) {
-        const int row = e >> 2, c = e & 3, pr = sm.piv[row];
-        RIGHT[pr * LD + c] = LEFT[row * LD + 4 + c]; RIGHT[PL + pr * LD + c] = LEFT[PL + row * LD + 4 + c];
-    }
-    pf_store(X0);                                                   // Y
-    pf_load(tape + (size_t)T_A * C::GMAT);
-    __syncthreads();
-    for (int e = threadIdx.x; e < NP * 4; e += C::NT) {
-        const int row = e >> 2, c = e & 3;
-        LEFT[row * LD + 4 + c] = RIGHT[row * LD + c]; LEFT[PL + row * LD + 4 + c] = RIGHT[PL + row * LD + c];
+    // ---- stage 1: l = Q^-T lam -> LEFT[:, 4:8]: one thin product with Q^-1, or the thin solve and the row un-permutation
+    if (tape_holds_inverse(tperm)) {
+        const c2 v = thin_tile<C, true, LD, PL>(X0, LEFT, warp, 0);
+        __syncthreads();
+        if (t >= 2) {
+            *reinterpret_cast<double2 *>(LEFT + frow * LD + 2 * t) = make_double2(v.r0, v.r1);
+            *reinterpret_cast<double2 *>(LEFT + PL + frow * LD + 2 * t) = make_double2(v.i0, v.i1);
+        }
+        pf_store(X0);                                               // Y
+        pf_load(tape + (size_t)T_A * C::GMAT);
+        __syncthreads();
+    } else {
+        lu_solve_thin_T<C>(X0, LEFT);
+        for (int e = threadIdx.x; e < NP * 4; e += C::NT) {
+            const int row = e >> 2, c = e & 3, pr = sm.piv[row];
+            RIGHT[pr * LD + c] = LEFT[row * LD + 4 + c]; RIGHT[PL + pr * LD + c] = LEFT[PL + row * LD + 4 + c];
+        }
+        pf_store(X0);                                               // Y
+        pf_load(tape + (size_t)T_A * C::GMAT);
+        __syncthreads();
+        for (int e = threadIdx.x; e < NP * 4; e += C::NT) {
+            const int row = e >> 2, c = e & 3;
+            LEFT[row * LD + 4 + c] = RIGHT[row * LD + c]; LEFT[PL + row * LD + 4 + c] = RIGHT[PL + row * LD + c];
+        }
     }
     // ---- stage 2: yp = Y p -> TMP[:, 8:12]
     {
@@ -891,17 +925,28 @@ __device__ void pade_backward_krylov(const Smem<C> &sm, const TapeFeed &tf, cons
     __syncthreads();
     tape_wait(tf, tf.bar0, tf.ph0);
     PROF_MARK(43);
-    // ---- stage 1: l = Q^-T lam (thin solve on PP1[:, 0:8]); the LU factors are dead afterwards: A2 -> X0
-    lu_solve_thin_T<C, TLD, TPL>(X0, PP1);
-    tape_fetch<C>(tf, X0, T_A2, tf.bar0);
-    for (int e = threadIdx.x; e < NP * 4; e += C::NT) {             // row un-permutation through EL
-        const int row = e >> 2, c = e & 3, pr = sm.piv[row];
-        EL[pr * ELD + c] = PP1[row * TLD + 4 + c]; EL[EPL + pr * ELD + c] = PP1[TPL + row * TLD + 4 + c];
-    }
-    __syncthreads();
-    for (int e = threadIdx.x; e < NP * 4; e += C::NT) {
-        const int row = e >> 2, c = e & 3;
-        PP1[row * TLD + 4 + c] = EL[row * ELD + c]; PP1[TPL + row * TLD + 4 + c] = EL[EPL + row * ELD + c];
+    // ---- stage 1: l = Q^-T lam -> PP1[:, 4:8]: one thin product with Q^-1, or the thin solve on PP1[:, 0:8] and the row
+    // un-permutation; Q^-1 / the LU factors are dead afterwards: A2 -> X0
+    if (tape_holds_inverse(tperm)) {
+        const c2 v = thin_tile<C, true, TLD, TPL>(X0, PP1, warp, 0);
+        __syncthreads();
+        tape_fetch<C>(tf, X0, T_A2, tf.bar0);
+        if (t >= 2) {
+            *reinterpret_cast<double2 *>(PP1 + frow * TLD + 2 * t) = make_double2(v.r0, v.r1);
+            *reinterpret_cast<double2 *>(PP1 + TPL + frow * TLD + 2 * t) = make_double2(v.i0, v.i1);
+        }
+    } else {
+        lu_solve_thin_T<C, TLD, TPL>(X0, PP1);
+        tape_fetch<C>(tf, X0, T_A2, tf.bar0);
+        for (int e = threadIdx.x; e < NP * 4; e += C::NT) {         // row un-permutation through EL
+            const int row = e >> 2, c = e & 3, pr = sm.piv[row];
+            EL[pr * ELD + c] = PP1[row * TLD + 4 + c]; EL[EPL + pr * ELD + c] = PP1[TPL + row * TLD + 4 + c];
+        }
+        __syncthreads();
+        for (int e = threadIdx.x; e < NP * 4; e += C::NT) {
+            const int row = e >> 2, c = e & 3;
+            PP1[row * TLD + 4 + c] = EL[row * ELD + c]; PP1[TPL + row * TLD + 4 + c] = EL[EPL + row * ELD + c];
+        }
     }
     __syncthreads();
     tape_wait(tf, tf.bar1, tf.ph1);

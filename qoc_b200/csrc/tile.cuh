@@ -319,7 +319,7 @@ __device__ __forceinline__ cplx crecip(cplx a) {
 // Semantics of zgesv (qoc/standard/functions/expm.py:246 -> numpy.linalg.solve -> LAPACK zgetrf/zgetrs): row
 // pivoting with pivot = first row maximising |re| + |im| (izamax).  Block size 8 = one DMMA tile.
 //
-// Storage after lu_factor_blocked ("LUi" format, also what the reverse-pass tape holds):
+// Storage after lu_factor_blocked ("LUi" format, also what the reverse-pass tape holds for pivoted slices):
 //   * off-diagonal blocks: L (below) and U (above) as usual;
 //   * every 8 x 8 diagonal block holds the INVERSES of its triangular factors: strictly lower part = strictly lower
 //     part of inv(L_kk) (unit diagonal implied), upper part incl. diagonal = inv(U_kk).  Triangular solves then are
@@ -561,66 +561,35 @@ __device__ void lu_factor_blocked(double *Q, int *perm, int *piv8) {
     }
 }
 
-// ---- blocked LU WITHOUT pivoting -------------------------------------------------------------------------------------
+// ---- inverse of the Pade denominator WITHOUT pivoting ----------------------------------------------------------------
 // For an anti-Hermitian argument A = -i H dt (every physical GRAPE problem: H0 and the control operators are Hermitian)
 // the Pade denominator Q = V - U is a polynomial of A with real coefficients: it is a normal matrix with eigenvalues
 // q(i lam) = b0 e^{-i lam / 2} (1 + O(1e-10)) for the eigenvalues i lam of A, so its Hermitian part is b0 cos(lam / 2) > 0
-// as long as |lam| <= ||A||_1 < pi.  A matrix with a positive definite Hermitian part has an LU factorisation without
-// pivoting whose growth is bounded (Golub & Van Loan, sec. 4.2.2: || |L||U| || <= n (||T|| + ||S T^-1 S||), T, S the
-// Hermitian / skew parts), i.e. it is backward stable, and zgesv's row exchanges buy nothing.  pade_forward takes this path
-// when the plan's operators are Hermitian and ||A||_1 < 2.5 (cos(1.25) = 0.32: growth below ~4); everything else goes
-// through the pivoted factorisation above.  Same LUi storage, identity permutation - the solves and the reverse pass
-// do not know the difference.
-// What it removes: the single-warp pivot search over the whole panel column (REDUX + broadcasts on 64 rows, the row
-// position bookkeeping, the row swaps of every column tile).  Per panel only the 8 x 8 diagonal block is factored by one
-// warp; L21 = A21 inv(U11) and U12 = inv(L11) A12 are DMMA tile products spread over all warps.
+// as long as |lam| <= ||A||_1 < pi.  A matrix with a positive definite Hermitian part can be eliminated without pivoting
+// with bounded growth (Golub & Van Loan, sec. 4.2.2: every Schur complement keeps a positive definite Hermitian part), and
+// over the range pade_forward admits here (Hermitian operators, ||A||_1 < 2.5, no squarings) the Pade-13 coefficients give
+// 1 <= |q(i lam)| / b0 <= 1.032, i.e. cond_2(Q) <= 1.032.  An explicit inverse is then as accurate as a solve, and
+// R0 = Q^-1 P is one dense product instead of two dependent block substitutions; the reverse passes apply Q^-T as a product
+// too.  Everything else goes through the pivoted factorisation above.
 
-// acc (8 x 8 tile) += A[ar0:+8, ak0:+8] * maskU(B[bk0:+8, bc0:+8]); maskU keeps the upper triangle incl. the diagonal of the
-// STORED block (the inv(U_kk) half of an LUi diagonal block)
-template <class C>
-__device__ __forceinline__ void tile_mma_bupper(c2 &acc, const double *A, int ar0, int ak0, const double *B, int bk0, int bc0) {
-    const int lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
-    double p1a = 0., p1b = 0., p2a = 0., p2b = 0., p3a = 0., p3b = 0.;
-#pragma unroll
-    for (int ks = 0; ks < 2; ++ks) {
-        const int aidx = (ar0 + g) * C::LD + ak0 + 4 * ks + t;
-        const double ar = A[aidx], ai = A[C::PLANE + aidx];
-        const int bidx = (bk0 + 4 * ks + t) * C::LD + bc0 + g;
-        double br = B[bidx], bi = B[C::PLANE + bidx];
-        if (4 * ks + t > g) { br = 0.; bi = 0.; }                  // stored row > stored column: the inv(L) half
-        dmma884(p1a, p1b, ar, br);
-        dmma884(p2a, p2b, ai, bi);
-        dmma884(p3a, p3b, ar + ai, br + bi);
-    }
-    acc.r0 += p1a - p2a; acc.r1 += p1b - p2b;
-    acc.i0 += p3a - p1a - p2a; acc.i1 += p3b - p1b - p2b;
-}
-
-// One warp: unpivoted LU of the 8 x 8 diagonal block at (j0, j0) and the inverses of its factors, in place (LUi format).
-// The block lives in registers in the DMMA accumulator layout - lane (g, t) holds row g, columns 2t and 2t + 1 - so all
-// 32 lanes work on every elimination step (8 shuffles + 8 DFMA per lane and step for the block; the dependent chain per
-// step is one pivot broadcast, the reciprocal (hardware seed + two Newton steps) and one complex multiply-add).
-//   * forward elimination runs on [A | Z], Z = I: afterwards A holds U (upper) and the multipliers (lower), Z = inv(L);
-//   * a backward (Jordan) sweep on Y = I with the rows scaled by 1 / u_jj gives Y = inv(U).
-// No pivoting: see the note above for when that is safe.
+// One warp: Gauss-Jordan inverse of an 8 x 8 tile held in the DMMA accumulator layout (lane (g, t): row g, columns 2t, 2t + 1),
+// no pivoting.  Step j scales row j by 1 / a_jj and eliminates column j from every other row of [A | Z], Z = I at the start;
+// the dependent chain per step is one pivot broadcast, the reciprocal (hardware seed + two Newton steps) and one complex
+// multiply-add.  Columns of A that have been eliminated are not read again and are left as they come out.
 __device__ __forceinline__ c2 shfl_c2(const c2 &v, int src) {
     constexpr unsigned FULL = 0xffffffffu;
     return {__shfl_sync(FULL, v.r0, src), __shfl_sync(FULL, v.r1, src), __shfl_sync(FULL, v.i0, src), __shfl_sync(FULL, v.i1, src)};
 }
-template <class C>
-__device__ void lu_diag_warp(double *Q, int j0) {
+__device__ __forceinline__ c2 gj_tile_inverse(c2 a) {
     constexpr unsigned FULL = 0xffffffffu;
     const int lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
-    c2 a = ld_ctile<C>(Q, j0, j0);
     c2 z = {g == 2 * t ? 1.0 : 0.0, g == 2 * t + 1 ? 1.0 : 0.0, 0., 0.};
-    c2 y = z;
-    cplx dinv[8];
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
         const int tj = j >> 1;
         const bool odd = (j & 1) != 0;
-        const double sr = odd ? a.r1 : a.r0, si = odd ? a.i1 : a.i0;     // this lane's entry of column j (if it owns one)
-        const double pr = __shfl_sync(FULL, sr, 4 * j + tj), pi = __shfl_sync(FULL, si, 4 * j + tj);      // u_jj
+        const double sr = odd ? a.r1 : a.r0, si = odd ? a.i1 : a.i0;     // this lane's entry of column j
+        const double pr = __shfl_sync(FULL, sr, 4 * j + tj), pi = __shfl_sync(FULL, si, 4 * j + tj);      // a_jj
         const double er = __shfl_sync(FULL, sr, 4 * g + tj), ei = __shfl_sync(FULL, si, 4 * g + tj);      // a_gj
         const c2 u = shfl_c2(a, 4 * j + t), w = shfl_c2(z, 4 * j + t);                                      // row j of A and Z
         const double nn = pr * pr + pi * pi;
@@ -629,85 +598,74 @@ __device__ void lu_diag_warp(double *Q, int j0) {
         dn = fma(dn, fma(-nn, dn, 1.0), dn);
         dn = fma(dn, fma(-nn, dn, 1.0), dn);
         const cplx inv = {pr * dn, -pi * dn};
-        dinv[j] = inv;
-        if (g > j) {
-            const cplx l = cmul({er, ei}, inv);
-            if (2 * t > j) { a.r0 -= l.r * u.r0 - l.i * u.i0; a.i0 -= l.r * u.i0 + l.i * u.r0; }
-            else if (2 * t == j) { a.r0 = l.r; a.i0 = l.i; }
-            if (2 * t + 1 > j) { a.r1 -= l.r * u.r1 - l.i * u.i1; a.i1 -= l.r * u.i1 + l.i * u.r1; }
-            else if (2 * t + 1 == j) { a.r1 = l.r; a.i1 = l.i; }
-            z.r0 -= l.r * w.r0 - l.i * w.i0; z.i0 -= l.r * w.i0 + l.i * w.r0;
-            z.r1 -= l.r * w.r1 - l.i * w.i1; z.i1 -= l.r * w.i1 + l.i * w.r1;
-        }
+        // row j: x <- x / a_jj; other rows: x <- x - (a_gj / a_jj) row_j
+        const cplx l = g == j ? cplx{0., 0.} : cmul({er, ei}, inv);
+        const double fr = g == j ? inv.r : -l.r, fi = g == j ? inv.i : -l.i;
+        const c2 base_a = g == j ? czero() : a, base_z = g == j ? czero() : z;
+        a = {base_a.r0 + fr * u.r0 - fi * u.i0, base_a.r1 + fr * u.r1 - fi * u.i1, base_a.i0 + fr * u.i0 + fi * u.r0, base_a.i1 + fr * u.i1 + fi * u.r1};
+        z = {base_z.r0 + fr * w.r0 - fi * w.i0, base_z.r1 + fr * w.r1 - fi * w.i1, base_z.i0 + fr * w.i0 + fi * w.r0, base_z.i1 + fr * w.i1 + fi * w.r1};
     }
-#pragma unroll
-    for (int j = 7; j >= 0; --j) {
-        const int tj = j >> 1;
-        const bool odd = (j & 1) != 0;
-        if (g == j) {
-            const cplx d = dinv[j];
-            const cplx y0 = cmul({y.r0, y.i0}, d), y1 = cmul({y.r1, y.i1}, d);
-            y = {y0.r, y1.r, y0.i, y1.i};
-        }
-        const c2 w = shfl_c2(y, 4 * j + t);                                                                 // row j of inv(U)
-        const double er = __shfl_sync(FULL, odd ? a.r1 : a.r0, 4 * g + tj), ei = __shfl_sync(FULL, odd ? a.i1 : a.i0, 4 * g + tj);   // u_gj
-        if (g < j) {
-            y.r0 -= er * w.r0 - ei * w.i0; y.i0 -= er * w.i0 + ei * w.r0;
-            y.r1 -= er * w.r1 - ei * w.i1; y.i1 -= er * w.i1 + ei * w.r1;
-        }
-    }
-    const c2 out = {g > 2 * t ? z.r0 : y.r0, g > 2 * t + 1 ? z.r1 : y.r1, g > 2 * t ? z.i0 : y.i0, g > 2 * t + 1 ? z.i1 : y.i1};
-    __syncwarp();
-    st_ctile<C>(Q, j0, j0, out);
-    __syncwarp();
+    return z;
 }
 
-// In-place blocked LU of Q without pivoting (LUi format, perm = identity).  Ends with a barrier.  Look-ahead: during the
-// trailing update of panel kb, warp 0 updates only the next diagonal tile and factors it straight away, the other warps
-// share the rest of the trailing matrix - the single-warp diagonal factorisation runs in the shadow of the update.
+// Q <- Q^-1 in place (W: scratch matrix of the same shape), block Gauss-Jordan on 8 x 8 tiles without pivoting.  Ends with
+// a barrier.  Step kb, with D^-1 = inv(Q[kb, kb]) already in the diagonal slot of the source:
+//     Q[kb, j] <- D^-1 Q[kb, j],   Q[i, j] <- Q[i, j] - Q[i, kb] Q[kb, j]  (new row kb),   Q[i, kb] <- -Q[i, kb] D^-1,
+//     Q[kb, kb] <- D^-1                                                                      (i, j != kb).
+// Warp j owns column tile j and writes it to the other buffer (source and destination alternate between Q and W), so a
+// step reads the old column kb while its owner writes the new one and needs one block barrier.  Look-ahead: the owner of
+// column kb + 1 updates its diagonal tile first and inverts it in registers, in the shadow of the other columns' updates.
+// Every step has NB (NB - 1) independent tile products of the update and NB - 1 of the row and column panels.
 template <class C>
-__device__ void lu_factor_blocked_nopiv(double *Q, int *perm) {
+__device__ void gj_invert_nopiv(double *Q, double *W) {
     constexpr int NB = C::NP / 8;
-    constexpr int HELP = C::NWARP > 1 ? C::NWARP - 1 : 1;          // warps sharing the trailing update beside warp 0
+    static_assert(NB == 1 || NB <= C::NWARP, "one warp per column tile");
+    static_assert(NB == 1 || NB % 2 == 0, "the inverse ends in Q after an even number of steps");
     const int warp = threadIdx.x >> 5;
-    for (int i = threadIdx.x; i < C::NP; i += C::NT) perm[i] = i;
-    __syncthreads();
     PROF_DECL
-    if (warp == 0) lu_diag_warp<C>(Q, 0);
+    if (warp == 0) st_ctile<C>(Q, 0, 0, gj_tile_inverse(ld_ctile<C>(Q, 0, 0)));
     __syncthreads();
-    PROF_MARK(14);
-    for (int kb = 0; kb < NB - 1; ++kb) {
-        const int j0 = kb * 8, nt = NB - kb - 1;
-        for (int x = warp; x < 2 * nt; x += C::NWARP) {
-            c2 v = czero();
-            if (x < nt) {                                          // U12 = inv(L11) A12
-                const int c0 = (kb + 1 + x) * 8;
-                tile_mma<C, false, MASK_LINV, false>(v, Q, j0, j0, Q, j0, c0);
+    PROF_MARK(17);
+    if constexpr (NB > 1) {
+        const int j = warp, c0 = warp * 8;
+        for (int kb = 0; kb < NB; ++kb) {
+            const double *S = (kb & 1) ? W : Q;
+            double *D = (kb & 1) ? Q : W;
+            const int k0 = kb * 8;
+            if (j < NB && j != kb) {
+                c2 r = czero();                                    // new row kb: D^-1 Q[kb, j]
+                tile_mma<C, false, MASK_NONE, false>(r, S, k0, k0, S, k0, c0);
+                st_ctile<C>(D, k0, c0, r);
                 __syncwarp();
-                st_ctile<C>(Q, j0, c0, v);
-            } else {                                               // L21 = A21 inv(U11)
-                const int r0 = (kb + 1 + x - nt) * 8;
-                tile_mma_bupper<C>(v, Q, r0, j0, Q, j0, j0);
-                __syncwarp();
-                st_ctile<C>(Q, r0, j0, v);
+                const bool ahead = j == kb + 1;
+                if (ahead) {                                       // the next diagonal tile first, then its inverse
+                    c2 v = ld_ctile<C>(S, c0, c0);
+                    tile_mma<C, false, MASK_NONE, true>(v, S, c0, k0, D, k0, c0);
+                    st_ctile<C>(D, c0, c0, gj_tile_inverse(v));
+                }
+                c2 v[NB];
+#pragma unroll
+                for (int i = 0; i < NB; ++i) v[i] = ld_ctile<C>(S, i * 8, c0);
+#pragma unroll
+                for (int i = 0; i < NB; ++i)
+                    if (i != kb && !(ahead && i == j)) tile_mma<C, false, MASK_NONE, true>(v[i], S, i * 8, k0, D, k0, c0);
+#pragma unroll
+                for (int i = 0; i < NB; ++i)
+                    if (i != kb && !(ahead && i == j)) st_ctile<C>(D, i * 8, c0, v[i]);
+            } else if (j == kb) {                                  // new column kb: -Q[i, kb] D^-1, and D^-1 itself
+                c2 v[NB];
+#pragma unroll
+                for (int i = 0; i < NB; ++i) {
+                    v[i] = czero();
+                    if (i != kb) tile_mma<C, false, MASK_NONE, true>(v[i], S, i * 8, k0, S, k0, k0);
+                    else v[i] = ld_ctile<C>(S, k0, k0);
+                }
+#pragma unroll
+                for (int i = 0; i < NB; ++i) st_ctile<C>(D, i * 8, c0, v[i]);
             }
+            __syncthreads();
+            PROF_MARK(18);
         }
-        __syncthreads();
-        // A22 -= L21 U12
-        if (C::NWARP == 1) {
-            for (int ct = kb + 1; ct < NB; ++ct) tile_update_rows<C, false>(Q, Q, kb, ct * 8, kb + 1, NB, 1);
-            lu_diag_warp<C>(Q, j0 + 8);
-        } else if (warp == 0) {
-            tile_update_rows<C, false>(Q, Q, kb, j0 + 8, kb + 1, kb + 2, 1);   // the next diagonal tile first ...
-            __syncwarp();
-            lu_diag_warp<C>(Q, j0 + 8);                                       // ... and its factorisation
-        } else {
-            // column tiles kb+1 .. NB-1 over the helper warps; in column kb+1 the diagonal tile belongs to warp 0
-            for (int ct = kb + 1 + (warp - 1); ct < NB; ct += HELP)
-                tile_update_rows<C, false>(Q, Q, kb, ct * 8, ct == kb + 1 ? kb + 2 : kb + 1, NB, 1);
-        }
-        __syncthreads();
-        PROF_MARK(15);
     }
 }
 

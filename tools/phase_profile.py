@@ -46,9 +46,12 @@ v = np.array(list(buf), dtype=np.float64)
 slices = v[0]
 ghz = 1.965
 us = v / slices / (ghz * 1e3)
-names = {1: "fwd coefs+magnus", 2: "fwd one-norm/scale", 3: "fwd pade polynomial (6 products)", 4: "fwd LU factor", 5: "fwd LU solve",
+names = {1: "fwd coefs+magnus", 2: "fwd one-norm/scale", 3: "fwd pade polynomial (6 products)", 4: "fwd LU factor (pivoted)",
+         5: "fwd LU solve (pivoted)", 19: "fwd Q^-1, block Gauss-Jordan (pivot-free)", 25: "fwd R0 = Q^-1 P product (pivot-free)",
          6: "fwd squarings/copy", 7: "fwd pade total + stores + chunk product", 9: "bwd coefs + ubar", 10: "bwd reverse squarings + tape loads",
-         11: "bwd transposed solve", 14: "  LU: panels (warp 0; all 8 per LU)", 15: "  LU: swaps + U12 + trailing update", 16: "  LU: writeback + diag inversion part of panels", 12: "bwd pade polynomial reverse", 13: "bwd pade total + magnus adjoint"}
+         11: "bwd transposed solve or Q^-T product", 14: "  LU: panels (warp 0; all 8 per LU)", 15: "  LU: swaps + U12 + trailing update",
+         16: "  LU: writeback + diag inversion part of panels", 17: "  Q^-1: first diagonal tile inverse (warp 0)",
+         18: "  Q^-1: block steps (NP / 8 per inverse)", 12: "bwd pade polynomial reverse", 13: "bwd pade total + magnus adjoint"}
 print("workload", name, "slices sampled by CTA 0:", int(slices))
 for k in sorted(names):
     print("  %-45s %8.2f us/slice" % (names[k], us[k]))
@@ -57,7 +60,7 @@ for k, nm in ((32, "scale A + store"), (33, "A2 product"), (34, "A2 store"), (35
               (38, "A6 store + epilogue"), (39, "A6 W1 product (half path: + A6 X1)"), (42, "epilogue + A6 X1 product (full path)"),
               (40, "epilogues + A reload"), (41, "Uo product"), (3, "Uo store + P, Q")):
     print("    poly: %-41s %8.2f us/slice" % (nm, us[k]))
-for k, nm in ((43, "stage 0: thin blocks + wait for LU"), (44, "stage 1: thin transposed solve + unpermute (+ wait A)"),
+for k, nm in ((43, "stage 0: thin blocks + wait for LU"), (44, "stage 1: l = Q^-T lam, thin product or solve + unpermute (+ wait A)"),
               (45, "stages 2-3: a = A^T l, chain start (+ wait A2)"), (46, "stage 4: two Krylov chains (6 steps)"),
               (47, "stage 5: rank-48 product + H = a2bar + a2bar^H (+ wait A)"), (12, "stage 6: dense product + anti-Hermitian part")):
     print("    krylov: %-50s %8.2f us/slice" % (nm, us[k]))
