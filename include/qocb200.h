@@ -325,6 +325,27 @@ int qocb_lindblad_cost_and_grad(qocb_lplan *plan, const double *controls, double
    Both return -1 on an ensemble plan. */
 int qocb_lindblad_forward(qocb_lplan *plan, const double *controls, double *cost, double *final_densities);
 int qocb_lindblad_backward(qocb_lplan *plan, const double *seeds, double *grad);
+/* LINDBLAD CONTROL BATCHES (multi-start optimisation, as qocb_set_control_batch on the Schroedinger path): B independent
+   control sets [B][M][KR] of ONE problem - one hamiltonian, lindblad_data, set of initial densities and cost terms - evaluated
+   in one launch of each kernel, one CTA per start, each with its own cost and gradient (no mean over starts).  Create the plan
+   with ensemble_count = B >= 1 and call qocb_lindblad_set_control_batch before qocb_lindblad_set_operators.  The drift,
+   K_half, the rates, the control operators and the time series are stored once; the controls, densities, tape, gradient and
+   result slots are per start.  Start b runs exactly the code, thread count and shared-memory layout of a one-member plan on
+   controls[b], so its cost, gradient, densities and stats are bit-identical to such a plan; B = 1 is an ordinary plan.
+   Time-dependent hamiltonians and rates are allowed: every start evaluates the shared series with its own controls.  Each
+   start has the tape capacity of an ensemble member; the batch calls return -4 when any start's tape filled and -5 when any
+   start's stage time left the series (qocb_lindblad_max_stage_time gives the largest over the starts).
+   qocb_lindblad_set_control_batch returns -1 once operators are set and for plans without controls (have_hamiltonian = 0 or
+   control_count = 0).  On a control batch qocb_lindblad_cost, qocb_lindblad_cost_and_grad, qocb_lindblad_forward,
+   qocb_lindblad_backward, qocb_lindblad_set_ensemble and qocb_lindblad_set_member_operators return -1;
+   qocb_lindblad_member_results gives each start's cost, gradient and stats, qocb_lindblad_get_densities [B][N][D][n][n] and
+   qocb_lindblad_stats the sums over the starts. */
+int qocb_lindblad_set_control_batch(qocb_lplan *plan);
+/* controls: [B][M][KR], costs: [B], final_densities: [B][D][n][n] or NULL.  Return codes as qocb_lindblad_cost_and_grad. */
+int qocb_lindblad_batch_cost(qocb_lplan *plan, const double *controls, double *costs, double *final_densities);
+/* grads: [B][M][KR], start b's gradient only */
+int qocb_lindblad_batch_cost_and_grad(qocb_lplan *plan, const double *controls, double *costs, double *grads,
+                                      double *final_densities);
 /* stats[0] = Runge-Kutta attempts, stats[1] = accepted steps of the last evaluation (sums over the members of an ensemble) */
 int qocb_lindblad_stats(qocb_lplan *plan, int64_t *stats);
 /* each member's results of the last evaluation: costs [E], grads [E][M][KR], stats [E][2]; any may be NULL */

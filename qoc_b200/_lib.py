@@ -33,6 +33,7 @@ EXPORTS = [
     "qocb_lindblad_max_stage_time", "qocb_lindblad_forward", "qocb_lindblad_backward", "qocb_lindblad_set_ensemble",
     "qocb_lindblad_member_results", "qocb_set_member_operators", "qocb_lindblad_set_member_operators",
     "qocb_set_control_batch", "qocb_batch_cost", "qocb_batch_cost_and_grad",
+    "qocb_lindblad_set_control_batch", "qocb_lindblad_batch_cost", "qocb_lindblad_batch_cost_and_grad",
 ]
 
 
@@ -160,6 +161,9 @@ def load():
     lib.qocb_lindblad_set_ensemble.argtypes = [vp, vp, vp]
     lib.qocb_lindblad_set_member_operators.argtypes = [vp, vp]
     lib.qocb_lindblad_member_results.argtypes = [vp, vp, vp, vp]
+    lib.qocb_lindblad_set_control_batch.argtypes = [vp]
+    lib.qocb_lindblad_batch_cost.argtypes = [vp, vp, vp, vp]
+    lib.qocb_lindblad_batch_cost_and_grad.argtypes = [vp, vp, vp, vp, vp]
     lib.qocb_flush_l2.argtypes = [vp]
     lib.qocb_shard_matrix_doubles.argtypes = [vp]
     lib.qocb_shard_vector_doubles.argtypes = [vp]

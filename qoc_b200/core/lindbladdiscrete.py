@@ -6,7 +6,8 @@ adaptive RKDP5 integration and the reverse pass - runs on the GPU through `Lindb
 """
 import numpy as np
 
-from qoc_b200.core.common import initialize_controls, slap_controls, strip_controls, clip_control_norms
+from qoc_b200.core.common import (batch_initial_controls, clip_control_norms, grape_lockstep, initialize_controls,
+                                  slap_controls, strip_controls)
 from qoc_b200.core.plan import LindbladPlan
 from qoc_b200.models import (Dummy, EvolveLindbladDiscreteState, EvolveLindbladResult, GrapeLindbladDiscreteState,
                              GrapeLindbladResult, InterpolationPolicy, ProgramType)
@@ -82,6 +83,39 @@ def grape_lindblad_discrete(control_count, control_eval_count, costs, evolution_
         if plan is not None:
             plan.close()
     return result
+
+
+def grape_lindblad_discrete_batch(control_count, control_eval_count, costs, evolution_time, initial_densities,
+                                  system_eval_count, initial_controls, complex_controls=False, cost_eval_step=1,
+                                  hamiltonian=None, impose_control_conditions=None,
+                                  interpolation_policy=InterpolationPolicy.LINEAR, iteration_count=1000, lindblad_data=None,
+                                  log_iteration_step=10, max_control_norms=None, min_error=0, optimizer=Adam(),
+                                  save_file_path=None):
+    """
+    Multi-start GRAPE on the Lindblad path: B optimisations of one problem from the initial pulses `initial_controls`
+    [B][M][K], run in lockstep with one batched GPU evaluation (`LindbladPlan(control_batch=B)`, one CTA per start) per
+    iteration.  Every other argument means what it means for `grape_lindblad_discrete`, and start b follows the trajectory
+    that `grape_lindblad_discrete(..., initial_controls=initial_controls[b])` would: its controls are clipped in place to
+    `max_control_norms` and passed through `impose_control_conditions` ([M][K] per call) before each evaluation, and its
+    optimiser state is its own.  A start whose error reaches `min_error` stops updating and keeps its best result.  Adam and
+    SGD are supported; L-BFGS-B, whose line search would couple the starts, and `save_file_path` raise NotImplementedError.
+
+    Returns:
+    results :: list of B GrapeLindbladResult (best_controls, best_error, best_final_densities, best_iteration)
+    """
+    controls0, max_control_norms = batch_initial_controls(
+        "grape_lindblad_discrete_batch", complex_controls, control_count, control_eval_count, evolution_time,
+        initial_controls, max_control_norms, optimizer, save_file_path)
+    plan = LindbladPlan(initial_densities, costs, evolution_time, system_eval_count, hamiltonian=hamiltonian,
+                        lindblad_data=lindblad_data, control_eval_count=control_eval_count, control_count=control_count,
+                        complex_controls=complex_controls, cost_eval_step=cost_eval_step,
+                        interpolation_policy=interpolation_policy, control_batch=controls0.shape[0])
+    try:
+        return grape_lockstep(plan.cost_and_grad, controls0, complex_controls, max_control_norms, impose_control_conditions,
+                              iteration_count, log_iteration_step, min_error, optimizer, GrapeLindbladResult,
+                              "best_final_densities")
+    finally:
+        plan.close()
 
 
 def _prepare_controls(params, pstate):

@@ -1098,12 +1098,31 @@ class LindbladPlan(object):
     [h_0 .. h_{E-1}] (callables like `hamiltonian`) its drift and control operators, and `ensemble_rates` [E][L] the decay
     rates of `lindblad_data`, member by member.  `cost` and `cost_and_grad` then return the member mean (control
     costs added once) with final densities [E][D][n][n], `intermediate_densities()` is [E][N][D][n][n] and `member_results()`
-    returns every member's cost, gradient and stats.  One member is the plain plan."""
+    returns every member's cost, gradient and stats.  One member is the plain plan.
+
+    Control batches (multi-start optimisation): `control_batch=B` evaluates B independent control sets of this one problem
+    per call, one CTA per start.  `cost(controls [B][M][K])` returns (errors [B], final densities [B][D][n][n]) and
+    `cost_and_grad` also grads [B][M][K], each start exactly what a one-member plan returns for its controls (control costs
+    added per start); `member_results()` and `intermediate_densities()` are per start.  Time-dependent problems are
+    allowed.  A batch needs controls (`hamiltonian` and control_count >= 1, else ValueError) and is not combinable with
+    ensembles or user-defined costs (NotImplementedError); both are raised before any device call."""
 
     def __init__(self, initial_densities, costs, evolution_time, system_eval_count, hamiltonian=None,
                  lindblad_data=None, control_eval_count=0, control_count=0, complex_controls=False, cost_eval_step=1,
                  interpolation_policy=InterpolationPolicy.LINEAR, device=0, max_rk_steps=0, structure=None,
-                 ensemble_drifts=None, ensemble_rates=None, ensemble_hamiltonians=None):
+                 ensemble_drifts=None, ensemble_rates=None, ensemble_hamiltonians=None, control_batch=None):
+        self.B = None
+        if control_batch is not None:
+            if isinstance(control_batch, bool) or not isinstance(control_batch, (int, np.integer)) or control_batch < 1:
+                raise ValueError("control_batch must be a positive integer, got {!r}".format(control_batch))
+            if hamiltonian is None or int(control_count) < 1:
+                raise ValueError("control batches need a hamiltonian and control_count >= 1: there are no controls to batch")
+            if ensemble_drifts is not None or ensemble_rates is not None or ensemble_hamiltonians is not None:
+                raise NotImplementedError("control batches cannot be combined with ensemble_drifts / ensemble_rates / "
+                                          "ensemble_hamiltonians")
+            if any(is_user_cost(c) for c in costs):
+                raise NotImplementedError("user-defined costs cannot be combined with control batches")
+            self.B = int(control_batch)
         if interpolation_policy != InterpolationPolicy.LINEAR:
             raise ValueError("The interpolation policy {} is not implemented for this method."
                              "".format(interpolation_policy))
@@ -1145,6 +1164,8 @@ class LindbladPlan(object):
         self.L = 0 if lops is None else lops.shape[0]
         h0s, rates, ops = self._ensemble_members(ensemble_drifts, ensemble_rates, ensemble_hamiltonians, td_h, td_l)
         self.E = 1 if h0s is None and rates is None else (h0s if h0s is not None else rates).shape[0]
+        if self.B is not None:
+            self.E = self.B
         member_ops = None                                # [E][KR][n][n] when the members' control operators differ
         if ops is not None:
             a_ops, member_ops = (ops[0], ops) if ops.ndim == 4 else (ops, None)
@@ -1247,13 +1268,15 @@ class LindbladPlan(object):
             raise RuntimeError("qoc_b200 CUDA Lindblad path failed (rc={}): {}".format(
                 rc, self.lib.qocb_lindblad_last_error(None).decode()))
         self.handle = handle
+        if self.B is not None:
+            self._check(self.lib.qocb_lindblad_set_control_batch(handle))
         h0c = None if su["h0"] is None else np.ascontiguousarray(su["h0"], dtype=np.complex128)
         a_ops = su["a_ops"]
         aoc = None if a_ops is None or a_ops.shape[0] == 0 else np.ascontiguousarray(a_ops, dtype=np.complex128)
         lops = None if su["lops"] is None else np.ascontiguousarray(su["lops"], dtype=np.complex128)
         self._check(self.lib.qocb_lindblad_set_operators(handle, _lib.ptr(h0c), _lib.ptr(aoc), _lib.ptr(su["gammas"]),
                                                          _lib.ptr(lops)))
-        if self.E > 1:
+        if self.E > 1 and self.B is None:
             self._check(self.lib.qocb_lindblad_set_ensemble(handle, _lib.ptr(self._members[0]), _lib.ptr(self._members[1])))
             if self._members[2] is not None:
                 self._check(self.lib.qocb_lindblad_set_member_operators(handle, _lib.ptr(self._members[2])))
@@ -1299,6 +1322,7 @@ class LindbladPlan(object):
             raise RuntimeError("qoc_b200 CUDA Lindblad path failed (rc={}): {}".format(rc, msg.decode() if msg else "?"))
 
     _real_channels = SchroedingerPlan._real_channels
+    _batch_channels = SchroedingerPlan._batch_channels
     _control_costs = SchroedingerPlan._control_costs
     cost_and_grad_autograd = SchroedingerPlan.cost_and_grad_autograd
 
@@ -1326,10 +1350,35 @@ class LindbladPlan(object):
         return seeds
 
     def _final_buffer(self):
-        shape = (self.D, self.n, self.n) if self.E == 1 else (self.E, self.D, self.n, self.n)
+        shape = (self.D, self.n, self.n) if self.E == 1 and self.B is None else (self.E, self.D, self.n, self.n)
         return np.empty(shape, dtype=np.complex128)
 
+    def _batch_eval(self, controls, want_grad):
+        """(errors [B], grads [B][M][K] or None, final densities [B][D][n][n]); host control costs are added per start."""
+        x = self._batch_channels(controls)
+        controls = np.asarray(controls)
+        out = np.zeros(self.B)
+        fd = self._final_buffer()
+        grads = None
+        if want_grad:
+            g = np.zeros((self.B, self.M, self.KR))
+            self._evaluate(lambda h: self.lib.qocb_lindblad_batch_cost_and_grad(h, _lib.ptr(x), _lib.ptr(out), _lib.ptr(g),
+                                                                                _lib.ptr(fd)))
+            grads = self._controls_grad(g, controls)
+        else:
+            self._evaluate(lambda h: self.lib.qocb_lindblad_batch_cost(h, _lib.ptr(x), _lib.ptr(out), _lib.ptr(fd)))
+        parts = [self._control_costs(controls[b], want_grad) for b in range(self.B)]
+        extras = np.array([v for v, _ in parts])
+        extra_grads = np.array([g for _, g in parts]) if want_grad and parts[0][1] is not None else None
+        self._last_extra = (extras, (controls.shape[1:], controls.dtype, extra_grads) if want_grad else None)
+        if extra_grads is not None:
+            grads = grads + extra_grads
+        return out + extras, grads, fd
+
     def cost(self, controls):
+        if self.B is not None:
+            errors, _, fd = self._batch_eval(controls, False)
+            return errors, fd
         x = self._real_channels(controls) if controls is not None else None
         out = np.zeros(1)
         fd = self._final_buffer()
@@ -1344,7 +1393,10 @@ class LindbladPlan(object):
     def cost_and_grad(self, controls):
         """(error, grads, final_densities); grads = dE/dRe(u) + i dE/dIm(u) for complex controls.  With user costs the
         forward pass keeps its tape, the host evaluates the user costs on the densities, and the reverse pass is seeded with
-        their numeric cotangents (qocb_lindblad_forward / qocb_lindblad_backward)."""
+        their numeric cotangents (qocb_lindblad_forward / qocb_lindblad_backward).  A control batch returns
+        (errors [B], grads [B][M][K], final densities [B][D][n][n])."""
+        if self.B is not None:
+            return self._batch_eval(controls, True)
         x = self._real_channels(controls)
         out = np.zeros(1)
         fd = self._final_buffer()
@@ -1375,16 +1427,16 @@ class LindbladPlan(object):
         return value + extra, grads, fd
 
     def _controls_grad(self, g, controls):
-        """dE/dRe u + i dE/dIm u in the controls' shape from the device gradient [M][KR]."""
+        """dE/dRe u + i dE/dIm u in the controls' shape from the device gradient [M][KR] ([B][M][KR] for a batch)."""
         if self.KR == 0:
             return np.zeros(controls.shape, dtype=controls.dtype)
-        return g[:, :self.K] + 1j * g[:, self.K:] if self.complex_controls else g
+        return g[..., :self.K] + 1j * g[..., self.K:] if self.complex_controls else g
 
     def member_results(self):
         """every member's (cost, gradient, stats) of the last evaluation: costs [E], gradients [E] in the controls' shape and
         dtype (None after `cost`), stats [E] as {"attempts", "accepted"}; the control costs are included in each member's
         cost and gradient, so member e equals a one-member plan built with its drift and rates (and the same control
-        operators)."""
+        operators).  For a control batch these are the starts' results, each with its own control costs."""
         costs = np.zeros(self.E)
         g = np.zeros((self.E, self.M, self.KR))
         st = np.zeros((self.E, 2), dtype=np.int64)
@@ -1399,7 +1451,8 @@ class LindbladPlan(object):
             grads = []
             for e in range(self.E):
                 ge = self._controls_grad(g[e], zero)
-                grads.append(ge + extra_grad if extra_grad is not None else ge)
+                eg = extra_grad if extra_grad is None or self.B is None else extra_grad[e]
+                grads.append(ge + eg if eg is not None else ge)
             grads = np.array(grads)
         return costs, grads, [{"attempts": int(a), "accepted": int(b)} for a, b in st]
 
@@ -1410,7 +1463,7 @@ class LindbladPlan(object):
 
     def intermediate_densities(self):
         shape = (self.N, self.D, self.n, self.n)
-        buf = np.empty(shape if self.E == 1 else (self.E,) + shape, dtype=np.complex128)
+        buf = np.empty(shape if self.E == 1 and self.B is None else (self.E,) + shape, dtype=np.complex128)
         self._check(self.lib.qocb_lindblad_get_densities(self.handle, _lib.ptr(buf)))
         return buf
 

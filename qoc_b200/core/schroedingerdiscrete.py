@@ -8,12 +8,13 @@ through `SchroedingerPlan`.
 """
 import numpy as np
 
-from qoc_b200.core.common import (initialize_controls, slap_controls, strip_controls, clip_control_norms)
+from qoc_b200.core.common import (_adam_rows, batch_initial_controls, clip_control_norms, grape_lockstep,  # noqa: F401
+                                  initialize_controls, slap_controls, strip_controls)
 from qoc_b200.core.plan import SchroedingerPlan, make_schroedinger_plan
 from qoc_b200.models import (Dummy, EvolveSchroedingerDiscreteState, EvolveSchroedingerResult,
                              GrapeSchroedingerDiscreteState, GrapeSchroedingerResult, InterpolationPolicy,
                              MagnusPolicy, ProgramType)
-from qoc_b200.standard.optimizers import SGD, Adam, LBFGSB
+from qoc_b200.standard.optimizers import Adam
 from qoc_b200.standard.utils import autograd_available
 
 
@@ -118,84 +119,19 @@ def grape_schroedinger_discrete_batch(control_count, control_eval_count, costs, 
     Returns:
     results :: list of B GrapeSchroedingerResult (best_controls, best_error, best_final_states, best_iteration)
     """
-    if save_file_path is not None:
-        raise NotImplementedError("grape_schroedinger_discrete_batch does not save to files; run the best start again "
-                                  "with grape_schroedinger_discrete to save it")
-    if isinstance(optimizer, LBFGSB):
-        raise NotImplementedError("L-BFGS-B is not supported for control batches: its line search would couple the starts")
-    if not isinstance(optimizer, (Adam, SGD)):
-        raise NotImplementedError("control batches run Adam or SGD, not {}".format(optimizer))
-    controls0 = np.asarray(initial_controls)
-    K, M = int(control_count), int(control_eval_count)
-    if controls0.ndim != 3 or controls0.shape[0] < 1 or controls0.shape[1:] != (M, K):
-        raise ValueError("initial_controls must have shape [B][{}][{}] with B >= 1, got {}".format(M, K, controls0.shape))
-    if not np.issubdtype(controls0.dtype, np.number):
-        raise ValueError("initial_controls must be numeric, got dtype {}".format(controls0.dtype))
-    B = controls0.shape[0]
-    for b in range(B):                  # the dtype and max-norm checks of the single-start program, per start
-        _, max_control_norms = initialize_controls(complex_controls, K, M, evolution_time, controls0[b], max_control_norms)
+    controls0, max_control_norms = batch_initial_controls(
+        "grape_schroedinger_discrete_batch", complex_controls, control_count, control_eval_count, evolution_time,
+        initial_controls, max_control_norms, optimizer, save_file_path)
     plan = SchroedingerPlan(hamiltonian, initial_states, costs, evolution_time, system_eval_count,
-                            control_eval_count=M, control_count=K, complex_controls=complex_controls,
-                            magnus_policy=magnus_policy, cost_eval_step=cost_eval_step,
-                            interpolation_policy=interpolation_policy, control_batch=B)
-    # optimiser format, one row per start: flat float64 ([Re | Im] for complex controls), as strip_controls
-    params = np.stack([strip_controls(complex_controls, controls0[b]) for b in range(B)]).astype(np.float64)
-    shape = (M, K)
-    results = [GrapeSchroedingerResult() for _ in range(B)]
-    stopped = np.zeros(B, dtype=bool)
-    adam = isinstance(optimizer, Adam)
-    moment, square_moment, steps = np.zeros_like(params), np.zeros_like(params), np.zeros((B, 1))
+                            control_eval_count=control_eval_count, control_count=control_count,
+                            complex_controls=complex_controls, magnus_policy=magnus_policy, cost_eval_step=cost_eval_step,
+                            interpolation_policy=interpolation_policy, control_batch=controls0.shape[0])
     try:
-        for iteration in range(iteration_count):
-            controls = np.empty((B, M, K), dtype=np.complex128 if complex_controls else np.float64)
-            for b in range(B):
-                c = slap_controls(complex_controls, params[b], shape)      # a view of params[b] for real controls
-                clip_control_norms(c, max_control_norms)
-                if impose_control_conditions is not None:
-                    c = impose_control_conditions(c)
-                controls[b] = c
-            errors, grads, finals = plan.cost_and_grad(controls)
-            active = np.nonzero(~stopped)[0]
-            for b in active:
-                if errors[b] < results[b].best_error:
-                    results[b].best_controls = controls[b].copy()
-                    results[b].best_error = float(errors[b])
-                    results[b].best_final_states = finals[b].copy()
-                    results[b].best_iteration = iteration
-            stopped[active] = errors[active] <= min_error
-            if log_iteration_step and iteration % log_iteration_step == 0:
-                print("{:>6d} | best error {:.12e} | median error {:.12e} | stopped {}/{}".format(
-                    iteration, min(r.best_error for r in results), float(np.median(errors)), int(stopped.sum()), B))
-            idx = np.nonzero(~stopped)[0]
-            if idx.size == 0:
-                break
-            g = np.stack([strip_controls(complex_controls, grads[b]) for b in idx])
-            if adam:
-                params[idx], moment[idx], square_moment[idx], steps[idx] = _adam_rows(
-                    optimizer, params[idx], g, moment[idx], square_moment[idx], steps[idx])
-            else:
-                params[idx] = params[idx] - optimizer.learning_rate * g
+        return grape_lockstep(plan.cost_and_grad, controls0, complex_controls, max_control_norms, impose_control_conditions,
+                              iteration_count, log_iteration_step, min_error, optimizer, GrapeSchroedingerResult,
+                              "best_final_states")
     finally:
         plan.close()
-    return results
-
-
-def _adam_rows(opt, params, grads, moment, square_moment, steps):
-    """`Adam.update` applied to every row on its own (one row per start; `steps` [rows][1] counts each row's updates):
-    the gradient norm of `scale_grads` is the row's own."""
-    lr = opt.initial_learning_rate
-    if opt.apply_learning_rate_decay:
-        lr = lr * np.exp(-np.divide(steps, opt.learning_rate_decay))
-    if opt.apply_scale_grads:
-        grads = grads / np.linalg.norm(grads, axis=1, keepdims=True) * opt.scale_grads
-    if opt.apply_clip_grads:
-        grads = np.clip(grads, -opt.clip_grads, opt.clip_grads)
-    t = steps + 1
-    moment = opt.beta_1 * moment + (1 - opt.beta_1) * grads
-    square_moment = opt.beta_2 * square_moment + (1 - opt.beta_2) * np.square(grads)
-    m_hat = moment / (1 - np.power(opt.beta_1, t))
-    v_hat = square_moment / (1 - np.power(opt.beta_2, t))
-    return params - lr * m_hat / (np.sqrt(v_hat) + opt.epsilon), moment, square_moment, t
 
 
 # --- optimiser callbacks ---------------------------------------------------------------------------------

@@ -17,7 +17,8 @@
 //
 // An ensemble plan (robust control over drifts and rates) launches E such CTAs at once: CTA e is member e and runs exactly
 // the code of a one-member plan on its own drift, rates, densities, tape and result slots (member_args); a small kernel
-// then forms the member mean in member order.
+// then forms the member mean in member order.  A control batch (multi-start optimisation) launches B CTAs the same way,
+// each on its own controls and the shared drift and rates, and returns every start's results without a mean.
 #include <algorithm>
 #include <cmath>
 #include <cstdio>
@@ -82,16 +83,21 @@ struct LArgs {
     const double2 *Kops;                        // [L][n*n] 1/2 B_l^dag B_l (tdr)
     double *tseen;                              // largest stage time of the forward pass
     const double2 *seeds;                       // [N][D*n*n] host-cost cotangents of the densities, or null
+    long long ctl_stride;                       // start stride of the controls of a control batch: M*KR
 };
 
-// the arguments of ensemble member blockIdx.x: per-member drift, K_half, rates, densities, tape, interval indices, global
-// work, cost, gradient, stats, stage time and tape-overflow flag sit at member-major offsets, and so do the control
-// operators when the members have their own (ops_stride > 0); rho0, Lindblad operators, cost terms, controls and the time
-// series are shared.  Member 0 is the whole plan when E = 1.
-__device__ __forceinline__ LArgs member_args(const LArgs &a0) {
+// the arguments of ensemble member blockIdx.x: per-member densities, tape, interval indices, global work, cost, gradient,
+// stats, stage time and tape-overflow flag sit at member-major offsets.  An ensemble (BATCH = false) also offsets the drift,
+// K_half and rates, and the control operators when the members have their own (ops_stride > 0); controls are shared.  A
+// control batch (BATCH = true) offsets the controls instead and shares drift, K_half and rates.  rho0, Lindblad operators,
+// cost terms and the time series are always shared.  Member 0 is the whole plan when E = 1.  BATCH is a template parameter,
+// not a run-time stride, so that ordinary and ensemble plans keep the exact instruction stream they had before control
+// batches (run-time strides cost cfg2_lindblad_n2 0.6 %; DESIGN.md section 3.3).
+template <bool BATCH> __device__ __forceinline__ LArgs member_args(const LArgs &a0) {
     LArgs a = a0;
     const size_t e = blockIdx.x, nn = (size_t)a.n * a.n, DE = (size_t)a.D * nn;
-    a.H0 += e * nn; a.Khalf += e * nn; a.gam += e * (size_t)max(a.L, 1);
+    if constexpr (BATCH) a.controls += e * a.ctl_stride;
+    else { a.H0 += e * nn; a.Khalf += e * nn; a.gam += e * (size_t)max(a.L, 1); }
     a.Aops += e * a.ops_stride;
     a.states += e * a.N * DE;
     a.tape_x += e * a.cap; a.tape_h += e * a.cap; a.tape_y += e * a.cap * DE; a.tape_k1 += e * a.cap * DE;
@@ -433,9 +439,9 @@ template <bool TD> __device__ void carve(const LArgs &a, unsigned char *smem, Ct
     for (int i = 0; i < narr; ++i) w.p[i] = base + (size_t)(i + 1) * DE;
 }
 
-template <bool TD> __global__ void __launch_bounds__(LNT) k_lindblad_forward(LArgs a0, int keep_tape) {
+template <bool TD, bool BATCH> __global__ void __launch_bounds__(LNT) k_lindblad_forward(LArgs a0, int keep_tape) {
     extern __shared__ __align__(16) unsigned char smem[];
-    const LArgs a = member_args(a0);
+    const LArgs a = member_args<BATCH>(a0);
     Ctx c(a);
     Work w;
     carve<TD>(a, smem, c, w, 12);
@@ -523,9 +529,9 @@ template <bool TD> __global__ void __launch_bounds__(LNT) k_lindblad_forward(LAr
     if (threadIdx.x == 0) { *a.cost = cost; a.stats[0] = attempts; a.stats[1] = accepted; if (TD) *a.tseen = c.tseen; }
 }
 
-template <bool TD> __global__ void __launch_bounds__(LNT) k_lindblad_backward(LArgs a0) {
+template <bool TD, bool BATCH> __global__ void __launch_bounds__(LNT) k_lindblad_backward(LArgs a0) {
     extern __shared__ __align__(16) unsigned char smem[];
-    const LArgs a = member_args(a0);
+    const LArgs a = member_args<BATCH>(a0);
     Ctx c(a);
     Work w;
     if (*a.err_flag) return;                          // the forward pass overflowed this member's tape: hit[] is not valid
@@ -649,6 +655,7 @@ struct qocb_lplan {
     int E = 1;                                     // ensemble members (one CTA each)
     bool ens_set = false;                          // qocb_lindblad_set_ensemble since the last qocb_lindblad_set_operators
     bool member_ops = false;                       // Aops holds [E][KR][n*n] (qocb_lindblad_set_member_operators)
+    bool batch = false;                            // control batch: E starts, controls [E][M][KR] (qocb_lindblad_set_control_batch)
     int cap = 0;                                   // tape capacity of one member
     bool ops_set = false, rho_set = false, costs_dirty = true, series_set = false;
     int NS = 0, segs = 0, deg = 0;                 // time series: NS = KC*(1+KR) + (time_dependent_rates ? L : 0)
@@ -668,6 +675,8 @@ struct qocb_lplan {
 };
 
 namespace {
+constexpr const char *kBatchOnly =
+    "this plan is a control batch: evaluate it with qocb_lindblad_batch_cost / qocb_lindblad_batch_cost_and_grad";
 int lfail(qocb_lplan *p, const char *msg, int rc) { if (p) p->err = msg; g_lerr = msg; return rc; }
 #define LTRY(p, expr) do { cudaError_t e__ = (expr); if (e__ != cudaSuccess) { char b__[512]; snprintf(b__, sizeof(b__), "%s failed: %s (%s:%d)", #expr, cudaGetErrorString(e__), __FILE__, __LINE__); return lfail(p, b__, -2); } } while (0)
 
@@ -684,6 +693,7 @@ LArgs make_largs(qocb_lplan *p) {
     a.work = p->work.p; a.work_in_smem = 0; a.ops_in_smem = p->ops_in_smem; a.grad = p->grad.p;
     a.KC = p->pb.channel_count; a.tdr = p->pb.time_dependent_rates; a.NS = p->NS; a.segs = p->segs; a.deg = p->deg;
     a.seg_w = p->seg_w; a.series = p->series.p; a.Kops = p->Kops.p; a.tseen = p->tseen.p; a.seeds = nullptr;
+    a.ctl_stride = (long long)a.M * a.KR;
     return a;
 }
 
@@ -725,14 +735,17 @@ int lindblad_threads(const qocb_lplan *p) {
     return DEl <= 64 ? 32 : (DEl <= 256 ? 128 : LNT);
 }
 
+// the kernels of a control batch with more than one start; B = 1 runs the ordinary kernels, for which start 0 is the plan
+bool per_start(const qocb_lplan *p) { return p->batch && p->E > 1; }
+
 // enqueues the forward pass (keep_tape: record the reverse-pass tape) after uploading the controls
 int launch_forward(qocb_lplan *p, const double *controls, bool keep_tape) {
     if (!p->ops_set || !p->rho_set) return lfail(p, "operators and densities must be set before evaluation", -1);
     if (p->NS > 0 && !p->series_set) return lfail(p, "time-dependent operators need qocb_lindblad_set_time_series before evaluation", -1);
-    if (p->E > 1 && !p->ens_set) return lfail(p, "an ensemble plan needs qocb_lindblad_set_ensemble after qocb_lindblad_set_operators", -1);
+    if (p->E > 1 && !p->batch && !p->ens_set) return lfail(p, "an ensemble plan needs qocb_lindblad_set_ensemble after qocb_lindblad_set_operators", -1);
     LTRY(p, cudaSetDevice(p->pb.device));
     if (upload_lcosts(p)) return -2;
-    const size_t cnt = (size_t)p->pb.control_eval_count * p->pb.control_count;
+    const size_t cnt = (size_t)p->pb.control_eval_count * p->pb.control_count * (p->batch ? p->E : 1);
     if (cnt) {
         if (!controls) return lfail(p, "controls is null", -1);
         LTRY(p, cudaMemcpyAsync(p->controls.p, controls, sizeof(double) * cnt, cudaMemcpyHostToDevice, p->stream));
@@ -740,8 +753,15 @@ int launch_forward(qocb_lplan *p, const double *controls, bool keep_tape) {
     LTRY(p, cudaMemsetAsync(p->err_flag.p, 0, sizeof(int) * p->E, p->stream));
     LArgs a = make_largs(p);
     a.work_in_smem = p->in_smem_fwd;
-    if (p->NS > 0) k_lindblad_forward<true><<<p->E, lindblad_threads(p), p->smem_fwd, p->stream>>>(a, keep_tape ? 1 : 0);
-    else k_lindblad_forward<false><<<p->E, lindblad_threads(p), p->smem_fwd, p->stream>>>(a, keep_tape ? 1 : 0);
+    const dim3 grid(p->E), block(lindblad_threads(p));
+    const int kt = keep_tape ? 1 : 0;
+    if (per_start(p)) {
+        if (p->NS > 0) k_lindblad_forward<true, true><<<grid, block, p->smem_fwd, p->stream>>>(a, kt);
+        else k_lindblad_forward<false, true><<<grid, block, p->smem_fwd, p->stream>>>(a, kt);
+    } else {
+        if (p->NS > 0) k_lindblad_forward<true, false><<<grid, block, p->smem_fwd, p->stream>>>(a, kt);
+        else k_lindblad_forward<false, false><<<grid, block, p->smem_fwd, p->stream>>>(a, kt);
+    }
     LTRY(p, cudaGetLastError());
     return 0;
 }
@@ -751,8 +771,14 @@ int launch_backward(qocb_lplan *p, const double2 *seeds) {
     LArgs a = make_largs(p);
     a.work_in_smem = p->in_smem_bwd;
     a.seeds = seeds;
-    if (p->NS > 0) k_lindblad_backward<true><<<p->E, lindblad_threads(p), p->smem_bwd, p->stream>>>(a);
-    else k_lindblad_backward<false><<<p->E, lindblad_threads(p), p->smem_bwd, p->stream>>>(a);
+    const dim3 grid(p->E), block(lindblad_threads(p));
+    if (per_start(p)) {
+        if (p->NS > 0) k_lindblad_backward<true, true><<<grid, block, p->smem_bwd, p->stream>>>(a);
+        else k_lindblad_backward<false, true><<<grid, block, p->smem_bwd, p->stream>>>(a);
+    } else {
+        if (p->NS > 0) k_lindblad_backward<true, false><<<grid, block, p->smem_bwd, p->stream>>>(a);
+        else k_lindblad_backward<false, false><<<grid, block, p->smem_bwd, p->stream>>>(a);
+    }
     LTRY(p, cudaGetLastError());
     return 0;
 }
@@ -768,14 +794,16 @@ int launch_mean(qocb_lplan *p, bool with_grad) {
 
 // copies the requested results to the host, waits for the stream and reports a stage time beyond the series (-5) or a
 // full tape (-4) of the last forward pass.  An ensemble returns the member mean, every member's final densities [E][D][n][n],
-// the largest stage time over members and -4 when any member's tape overflowed.
+// the largest stage time over members and -4 when any member's tape overflowed.  A control batch returns every start's
+// cost [B], gradient [B][M][KR] and final densities [B][D][n][n], with the same stage-time and tape rules over the starts.
 int finish_lindblad(qocb_lplan *p, double *cost, double *grad, double *final_densities) {
     const size_t cnt = (size_t)p->pb.control_eval_count * p->pb.control_count;
-    const bool ens = p->E > 1;
+    const bool ens = p->E > 1, mean = ens && !p->batch;
+    const size_t R = p->batch ? p->E : 1;                        // results per call
     std::vector<int> flags(p->E, 0);
     LTRY(p, cudaMemcpyAsync(flags.data(), p->err_flag.p, sizeof(int) * p->E, cudaMemcpyDeviceToHost, p->stream));
-    if (cost) LTRY(p, cudaMemcpyAsync(cost, ens ? p->cost_mean.p : p->cost.p, sizeof(double), cudaMemcpyDeviceToHost, p->stream));
-    if (grad && cnt) LTRY(p, cudaMemcpyAsync(grad, ens ? p->grad_mean.p : p->grad.p, sizeof(double) * cnt, cudaMemcpyDeviceToHost, p->stream));
+    if (cost) LTRY(p, cudaMemcpyAsync(cost, mean ? p->cost_mean.p : p->cost.p, sizeof(double) * R, cudaMemcpyDeviceToHost, p->stream));
+    if (grad && cnt) LTRY(p, cudaMemcpyAsync(grad, mean ? p->grad_mean.p : p->grad.p, sizeof(double) * cnt * R, cudaMemcpyDeviceToHost, p->stream));
     const size_t DE = (size_t)p->pb.density_count * p->pb.hilbert_size * p->pb.hilbert_size, N = p->pb.system_eval_count;
     if (final_densities && !ens)
         LTRY(p, cudaMemcpyAsync(final_densities, p->states.p + (N - 1) * DE, sizeof(double2) * DE,
@@ -783,9 +811,10 @@ int finish_lindblad(qocb_lplan *p, double *cost, double *grad, double *final_den
     if (final_densities && ens)                                  // row N-1 of every member's [N][DE] block
         LTRY(p, cudaMemcpy2DAsync(final_densities, sizeof(double2) * DE, p->states.p + (N - 1) * DE, sizeof(double2) * N * DE,
                                   sizeof(double2) * DE, p->E, cudaMemcpyDeviceToHost, p->stream));
-    double tseen = 0.;
-    if (p->NS > 0) LTRY(p, cudaMemcpyAsync(&tseen, ens ? p->tseen_max.p : p->tseen.p, sizeof(double), cudaMemcpyDeviceToHost, p->stream));
+    std::vector<double> ts(R, 0.);
+    if (p->NS > 0) LTRY(p, cudaMemcpyAsync(ts.data(), mean ? p->tseen_max.p : p->tseen.p, sizeof(double) * R, cudaMemcpyDeviceToHost, p->stream));
     LTRY(p, cudaStreamSynchronize(p->stream));
+    const double tseen = *std::max_element(ts.begin(), ts.end());
     if (p->NS > 0 && tseen > p->segs * p->seg_w)
         return lfail(p, "a Runge-Kutta stage time lies beyond the time series: extend it (qocb_lindblad_max_stage_time)", -5);
     for (int f : flags)
@@ -859,10 +888,14 @@ int qocb_lindblad_create(const qocb_lindblad_problem *pb, qocb_lplan **out) {
     p->smem_fwd = p->in_smem_fwd ? need_f : fixed; p->smem_bwd = p->in_smem_bwd ? need_b : fixed;
     if (fixed > limit) { g_lerr = "hilbert_size too large for the Lindblad kernels' shared-memory operators"; delete p; return -1; }
     CTRY(p->work.alloc((p->in_smem_fwd && p->in_smem_bwd ? 1 : E) * 24 * DE));   // one slice per member when it is used
-    CTRY(cudaFuncSetAttribute(k_lindblad_forward<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
-    CTRY(cudaFuncSetAttribute(k_lindblad_backward<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
-    CTRY(cudaFuncSetAttribute(k_lindblad_forward<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
-    CTRY(cudaFuncSetAttribute(k_lindblad_backward<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
+    CTRY(cudaFuncSetAttribute(k_lindblad_forward<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
+    CTRY(cudaFuncSetAttribute(k_lindblad_backward<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
+    CTRY(cudaFuncSetAttribute(k_lindblad_forward<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
+    CTRY(cudaFuncSetAttribute(k_lindblad_backward<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
+    CTRY(cudaFuncSetAttribute(k_lindblad_forward<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
+    CTRY(cudaFuncSetAttribute(k_lindblad_backward<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
+    CTRY(cudaFuncSetAttribute(k_lindblad_forward<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
+    CTRY(cudaFuncSetAttribute(k_lindblad_backward<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
 #undef CTRY
     *out = p;
     return 0;
@@ -902,7 +935,7 @@ int qocb_lindblad_set_operators(qocb_lplan *p, const double *h0, const double *a
         build_khalf(lops, gammas, n, L, kh.data());
         LTRY(p, cudaMemcpy(p->Khalf.p, kh.data(), sizeof(double2) * nn, cudaMemcpyHostToDevice));
     }
-    if (p->E > 1) {                                                         // kept for the members qocb_lindblad_set_ensemble leaves alone
+    if (p->E > 1 && !p->batch) {                                            // kept for the members qocb_lindblad_set_ensemble leaves alone
         p->h_h0.assign(2 * (size_t)nn, 0.0);
         if (p->pb.have_hamiltonian) std::copy(h0, h0 + 2 * (size_t)nn, p->h_h0.begin());
         p->h_gam.assign(gammas && L > 0 && !p->pb.time_dependent_rates ? gammas : nullptr,
@@ -919,6 +952,7 @@ int qocb_lindblad_set_operators(qocb_lplan *p, const double *h0, const double *a
 int qocb_lindblad_set_ensemble(qocb_lplan *p, const double *h0s, const double *gammas) {
     if (!p) return -1;
     if (p->E <= 1) return lfail(p, "qocb_lindblad_set_ensemble needs ensemble_count > 1", -1);
+    if (p->batch) return lfail(p, "qocb_lindblad_set_ensemble does not apply to a control batch", -1);
     if (!p->ops_set) return lfail(p, "qocb_lindblad_set_operators must come before qocb_lindblad_set_ensemble", -1);
     if (h0s && (!p->pb.have_hamiltonian || p->pb.channel_count > 0))
         return lfail(p, "member drifts need a time-independent hamiltonian (have_hamiltonian = 1, channel_count = 0)", -1);
@@ -948,6 +982,7 @@ int qocb_lindblad_set_ensemble(qocb_lplan *p, const double *h0s, const double *g
 /* a_ops: [E][KR][n][n], member e's control operators */
 int qocb_lindblad_set_member_operators(qocb_lplan *p, const double *a_ops) {
     if (!p || !a_ops) return lfail(p, "null argument", -1);
+    if (p->batch) return lfail(p, "qocb_lindblad_set_member_operators does not apply to a control batch", -1);
     if (!p->ops_set) return lfail(p, "qocb_lindblad_set_operators must come before qocb_lindblad_set_member_operators", -1);
     if (!p->pb.have_hamiltonian || p->pb.channel_count > 0)
         return lfail(p, "member operators need a time-independent hamiltonian (have_hamiltonian = 1, channel_count = 0)", -1);
@@ -982,6 +1017,12 @@ int qocb_lindblad_max_stage_time(qocb_lplan *p, double *t) {
     if (!p || !t) return lfail(p, "null argument", -1);
     if (p->NS == 0) return lfail(p, "this plan has no time series", -1);
     LTRY(p, cudaSetDevice(p->pb.device));
+    if (p->batch) {                                                         // the largest over the starts
+        std::vector<double> ts(p->E);
+        LTRY(p, cudaMemcpy(ts.data(), p->tseen.p, sizeof(double) * p->E, cudaMemcpyDeviceToHost));
+        *t = *std::max_element(ts.begin(), ts.end());
+        return 0;
+    }
     LTRY(p, cudaMemcpy(t, p->E > 1 ? p->tseen_max.p : p->tseen.p, sizeof(double), cudaMemcpyDeviceToHost));
     return 0;
 }
@@ -1019,6 +1060,7 @@ int qocb_lindblad_add_cost(qocb_lplan *p, int32_t kind, int32_t step_cost, doubl
 
 int qocb_lindblad_cost(qocb_lplan *p, const double *controls, double *cost, double *final_densities) {
     if (!p) return -1;
+    if (p->batch) return lfail(p, kBatchOnly, -1);
     p->tape_ok = false;
     if (int rc = launch_forward(p, controls, false)) return rc;
     if (p->E > 1)
@@ -1028,6 +1070,7 @@ int qocb_lindblad_cost(qocb_lplan *p, const double *controls, double *cost, doub
 
 int qocb_lindblad_cost_and_grad(qocb_lplan *p, const double *controls, double *cost, double *grad, double *final_densities) {
     if (!p) return -1;
+    if (p->batch) return lfail(p, kBatchOnly, -1);
     p->tape_ok = false;
     if (int rc = launch_forward(p, controls, true)) return rc;
     const bool with_grad = (size_t)p->pb.control_eval_count * p->pb.control_count > 0;
@@ -1040,6 +1083,7 @@ int qocb_lindblad_cost_and_grad(qocb_lplan *p, const double *controls, double *c
 
 int qocb_lindblad_forward(qocb_lplan *p, const double *controls, double *cost, double *final_densities) {
     if (!p) return -1;
+    if (p->batch) return lfail(p, kBatchOnly, -1);
     p->tape_ok = false;
     if (p->E > 1) return lfail(p, "qocb_lindblad_forward / qocb_lindblad_backward do not run ensemble plans", -1);
     if (int rc = launch_forward(p, controls, true)) return rc;
@@ -1051,6 +1095,7 @@ int qocb_lindblad_forward(qocb_lplan *p, const double *controls, double *cost, d
 /* seeds: [N][D][n][n] complex or NULL; row k is added to the cotangent of the densities at system step k */
 int qocb_lindblad_backward(qocb_lplan *p, const double *seeds, double *grad) {
     if (!p) return -1;
+    if (p->batch) return lfail(p, kBatchOnly, -1);
     if (p->E > 1) return lfail(p, "qocb_lindblad_forward / qocb_lindblad_backward do not run ensemble plans", -1);
     const size_t cnt = (size_t)p->pb.control_eval_count * p->pb.control_count;
     if (!cnt) return 0;
@@ -1063,6 +1108,39 @@ int qocb_lindblad_backward(qocb_lplan *p, const double *seeds, double *grad) {
     }
     if (int rc = launch_backward(p, seeds ? p->seeds.p : nullptr)) return rc;
     return finish_lindblad(p, nullptr, grad, nullptr);
+}
+
+int qocb_lindblad_set_control_batch(qocb_lplan *p) {
+    if (!p) return -1;
+    if (p->ops_set) return lfail(p, "qocb_lindblad_set_control_batch must come before qocb_lindblad_set_operators", -1);
+    if (!p->pb.have_hamiltonian || p->pb.control_count == 0)
+        return lfail(p, "a control batch needs controls (have_hamiltonian = 1 and control_count > 0)", -1);
+    LTRY(p, cudaSetDevice(p->pb.device));
+    const size_t nn = (size_t)p->pb.hilbert_size * p->pb.hilbert_size;
+    LTRY(p, p->controls.alloc((size_t)p->E * p->pb.control_eval_count * p->pb.control_count));
+    LTRY(p, p->H0.alloc(nn)); LTRY(p, p->Khalf.alloc(nn));                 // drift, K_half and rates are stored once
+    LTRY(p, p->gam.alloc(std::max(1, p->pb.lindblad_count)));
+    LTRY(p, cudaMemset(p->H0.p, 0, sizeof(double2) * nn)); LTRY(p, cudaMemset(p->Khalf.p, 0, sizeof(double2) * nn));
+    p->batch = true;
+    return 0;
+}
+
+int qocb_lindblad_batch_cost(qocb_lplan *p, const double *controls, double *costs, double *final_densities) {
+    if (!p) return -1;
+    if (!p->batch) return lfail(p, "qocb_lindblad_batch_cost needs qocb_lindblad_set_control_batch", -1);
+    p->tape_ok = false;
+    if (int rc = launch_forward(p, controls, false)) return rc;
+    return finish_lindblad(p, costs, nullptr, final_densities);
+}
+
+int qocb_lindblad_batch_cost_and_grad(qocb_lplan *p, const double *controls, double *costs, double *grads,
+                                      double *final_densities) {
+    if (!p) return -1;
+    if (!p->batch) return lfail(p, "qocb_lindblad_batch_cost_and_grad needs qocb_lindblad_set_control_batch", -1);
+    p->tape_ok = false;
+    if (int rc = launch_forward(p, controls, true)) return rc;
+    if (int rc = launch_backward(p, nullptr)) return rc;
+    return finish_lindblad(p, costs, grads, final_densities);
 }
 
 /* stats[0] = Runge-Kutta attempts, stats[1] = accepted steps of the last evaluation (sums over the members of an ensemble) */
