@@ -107,6 +107,19 @@ int qocb_set_states(qocb_plan *plan, const double *psi0);
    weight = cost_multiplier / normalisation; step_cost != 0: evaluated at every cost step, else final step only */
 int qocb_add_cost(qocb_plan *plan, int32_t kind, int32_t step_cost, double weight,
                   const double *vectors, const int32_t *counts, int32_t fmax);
+/* MEMBER INITIAL STATES AND COST TARGETS (band-selective and multi-target ensembles).  psi0: [E][S][n] complex, member e's
+   own initial states; call after qocb_set_states, whose [S][n] it replaces for every member (a later qocb_set_states
+   returns the plan to shared states).  The buffer grows to E copies; the kernels read member e's at e * S * n.  Returns -1
+   for control batches, hilbert_size > 64, time-sliced and state-sharded plans. */
+int qocb_set_member_states(qocb_plan *plan, const double *psi0);
+/* a cost term whose vectors differ per member: vectors [E][S][fmax][n] complex, counts [S] (or NULL) shared by all
+   members; kind, step_cost and weight as for qocb_add_cost.  Member e's inner products and seeds use its own vectors.
+   Shared and member terms may be mixed; once a plan has a member term its device table holds one block of all terms per
+   member (shared vectors copied into every block), and each member's kernels read their block as a one-member plan reads
+   its table.  Identical vectors for every member give the bits of the same term added with qocb_add_cost.  Returns -1
+   where qocb_set_member_states does. */
+int qocb_add_member_cost(qocb_plan *plan, int32_t kind, int32_t step_cost, double weight,
+                         const double *vectors, const int32_t *counts, int32_t fmax);
 int qocb_clear_costs(qocb_plan *plan);
 
 /* controls: [M][KR] real.  cost: 1 double.  final_states: [E][S][n] complex or NULL. */
@@ -246,8 +259,9 @@ int qocb_expm_batched_bench(int32_t n, int64_t batch, double norm_scale, int32_t
 
    ENSEMBLES (robust control over drifts, control operators and decay rates).  ensemble_count = E > 1 runs E members, one CTA
    each, in one launch of each kernel.  Members differ in the drift H0 and/or the rates gamma_l (qocb_lindblad_set_ensemble)
-   and optionally in the control operators (qocb_lindblad_set_member_operators); rho0, Lindblad operators, cost terms,
-   controls and the time series are shared.  Every member runs exactly the code and the launch
+   and optionally in the control operators (qocb_lindblad_set_member_operators), the initial densities
+   (qocb_lindblad_set_member_densities) and the cost matrices (qocb_lindblad_add_member_cost); the Lindblad operators,
+   the cost term structure, controls and the time series are shared.  Every member runs exactly the code and the launch
    layout of a one-member plan of the same shape, so its results are bit-identical to such a plan built with its drift and
    rates.  The cost and gradient are the member mean: sums in member order 0..E-1 divided by E (no atomics).  Each member has
    its own tape of max_rk_steps steps (0: max(4096, min(2^20, 8 GiB / (E * 2 * D n^2 * 16 B)))); a member whose forward
@@ -303,6 +317,18 @@ int qocb_lindblad_set_densities(qocb_lplan *plan, const double *rho0);
 /* mats: [D][fmax][n][n]; counts: [D] or NULL; weight = cost_multiplier / normalisation; step_cost as above */
 int qocb_lindblad_add_cost(qocb_lplan *plan, int32_t kind, int32_t step_cost, double weight, const double *mats,
                            const int32_t *counts, int32_t fmax);
+/* MEMBER INITIAL DENSITIES AND COST TARGETS.  rho0: [E][D][n][n], member e's own initial densities (replaces those of
+   qocb_lindblad_set_densities for every member; a later qocb_lindblad_set_densities returns to shared densities).
+   Returns -1 for a control batch.  Each member still runs the thread count,
+   shared-memory layout and code of a one-member plan, reading its own rho0 and cost matrices, so its results are
+   bit-identical to a one-member plan built with its data.  The split calls qocb_lindblad_forward / _backward refuse
+   ensembles, so they never see member data. */
+int qocb_lindblad_set_member_densities(qocb_lplan *plan, const double *rho0);
+/* a density cost whose matrices differ per member: mats [E][D][fmax][n][n], counts [D] (or NULL) shared by the members;
+   kind, step_cost and weight as for qocb_lindblad_add_cost.  Shared and member terms may be mixed.  Returns -1 for a
+   control batch. */
+int qocb_lindblad_add_member_cost(qocb_lplan *plan, int32_t kind, int32_t step_cost, double weight, const double *mats,
+                                  const int32_t *counts, int32_t fmax);
 /* controls: [M][KR]; final_densities: [D][n][n] or NULL; grad: [M][KR].  Ensemble: member-mean cost and gradient, and
    final_densities [E][D][n][n] */
 int qocb_lindblad_cost(qocb_lplan *plan, const double *controls, double *cost, double *final_densities);
@@ -337,7 +363,8 @@ int qocb_lindblad_backward(qocb_lplan *plan, const double *seeds, double *grad);
    start's stage time left the series (qocb_lindblad_max_stage_time gives the largest over the starts).
    qocb_lindblad_set_control_batch returns -1 once operators are set and for plans without controls (have_hamiltonian = 0 or
    control_count = 0).  On a control batch qocb_lindblad_cost, qocb_lindblad_cost_and_grad, qocb_lindblad_forward,
-   qocb_lindblad_backward, qocb_lindblad_set_ensemble and qocb_lindblad_set_member_operators return -1;
+   qocb_lindblad_backward, qocb_lindblad_set_ensemble, qocb_lindblad_set_member_operators,
+   qocb_lindblad_set_member_densities and qocb_lindblad_add_member_cost return -1;
    qocb_lindblad_member_results gives each start's cost, gradient and stats, qocb_lindblad_get_densities [B][N][D][n][n] and
    qocb_lindblad_stats the sums over the starts. */
 int qocb_lindblad_set_control_batch(qocb_lplan *plan);

@@ -34,6 +34,7 @@ EXPORTS = [
     "qocb_lindblad_member_results", "qocb_set_member_operators", "qocb_lindblad_set_member_operators",
     "qocb_set_control_batch", "qocb_batch_cost", "qocb_batch_cost_and_grad",
     "qocb_lindblad_set_control_batch", "qocb_lindblad_batch_cost", "qocb_lindblad_batch_cost_and_grad",
+    "qocb_set_member_states", "qocb_add_member_cost", "qocb_lindblad_set_member_densities", "qocb_lindblad_add_member_cost",
 ]
 
 
@@ -121,6 +122,8 @@ def load():
     lib.qocb_set_node_map.argtypes = [vp, vp, vp]
     lib.qocb_set_states.argtypes = [vp, vp]
     lib.qocb_add_cost.argtypes = [vp, i32, i32, dbl, vp, vp, i32]
+    lib.qocb_set_member_states.argtypes = [vp, vp]
+    lib.qocb_add_member_cost.argtypes = [vp, i32, i32, dbl, vp, vp, i32]
     lib.qocb_clear_costs.argtypes = [vp]
     lib.qocb_cost.argtypes = [vp, vp, vp, vp]
     lib.qocb_cost_and_grad.argtypes = [vp, vp, vp, vp, vp]
@@ -150,6 +153,8 @@ def load():
     lib.qocb_lindblad_set_operators.argtypes = [vp, vp, vp, vp, vp]
     lib.qocb_lindblad_set_densities.argtypes = [vp, vp]
     lib.qocb_lindblad_add_cost.argtypes = [vp, i32, i32, dbl, vp, vp, i32]
+    lib.qocb_lindblad_set_member_densities.argtypes = [vp, vp]
+    lib.qocb_lindblad_add_member_cost.argtypes = [vp, i32, i32, dbl, vp, vp, i32]
     lib.qocb_lindblad_cost.argtypes = [vp, vp, vp, vp]
     lib.qocb_lindblad_cost_and_grad.argtypes = [vp, vp, vp, vp, vp]
     lib.qocb_lindblad_forward.argtypes = [vp, vp, vp, vp]

@@ -309,6 +309,68 @@ def is_user_cost(cost):
             and getattr(t, "control_value_and_grad", Cost.control_value_and_grad) is Cost.control_value_and_grad)
 
 
+def _is_control_only(cost):
+    from qoc_b200.models.cost import Cost
+    return getattr(type(cost), "control_value_and_grad", Cost.control_value_and_grad) is not Cost.control_value_and_grad
+
+
+def member_count(**counts):
+    """the common member count of the ensemble arguments that are given (name=count or None); ValueError when they differ."""
+    given = {k: v for k, v in counts.items() if v is not None}
+    if len(set(given.values())) > 1:
+        raise ValueError("the ensemble arguments disagree on the member count: " +
+                         ", ".join("{} has {}".format(k, v) for k, v in sorted(given.items())))
+    return next(iter(given.values())) if given else None
+
+
+def member_cost_terms(costs, ensemble_costs, terms_of, is_user):
+    """device terms whose vectors (or matrices) differ per member: [(kind, step, weight, vecs [E][...], counts)], one per
+    device term of the state (or density) costs in `costs`, member e's from `ensemble_costs[e]` through each cost's own
+    `terms_of(c)` (`device_terms` / `device_terms_density`).  Every member list must produce the same term sequence as the
+    state costs in `costs` - kind, step flag, weight, vector shapes and counts - else ValueError; control-only costs belong in
+    `costs` (ValueError), user-defined ones are not supported (NotImplementedError).  Nothing touches a device."""
+    lists = list(ensemble_costs)
+    if not lists:
+        raise ValueError("ensemble_costs needs at least one member")
+
+    def terms(cs, where):
+        out = []
+        for c in cs:
+            if is_user(c):
+                raise NotImplementedError("user-defined costs cannot be combined with ensemble_costs ({})".format(where))
+            if where != "costs" and _is_control_only(c):
+                raise ValueError("{} holds the control-only cost {}: control costs are shared, pass them in `costs`".format(
+                    where, c))
+            if _is_control_only(c):
+                continue
+            ts = terms_of(c)
+            if ts is None:
+                raise NotImplementedError("The cost {} in {} has no B200 device descriptor for this path (no CPU "
+                                          "fallback).".format(c, where))
+            for kind, step, weight, vecs, counts in ts:
+                vecs = np.ascontiguousarray(vecs, dtype=np.complex128)
+                counts = np.full(vecs.shape[0], vecs.shape[1], dtype=np.int32) if counts is None else \
+                    np.ascontiguousarray(counts, dtype=np.int32)
+                out.append((int(kind), int(step), float(weight), vecs, counts))
+        return out
+    nominal = terms(costs, "costs")
+    members = []
+    for e, cs in enumerate(lists):
+        if not isinstance(cs, (list, tuple)):
+            raise ValueError("ensemble_costs[{}] must be a list of costs".format(e))
+        got = terms(cs, "ensemble_costs[{}]".format(e))
+        if len(got) != len(nominal):
+            raise ValueError("ensemble_costs[{}] gives {} device terms, the state costs in `costs` {}".format(
+                e, len(got), len(nominal)))
+        for i, (a, b) in enumerate(zip(got, nominal)):
+            if a[:3] != b[:3] or a[3].shape != b[3].shape or not np.array_equal(a[4], b[4]):
+                raise ValueError("ensemble_costs[{}] term {} differs from the state costs in `costs` in its kind, step flag, "
+                                 "weight, vector shape or counts".format(e, i))
+        members.append(got)
+    return [(b[0], b[1], b[2], np.ascontiguousarray(np.stack([m[i][3] for m in members])), b[4])
+            for i, b in enumerate(nominal)]
+
+
 class SchroedingerPlan(object):
     """Device plan for `_evaluate_schroedinger_discrete` and its jacobian (schroedingerdiscrete.py:356-438,
     :318).  `cost(controls)` and `cost_and_grad(controls)` take controls in cost-function format
@@ -319,10 +381,17 @@ class SchroedingerPlan(object):
                  magnus_policy=MagnusPolicy.M2, cost_eval_step=1,
                  interpolation_policy=InterpolationPolicy.LINEAR, device=0, store_tape=True,
                  chunks_per_member=0, ensemble_drifts=None, structure=None, slice_range=None, state_slice=None,
-                 ensemble_hamiltonians=None, control_batch=None):
+                 ensemble_hamiltonians=None, control_batch=None, ensemble_initial_states=None, ensemble_costs=None):
         """`ensemble_drifts` [E][n][n] (members differ in the drift) or `ensemble_hamiltonians` [h_0 .. h_{E-1}] (callables
         like `hamiltonian`: members differ in the drift and the control operators, e.g. drive-amplitude or crosstalk errors)
         make a robust-control ensemble: cost and gradient are the member mean, final and intermediate states per member.
+
+        `ensemble_initial_states` [E][S][n][1] and `ensemble_costs` (E lists of state costs) give every member its own
+        initial states and cost targets (band-selective and multi-target pulses), alone or with the member hamiltonians:
+        member e's states replace `initial_states`, and the target / forbidden vectors of its list replace those of the
+        state costs in `costs`, which set the term structure every list must repeat (ValueError otherwise).  Control costs
+        stay in `costs`, added once.  Not combinable with control batches, sharding, user-defined costs, time-dependent or
+        non-linear hamiltonians, or n > 64 (NotImplementedError, before any device call).
 
         `control_batch=B` evaluates B independent control sets of this one problem per call (multi-start optimisation):
         `cost(controls [B][M][K])` returns (errors [B], final states [B][S][n][1]), `cost_and_grad` also grads [B][M][K],
@@ -331,16 +400,21 @@ class SchroedingerPlan(object):
         call)."""
         if ensemble_drifts is not None and ensemble_hamiltonians is not None:
             raise ValueError("pass ensemble_drifts or ensemble_hamiltonians, not both")
-        ensemble = ensemble_drifts is not None or ensemble_hamiltonians is not None
+        member_data = ensemble_initial_states is not None or ensemble_costs is not None
+        ensemble = ensemble_drifts is not None or ensemble_hamiltonians is not None or member_data
         self.B = None
         if control_batch is not None:
             if isinstance(control_batch, bool) or not isinstance(control_batch, (int, np.integer)) or control_batch < 1:
                 raise ValueError("control_batch must be a positive integer, got {!r}".format(control_batch))
+            if member_data:
+                raise NotImplementedError("control batches cannot be combined with ensemble_initial_states / ensemble_costs")
             if ensemble:
                 raise NotImplementedError("control batches cannot be combined with ensemble_drifts / ensemble_hamiltonians")
             if slice_range is not None or state_slice is not None:
                 raise NotImplementedError("control batches cannot be combined with time-slice or state sharding")
             self.B = int(control_batch)
+        if member_data and slice_range is not None:
+            raise NotImplementedError("ensemble_initial_states / ensemble_costs cannot be combined with time-slice sharding")
         if interpolation_policy != InterpolationPolicy.LINEAR:
             raise NotImplementedError("The interpolation policy {} is not yet supported for this method."
                                       "".format(interpolation_policy))
@@ -371,8 +445,20 @@ class SchroedingerPlan(object):
         user_cost = lambda c: (getattr(type(c), "device_terms", Cost.device_terms) is Cost.device_terms and
                                getattr(type(c), "control_value_and_grad", Cost.control_value_and_grad) is
                                Cost.control_value_and_grad)
-        if ensemble_hamiltonians is not None and any(user_cost(c) for c in self.costs):
+        if (ensemble_hamiltonians is not None or member_data) and any(user_cost(c) for c in self.costs):
             raise NotImplementedError("user-defined costs cannot be combined with ensembles or sharded plans")
+        member_states = member_terms = None
+        if member_data:
+            if self.n > 64:
+                raise NotImplementedError("ensemble_initial_states / ensemble_costs are not implemented for hilbert_size > 64")
+            if ensemble_initial_states is not None:
+                member_states = np.asarray(ensemble_initial_states)
+                if member_states.ndim != 4 or member_states.shape[0] < 1 or member_states.shape[1:] != initial_states.shape:
+                    raise ValueError("ensemble_initial_states must have shape [E]{}, got {}".format(
+                        list(initial_states.shape), member_states.shape))
+            if ensemble_costs is not None:
+                member_terms = member_cost_terms(self.costs, ensemble_costs, lambda c: c.device_terms(self.S_total, self.n),
+                                                 user_cost)
         if self.B is not None:
             if any(user_cost(c) for c in self.costs):
                 raise NotImplementedError("user-defined costs cannot be combined with control batches")
@@ -383,10 +469,12 @@ class SchroedingerPlan(object):
                 structure = extract_hamiltonian_structure(hamiltonian, self.K, self.complex_controls, evolution_time,
                                                           system_eval_count=self.N, magnus_order=magnus_policy.order)
             except NonlinearHamiltonian as err:
-                if self.B is None:
+                if self.B is None and not member_data:
                     raise
-                # a plain NotImplementedError: make_schroedinger_plan must not route a batch to NonlinearSchroedingerPlan
-                raise NotImplementedError("control batches need a hamiltonian affine in the controls: {}".format(err)) from err
+                # a plain NotImplementedError: make_schroedinger_plan must not route a batch or member data to
+                # NonlinearSchroedingerPlan
+                raise NotImplementedError("{} need a hamiltonian affine in the controls: {}".format(
+                    "control batches" if self.B is not None else "ensemble_initial_states / ensemble_costs", err)) from err
         self.structure = structure
         h0, a_ops = structure[0], structure[1]
         node_map = structure[2:] if len(structure) == 4 else None
@@ -396,6 +484,9 @@ class SchroedingerPlan(object):
             raise NotImplementedError("ensemble drifts with a time-dependent hamiltonian are not supported")
         if node_map is not None and ensemble_hamiltonians is not None:
             raise NotImplementedError("ensemble hamiltonians with a time-dependent hamiltonian are not supported")
+        if node_map is not None and member_data:
+            raise NotImplementedError("ensemble_initial_states / ensemble_costs with a time-dependent hamiltonian are not "
+                                      "supported")
         if h0.shape[0] != self.n:
             raise ValueError("hamiltonian size {} does not match the states' hilbert size {}".format(h0.shape[0], self.n))
         member_ops = None                        # [E][KR][n][n] when the members' control operators differ
@@ -408,6 +499,13 @@ class SchroedingerPlan(object):
                 member_ops, a_ops = a_ops, a_ops[0]
         else:
             h0s = np.ascontiguousarray(h0[None], dtype=np.complex128)
+        if member_data:
+            E = member_count(**{"ensemble_drifts" if ensemble_hamiltonians is None else "ensemble_hamiltonians":
+                                None if ensemble_drifts is None and ensemble_hamiltonians is None else h0s.shape[0],
+                                "ensemble_initial_states": None if member_states is None else member_states.shape[0],
+                                "ensemble_costs": None if ensemble_costs is None else len(ensemble_costs)})
+            if ensemble_drifts is None and ensemble_hamiltonians is None:     # the drift-only route with identical drifts
+                h0s = np.ascontiguousarray(np.broadcast_to(h0, (E,) + h0.shape), dtype=np.complex128)
         self.E = h0s.shape[0] if self.B is None else self.B
         pb = _lib.Problem(hilbert_size=self.n, state_count=self.S, control_count=self.KR,
                           control_eval_count=self.M, system_eval_count=self.N,
@@ -434,9 +532,14 @@ class SchroedingerPlan(object):
             _lib.check(self.lib.qocb_set_node_map(handle, _lib.ptr(offset), _lib.ptr(gain) if self.KR else None), handle)
         psi0 = np.ascontiguousarray(initial_states.reshape(self.S, self.n), dtype=np.complex128)
         _lib.check(self.lib.qocb_set_states(handle, _lib.ptr(psi0)), handle)
+        if member_states is not None:
+            mpsi = np.ascontiguousarray(member_states.reshape(self.E, self.S, self.n), dtype=np.complex128)
+            _lib.check(self.lib.qocb_set_member_states(handle, _lib.ptr(mpsi)), handle)
         self.control_costs = []
         self.user_costs = []
         for c in self.costs:
+            if member_terms is not None and not _is_control_only(c):
+                continue                                 # its terms are added per member below
             if user_cost(c):
                 # a user-defined Cost subclass (qoc/models/cost.py:5-51): only `cost(controls, states, step)` exists.  Its value and
                 # a numeric cotangent of the final states are computed on the host around qocb_forward / qocb_backward.
@@ -463,6 +566,9 @@ class SchroedingerPlan(object):
                 _lib.check(self.lib.qocb_add_cost(handle, kind, step, float(weight), _lib.ptr(vecs),
                                                   None if cnt is None else cnt.ctypes.data_as(ctypes.c_void_p),
                                                   vecs.shape[1]), handle)
+        for kind, step, weight, vecs, cnt in member_terms or []:
+            _lib.check(self.lib.qocb_add_member_cost(handle, kind, step, weight, _lib.ptr(vecs),
+                                                     cnt.ctypes.data_as(ctypes.c_void_p), vecs.shape[2]), handle)
 
     # -- helpers ------------------------------------------------------------------------------------
     def _real_channels(self, controls):
@@ -1098,7 +1204,12 @@ class LindbladPlan(object):
     [h_0 .. h_{E-1}] (callables like `hamiltonian`) its drift and control operators, and `ensemble_rates` [E][L] the decay
     rates of `lindblad_data`, member by member.  `cost` and `cost_and_grad` then return the member mean (control
     costs added once) with final densities [E][D][n][n], `intermediate_densities()` is [E][N][D][n][n] and `member_results()`
-    returns every member's cost, gradient and stats.  One member is the plain plan.
+    returns every member's cost, gradient and stats.  One member is the plain plan.  `ensemble_initial_densities` [E][D][n][n]
+    and `ensemble_costs` (E lists of density costs) give every member its own initial densities and cost targets, alone or
+    with the arguments above (every E must agree): member e's densities replace `initial_densities`, and the target /
+    forbidden matrices of its list replace those of the density costs in `costs`, which set the term structure every list
+    must repeat (ValueError otherwise); control costs stay in `costs`.  Each member is still bit-identical to a one-member
+    plan built with its data.  Time dependence is allowed where the ensemble arguments it is combined with allow it.
 
     Control batches (multi-start optimisation): `control_batch=B` evaluates B independent control sets of this one problem
     per call, one CTA per start.  `cost(controls [B][M][K])` returns (errors [B], final densities [B][D][n][n]) and
@@ -1110,13 +1221,18 @@ class LindbladPlan(object):
     def __init__(self, initial_densities, costs, evolution_time, system_eval_count, hamiltonian=None,
                  lindblad_data=None, control_eval_count=0, control_count=0, complex_controls=False, cost_eval_step=1,
                  interpolation_policy=InterpolationPolicy.LINEAR, device=0, max_rk_steps=0, structure=None,
-                 ensemble_drifts=None, ensemble_rates=None, ensemble_hamiltonians=None, control_batch=None):
+                 ensemble_drifts=None, ensemble_rates=None, ensemble_hamiltonians=None, control_batch=None,
+                 ensemble_initial_densities=None, ensemble_costs=None):
         self.B = None
+        member_data = ensemble_initial_densities is not None or ensemble_costs is not None
         if control_batch is not None:
             if isinstance(control_batch, bool) or not isinstance(control_batch, (int, np.integer)) or control_batch < 1:
                 raise ValueError("control_batch must be a positive integer, got {!r}".format(control_batch))
             if hamiltonian is None or int(control_count) < 1:
                 raise ValueError("control batches need a hamiltonian and control_count >= 1: there are no controls to batch")
+            if member_data:
+                raise NotImplementedError("control batches cannot be combined with ensemble_initial_densities / "
+                                          "ensemble_costs")
             if ensemble_drifts is not None or ensemble_rates is not None or ensemble_hamiltonians is not None:
                 raise NotImplementedError("control batches cannot be combined with ensemble_drifts / ensemble_rates / "
                                           "ensemble_hamiltonians")
@@ -1163,7 +1279,28 @@ class LindbladPlan(object):
             raise ValueError("hamiltonian size {} does not match the densities' hilbert size {}".format(h0.shape[0], self.n))
         self.L = 0 if lops is None else lops.shape[0]
         h0s, rates, ops = self._ensemble_members(ensemble_drifts, ensemble_rates, ensemble_hamiltonians, td_h, td_l)
+        self._member_rho0 = self._member_terms = None
+        if member_data:
+            if any(is_user_cost(c) for c in self.costs):
+                raise NotImplementedError("user-defined costs cannot be combined with ensembles")
+            if ensemble_initial_densities is not None:
+                self._member_rho0 = np.ascontiguousarray(ensemble_initial_densities, dtype=np.complex128)
+                if self._member_rho0.ndim != 4 or self._member_rho0.shape[0] < 1 or self._member_rho0.shape[1:] != rho0.shape:
+                    raise ValueError("ensemble_initial_densities must have shape [E]{}, got {}".format(
+                        list(rho0.shape), self._member_rho0.shape))
+            if ensemble_costs is not None:
+                self._member_terms = member_cost_terms(
+                    self.costs, ensemble_costs,
+                    lambda c: c.device_terms_density(self.D, self.n) if hasattr(c, "device_terms_density") else None,
+                    is_user_cost)
+            E = member_count(**{"ensemble_drifts" if ensemble_hamiltonians is None else "ensemble_hamiltonians":
+                                None if h0s is None else h0s.shape[0],
+                                "ensemble_rates": None if rates is None else rates.shape[0],
+                                "ensemble_initial_densities": None if self._member_rho0 is None else self._member_rho0.shape[0],
+                                "ensemble_costs": None if ensemble_costs is None else len(ensemble_costs)})
         self.E = 1 if h0s is None and rates is None else (h0s if h0s is not None else rates).shape[0]
+        if member_data:
+            self.E = E
         if self.B is not None:
             self.E = self.B
         member_ops = None                                # [E][KR][n][n] when the members' control operators differ
@@ -1188,6 +1325,8 @@ class LindbladPlan(object):
             if is_user_cost(c):
                 self.user_costs.append(c)
                 continue
+            if self._member_terms is not None and not _is_control_only(c):
+                continue                                 # its terms are added per member below
             terms = c.device_terms_density(self.D, self.n) if hasattr(c, "device_terms_density") else None
             if not terms:
                 # only genuine control-only costs (classes that override the analytic hook) may skip the device: a state
@@ -1200,9 +1339,13 @@ class LindbladPlan(object):
                 self.control_costs.append(c)
             for kind, step, weight, mats, counts in terms:
                 term = (kind, step, float(weight), np.ascontiguousarray(mats, dtype=np.complex128),
-                        None if counts is None else np.ascontiguousarray(counts, dtype=np.int32))
+                        None if counts is None else np.ascontiguousarray(counts, dtype=np.int32), False)
                 self._terms.append(term)
                 self._add_term(term)
+        for kind, step, weight, mats, counts in self._member_terms or []:
+            term = (kind, step, weight, mats, counts, True)
+            self._terms.append(term)
+            self._add_term(term)
         # user costs by system step, where the reference evaluates them (lindbladdiscrete.py:384-441): step costs at every
         # k % cost_eval_step == 0, k != 0, the others once on the final densities
         ces = int(cost_eval_step)
@@ -1281,14 +1424,17 @@ class LindbladPlan(object):
             if self._members[2] is not None:
                 self._check(self.lib.qocb_lindblad_set_member_operators(handle, _lib.ptr(self._members[2])))
         self._check(self.lib.qocb_lindblad_set_densities(handle, _lib.ptr(su["rho0"])))
+        if self._member_rho0 is not None:
+            self._check(self.lib.qocb_lindblad_set_member_densities(handle, _lib.ptr(self._member_rho0)))
         if st is not None:
             self._check(self.lib.qocb_lindblad_set_time_series(handle, st.segments, st.degree, st.width, _lib.ptr(st.series)))
 
     def _add_term(self, term):
-        kind, step, weight, mats, cnt = term
-        self._check(self.lib.qocb_lindblad_add_cost(self.handle, kind, step, weight, _lib.ptr(mats),
-                                                    None if cnt is None else cnt.ctypes.data_as(ctypes.c_void_p),
-                                                    mats.shape[1]))
+        """term: (kind, step, weight, mats, counts, member) - mats [D][fmax][n][n], or [E][D][fmax][n][n] for a member term"""
+        kind, step, weight, mats, cnt, member = term
+        add = self.lib.qocb_lindblad_add_member_cost if member else self.lib.qocb_lindblad_add_cost
+        self._check(add(self.handle, kind, step, weight, _lib.ptr(mats),
+                        None if cnt is None else cnt.ctypes.data_as(ctypes.c_void_p), mats.shape[2 if member else 1]))
 
     _MAX_RANGE_EXTENSIONS = 4
 

@@ -433,14 +433,30 @@ class StateShardedPlan(object):
             self.plan.close()
 
 
+def member_share(rank, world, **members):
+    """rank's block of every per-member argument given (name=[E] sequence or None): (local arguments, (first, end), E).
+    The members are block-partitioned as `slice_bounds` partitions slices; ValueError when the arguments disagree on E."""
+    given = {k: v for k, v in members.items() if v is not None}
+    counts = {k: len(v) for k, v in given.items()}
+    if len(set(counts.values())) != 1:
+        raise ValueError("the per-member arguments disagree on the member count: " +
+                         ", ".join("{} has {}".format(k, v) for k, v in sorted(counts.items())))
+    E = next(iter(counts.values()))
+    b = slice_bounds(E, world)
+    lo, hi = b[rank], b[rank + 1]
+    return {k: v[lo:hi] for k, v in given.items()}, (lo, hi), E
+
+
 class EnsembleShardedPlan(object):
     """robust-control ensembles (cfg5): members that differ in the drift (`ensemble_drifts`) or in drift and control
-    operators (`ensemble_hamiltonians`, callables like `hamiltonian`) are independent units, block-partitioned across the
-    ranks; one NCCL all-reduce of [gradient | cost] on the plan stream ends the evaluation - inside the device-timed region,
-    no host bounce.  Cost = mean over members.  `cost_and_grad` returns the final states of the LOCAL members."""
+    operators (`ensemble_hamiltonians`, callables like `hamiltonian`), and optionally in their initial states and cost
+    targets (`ensemble_initial_states`, `ensemble_costs`; a shared drift is `ensemble_drifts=[h0] * E`), are independent
+    units, block-partitioned across the ranks; one NCCL all-reduce of [gradient | cost] on the plan stream ends the
+    evaluation - inside the device-timed region, no host bounce.  Cost = mean over members.  `cost_and_grad` returns the
+    final states of the LOCAL members."""
 
     def __init__(self, hamiltonian, initial_states, costs, evolution_time, system_eval_count, ensemble_drifts=None, device=0,
-                 group=None, ensemble_hamiltonians=None, **kw):
+                 group=None, ensemble_hamiltonians=None, ensemble_initial_states=None, ensemble_costs=None, **kw):
         if (ensemble_drifts is None) == (ensemble_hamiltonians is None):
             raise ValueError("EnsembleShardedPlan needs exactly one of ensemble_drifts and ensemble_hamiltonians")
         import torch
@@ -448,14 +464,13 @@ class EnsembleShardedPlan(object):
         self.torch, self.dist, self.group = torch, dist, group
         self.rank, self.world = dist.get_rank(group), dist.get_world_size(group)
         self.comm = TorchDistComm(group)
-        members = np.asarray(ensemble_drifts) if ensemble_hamiltonians is None else list(ensemble_hamiltonians)
-        self.E_total = len(members)
-        b = slice_bounds(self.E_total, self.world)
-        self.member_range = (b[self.rank], b[self.rank + 1])
-        local = members[b[self.rank]:b[self.rank + 1]]
+        local, self.member_range, self.E_total = member_share(
+            self.rank, self.world, ensemble_drifts=None if ensemble_drifts is None else np.asarray(ensemble_drifts),
+            ensemble_hamiltonians=None if ensemble_hamiltonians is None else list(ensemble_hamiltonians),
+            ensemble_initial_states=None if ensemble_initial_states is None else np.asarray(ensemble_initial_states),
+            ensemble_costs=None if ensemble_costs is None else list(ensemble_costs))
         self.plan = SchroedingerPlan(hamiltonian, initial_states, costs, evolution_time, system_eval_count, device=device,
-                                     **(dict(ensemble_drifts=local) if ensemble_hamiltonians is None
-                                        else dict(ensemble_hamiltonians=local)), **kw)
+                                     **local, **kw)
         p = self.plan
         self.KR, self.K, self.M, self.S, self.n, self.E = p.KR, p.K, p.M, p.S, p.n, p.E
         self.complex_controls = p.complex_controls

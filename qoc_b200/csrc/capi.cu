@@ -564,6 +564,8 @@ struct qocb_plan {
     DevBuf<CostTerm> terms;
     std::vector<CostTerm> h_terms;
     std::vector<double> h_vecs;
+    std::vector<int> h_term_members;    // per term: 1 shared, E member term (h_vecs holds its [E][S][fmax] vectors)
+    long long vecs_mstride = 0;         // doubles per member of the uploaded vector table (0: no member terms)
     std::vector<int> h_counts;
     int ip_total = 0;
     int coh_total = 0;                  // overlap-sum slots of the coherent target terms (state sharding)
@@ -580,6 +582,7 @@ struct qocb_plan {
     bool drift_hermitian = false;       // H0 of every member is Hermitian (qocb_set_member_operators recomputes `hermitian`)
     bool member_ops = false;            // G, C0 and Cs hold every member's own control operators (qocb_set_member_operators)
     bool batch = false;                 // control batch (qocb_set_control_batch): member b has its own controls, cost and gradient
+    bool member_states = false;         // psi0 holds [E][S][2][NP], every member's own initial states (qocb_set_member_states)
     double *h_pinned = nullptr;         // [ctl_doubles controls | ctl_doubles grad | cost_count costs]
     // CUDA graph of one whole host-facing evaluation (H2D controls, all kernels, D2H of gradient, cost, final states and the
     // error flag): replayed by qocb_cost / qocb_cost_and_grad from the third call on - launch-bound small problems gain 2x
@@ -730,6 +733,8 @@ SweepArgs make_sargs(qocb_plan *p) {
         s.member_chunk0 = p->mc0_lvl.p + 2 * p->levels;
     }
     s.psi = p->psi.p; s.lam = p->lam.p; s.part = p->part.p; s.cost_part = p->cost_part.p; s.psi_in = p->psi0.p;
+    s.psi_mstride = p->member_states ? p->pb.state_count * 2 * p->NP : 0;
+    s.vecs_mstride = p->vecs_mstride;
     s.S_norm = p->state_sharded ? p->pb.state_total : p->pb.state_count;
     s.const_on = (!p->state_sharded || p->pb.state_first == 0) ? 1 : 0;
     s.coh_out = p->state_sharded ? p->coh_out : nullptr;
@@ -755,14 +760,35 @@ void pick_levels(qocb_plan *p) {
     else { p->levels = p->lv3s; p->coarse = p->lv3c; }
 }
 
+// with member terms (qocb_add_member_cost) the device table holds one block per member - its own vectors of member terms,
+// copies of the shared ones - with the terms' offsets inside a block, so member e's kernels read block e exactly as a
+// one-member plan reads its table
 int upload_costs(qocb_plan *p) {
     if (p->terms.n == p->h_terms.size() && p->terms.n > 0) return 0;
-    CU_TRY(p, p->terms.alloc(std::max<size_t>(1, p->h_terms.size())));
-    CU_TRY(p, p->vecs.alloc(std::max<size_t>(1, p->h_vecs.size())));
+    std::vector<CostTerm> terms = p->h_terms;
+    std::vector<double> packed;
+    const std::vector<double> *vecs = &p->h_vecs;
+    p->vecs_mstride = 0;
+    if (std::any_of(p->h_term_members.begin(), p->h_term_members.end(), [](int m) { return m > 1; })) {
+        const size_t E = p->pb.ensemble_count, S = p->pb.state_count, V = 2 * (size_t)p->NP;
+        size_t per = 0;                                                 // vectors of one member over all terms
+        for (auto &t : terms) { t.vec_off = (int)per; per += S * t.fmax; }
+        packed.resize(E * per * V);
+        for (size_t e = 0; e < E; ++e)
+            for (size_t i = 0; i < terms.size(); ++i) {
+                const size_t cnt = S * terms[i].fmax * V;
+                const double *src = p->h_vecs.data() + (size_t)p->h_terms[i].vec_off * V + (p->h_term_members[i] > 1 ? e * cnt : 0);
+                std::copy(src, src + cnt, packed.begin() + (e * per + terms[i].vec_off) * V);
+            }
+        vecs = &packed;
+        p->vecs_mstride = (long long)(per * V);
+    }
+    CU_TRY(p, p->terms.alloc(std::max<size_t>(1, terms.size())));
+    CU_TRY(p, p->vecs.alloc(std::max<size_t>(1, vecs->size())));
     CU_TRY(p, p->counts.alloc(std::max<size_t>(1, p->h_counts.size())));
-    if (!p->h_terms.empty()) {
-        CU_TRY(p, cudaMemcpy(p->terms.p, p->h_terms.data(), sizeof(CostTerm) * p->h_terms.size(), cudaMemcpyHostToDevice));
-        CU_TRY(p, cudaMemcpy(p->vecs.p, p->h_vecs.data(), sizeof(double) * p->h_vecs.size(), cudaMemcpyHostToDevice));
+    if (!terms.empty()) {
+        CU_TRY(p, cudaMemcpy(p->terms.p, terms.data(), sizeof(CostTerm) * terms.size(), cudaMemcpyHostToDevice));
+        CU_TRY(p, cudaMemcpy(p->vecs.p, vecs->data(), sizeof(double) * vecs->size(), cudaMemcpyHostToDevice));
         CU_TRY(p, cudaMemcpy(p->counts.p, p->h_counts.data(), sizeof(int) * p->h_counts.size(), cudaMemcpyHostToDevice));
     }
     return 0;
@@ -2054,24 +2080,63 @@ int qocb_set_states(qocb_plan *p, const double *psi0) {
         }
     CU_TRY(p, cudaMemcpy(p->psi0.p, buf.data(), sizeof(double) * buf.size(), cudaMemcpyHostToDevice));
     p->states_set = true;
+    if (p->member_states) { p->member_states = false; drop_graphs(p); }      // shared states again
+    return 0;
+}
+
+// per-member data (qocb_set_member_states, qocb_add_member_cost) needs the unsharded n <= 64 path and an ensemble plan
+static bool refuse_member_data(qocb_plan *p, const char *call) {
+    const char *why = p->batch ? "control batches share their initial states and cost targets"
+                      : p->large ? "is not implemented for hilbert_size > 64"
+                      : (p->sharded || p->state_sharded) ? "is not implemented for time-sharded or state-sharded plans" : nullptr;
+    if (!why) return false;
+    set_error(p, (std::string(call) + ": " + why).c_str());
+    return true;
+}
+
+int qocb_set_member_states(qocb_plan *p, const double *psi0) {
+    if (!p || !psi0) { set_error(p, "null argument"); return -1; }
+    if (refuse_member_data(p, "qocb_set_member_states")) return -1;
+    if (!p->states_set) { set_error(p, "qocb_set_member_states needs qocb_set_states first"); return -1; }
+    drop_graphs(p);
+    CU_TRY(p, cudaSetDevice(p->pb.device));
+    CU_TRY(p, cudaStreamSynchronize(p->stream));                          // no evaluation in flight reads psi0
+    const int n = p->pb.hilbert_size, NP = p->NP, S = p->pb.state_count, E = p->pb.ensemble_count;
+    const size_t VS = (size_t)S * 2 * NP;
+    std::vector<double> buf((size_t)E * VS, 0.0);
+    for (size_t es = 0; es < (size_t)E * S; ++es)
+        for (int a = 0; a < n; ++a) {
+            buf[es * 2 * NP + a] = psi0[2 * (es * n + a)];
+            buf[es * 2 * NP + NP + a] = psi0[2 * (es * n + a) + 1];
+        }
+    CU_TRY(p, p->psi0.alloc(buf.size()));
+    CU_TRY(p, cudaMemcpy(p->psi0.p, buf.data(), sizeof(double) * buf.size(), cudaMemcpyHostToDevice));
+    p->member_states = true;
     return 0;
 }
 
 int qocb_clear_costs(qocb_plan *p) {
     if (!p) return -1;
     drop_graphs(p);
-    p->h_terms.clear(); p->h_vecs.clear(); p->h_counts.clear(); p->ip_total = 0; p->coh_total = 0; p->have_step_costs = false;
+    p->h_terms.clear(); p->h_vecs.clear(); p->h_counts.clear(); p->h_term_members.clear(); p->ip_total = 0; p->coh_total = 0;
+    p->have_step_costs = false;
     pick_levels(p);
     p->terms.release();
     return 0;
 }
 
-int qocb_add_cost(qocb_plan *p, int32_t kind, int32_t step_cost, double weight, const double *vectors,
-                  const int32_t *counts, int32_t fmax) {
+// members: 1 for a shared term (vectors [S][fmax][n]), E for a member term (vectors [E][S][fmax][n]; upload_costs lays
+// them out per member)
+static int add_cost_term(qocb_plan *p, int32_t kind, int32_t step_cost, double weight, const double *vectors, const int32_t *counts,
+                  int32_t fmax, int members) {
     if (!p || !vectors) { set_error(p, "null argument"); return -1; }
     if (kind < 0 || kind > 2 || fmax < 1) { set_error(p, "bad cost kind or fmax"); return -1; }
     if (kind != QOCB_COST_FORBID && fmax != 1) { set_error(p, "target costs take one vector per state"); return -1; }
     const int n = p->pb.hilbert_size, NP = p->NP, S = p->pb.state_count;
+    for (int s = 0; s < S; ++s) {
+        const int F = counts ? counts[s] : fmax;
+        if (F < 1 || F > fmax) { set_error(p, "counts[s] must be in [1, fmax]"); return -1; }
+    }
     CostTerm t;
     t.kind = kind; t.step = step_cost ? 1 : 0; t.fmax = fmax; t.w = weight;
     t.vec_off = (int)(p->h_vecs.size() / (2 * (size_t)NP));
@@ -2080,26 +2145,33 @@ int qocb_add_cost(qocb_plan *p, int32_t kind, int32_t step_cost, double weight, 
     p->ip_total += S * fmax;
     t.coh_off = p->coh_total;
     if (kind == QOCB_COST_TARGET_COHERENT) p->coh_total += t.step ? (p->pb.system_eval_count - 1) / p->pb.cost_eval_step : 1;
-    const size_t base = p->h_vecs.size();
-    p->h_vecs.resize(base + (size_t)S * fmax * 2 * NP, 0.0);
-    for (int s = 0; s < S; ++s) {
-        const int F = counts ? counts[s] : fmax;
-        if (F < 1 || F > fmax) { set_error(p, "counts[s] must be in [1, fmax]"); return -1; }
-        p->h_counts.push_back(F);
-        for (int f = 0; f < fmax; ++f)
-            for (int a = 0; a < n; ++a) {
-                const size_t src = 2 * (((size_t)s * fmax + f) * n + a);
-                const size_t dst = base + ((size_t)s * fmax + f) * 2 * NP;
-                p->h_vecs[dst + a] = vectors[src];
-                p->h_vecs[dst + NP + a] = vectors[src + 1];
-            }
-    }
+    const size_t base = p->h_vecs.size(), nvec = (size_t)members * S * fmax;
+    p->h_vecs.resize(base + nvec * 2 * NP, 0.0);
+    for (int s = 0; s < S; ++s) p->h_counts.push_back(counts ? counts[s] : fmax);
+    for (size_t v = 0; v < nvec; ++v)                               // [members][S][fmax] vectors of n, planar with padding
+        for (int a = 0; a < n; ++a) {
+            p->h_vecs[base + v * 2 * NP + a] = vectors[2 * (v * n + a)];
+            p->h_vecs[base + v * 2 * NP + NP + a] = vectors[2 * (v * n + a) + 1];
+        }
     p->h_terms.push_back(t);
+    p->h_term_members.push_back(members);
     if (t.step) p->have_step_costs = true;
     pick_levels(p);
     p->terms.release();          // force re-upload
     drop_graphs(p);
     return 0;
+}
+
+int qocb_add_cost(qocb_plan *p, int32_t kind, int32_t step_cost, double weight, const double *vectors,
+                  const int32_t *counts, int32_t fmax) {
+    return add_cost_term(p, kind, step_cost, weight, vectors, counts, fmax, 1);
+}
+
+int qocb_add_member_cost(qocb_plan *p, int32_t kind, int32_t step_cost, double weight, const double *vectors,
+                         const int32_t *counts, int32_t fmax) {
+    if (!p) { set_error(p, "null argument"); return -1; }
+    if (refuse_member_data(p, "qocb_add_member_cost")) return -1;
+    return add_cost_term(p, kind, step_cost, weight, vectors, counts, fmax, p->pb.ensemble_count);
 }
 
 int qocb_upload_controls(qocb_plan *p, const double *controls) {

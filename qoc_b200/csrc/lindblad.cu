@@ -84,20 +84,24 @@ struct LArgs {
     double *tseen;                              // largest stage time of the forward pass
     const double2 *seeds;                       // [N][D*n*n] host-cost cotangents of the densities, or null
     long long ctl_stride;                       // start stride of the controls of a control batch: M*KR
+    long long mat_stride;                       // member stride of mats with member data: all terms' matrices of one member
 };
 
 // the arguments of ensemble member blockIdx.x: per-member densities, tape, interval indices, global work, cost, gradient,
 // stats, stage time and tape-overflow flag sit at member-major offsets.  An ensemble (BATCH = false) also offsets the drift,
 // K_half and rates, and the control operators when the members have their own (ops_stride > 0); controls are shared.  A
-// control batch (BATCH = true) offsets the controls instead and shares drift, K_half and rates.  rho0, Lindblad operators,
-// cost terms and the time series are always shared.  Member 0 is the whole plan when E = 1.  BATCH is a template parameter,
-// not a run-time stride, so that ordinary and ensemble plans keep the exact instruction stream they had before control
-// batches (run-time strides cost cfg2_lindblad_n2 0.6 %; DESIGN.md section 3.3).
-template <bool BATCH> __device__ __forceinline__ LArgs member_args(const LArgs &a0) {
+// control batch (BATCH = true) offsets the controls instead and shares drift, K_half and rates.  With member data
+// (MDATA = true: member initial densities or cost matrices) rho0 is [E][D n^2] and mats [E][mat_stride], every member's own
+// copy; otherwise rho0, the cost terms and their matrices are shared.  Lindblad operators and the time series are always
+// shared.  Member 0 is the whole plan when E = 1.  BATCH and MDATA are template parameters, not run-time strides, so that
+// ordinary and ensemble plans keep the exact instruction stream they had before control batches and member data (run-time
+// strides cost cfg2_lindblad_n2 0.6 %; DESIGN.md section 3.3).
+template <bool BATCH, bool MDATA> __device__ __forceinline__ LArgs member_args(const LArgs &a0) {
     LArgs a = a0;
     const size_t e = blockIdx.x, nn = (size_t)a.n * a.n, DE = (size_t)a.D * nn;
     if constexpr (BATCH) a.controls += e * a.ctl_stride;
     else { a.H0 += e * nn; a.Khalf += e * nn; a.gam += e * (size_t)max(a.L, 1); }
+    if constexpr (MDATA) { a.rho0 += e * DE; a.mats += e * a.mat_stride; }
     a.Aops += e * a.ops_stride;
     a.states += e * a.N * DE;
     a.tape_x += e * a.cap; a.tape_h += e * a.cap; a.tape_y += e * a.cap * DE; a.tape_k1 += e * a.cap * DE;
@@ -439,9 +443,9 @@ template <bool TD> __device__ void carve(const LArgs &a, unsigned char *smem, Ct
     for (int i = 0; i < narr; ++i) w.p[i] = base + (size_t)(i + 1) * DE;
 }
 
-template <bool TD, bool BATCH> __global__ void __launch_bounds__(LNT) k_lindblad_forward(LArgs a0, int keep_tape) {
+template <bool TD, bool BATCH, bool MDATA> __global__ void __launch_bounds__(LNT) k_lindblad_forward(LArgs a0, int keep_tape) {
     extern __shared__ __align__(16) unsigned char smem[];
-    const LArgs a = member_args<BATCH>(a0);
+    const LArgs a = member_args<BATCH, MDATA>(a0);
     Ctx c(a);
     Work w;
     carve<TD>(a, smem, c, w, 12);
@@ -529,9 +533,9 @@ template <bool TD, bool BATCH> __global__ void __launch_bounds__(LNT) k_lindblad
     if (threadIdx.x == 0) { *a.cost = cost; a.stats[0] = attempts; a.stats[1] = accepted; if (TD) *a.tseen = c.tseen; }
 }
 
-template <bool TD, bool BATCH> __global__ void __launch_bounds__(LNT) k_lindblad_backward(LArgs a0) {
+template <bool TD, bool BATCH, bool MDATA> __global__ void __launch_bounds__(LNT) k_lindblad_backward(LArgs a0) {
     extern __shared__ __align__(16) unsigned char smem[];
-    const LArgs a = member_args<BATCH>(a0);
+    const LArgs a = member_args<BATCH, MDATA>(a0);
     Ctx c(a);
     Work w;
     if (*a.err_flag) return;                          // the forward pass overflowed this member's tape: hit[] is not valid
@@ -656,6 +660,8 @@ struct qocb_lplan {
     bool ens_set = false;                          // qocb_lindblad_set_ensemble since the last qocb_lindblad_set_operators
     bool member_ops = false;                       // Aops holds [E][KR][n*n] (qocb_lindblad_set_member_operators)
     bool batch = false;                            // control batch: E starts, controls [E][M][KR] (qocb_lindblad_set_control_batch)
+    bool mdata = false;                            // member data uploaded: rho0 [E][DE], mats [E][mat_stride] (MDATA kernels)
+    long long mat_stride = 0;
     int cap = 0;                                   // tape capacity of one member
     bool ops_set = false, rho_set = false, costs_dirty = true, series_set = false;
     int NS = 0, segs = 0, deg = 0;                 // time series: NS = KC*(1+KR) + (time_dependent_rates ? L : 0)
@@ -668,6 +674,8 @@ struct qocb_lplan {
     Buf<long long> stats;
     Buf<DTerm> terms;
     std::vector<DTerm> h_terms; std::vector<double2> h_mats; std::vector<int> h_counts;
+    std::vector<int> h_term_members;               // per term: 1 shared, E member term (h_mats holds [E][D][fmax][n n])
+    std::vector<double2> h_rho0, h_member_rho0;    // [D][n n] of qocb_lindblad_set_densities; [E][D][n n] or empty
     std::vector<double> h_h0, h_gam, h_lops;       // the plan's operators (E > 1): members without their own take these
     size_t smem_fwd = 0, smem_bwd = 0;
     int in_smem_fwd = 0, in_smem_bwd = 0, ops_in_smem = 0;
@@ -694,6 +702,7 @@ LArgs make_largs(qocb_lplan *p) {
     a.KC = p->pb.channel_count; a.tdr = p->pb.time_dependent_rates; a.NS = p->NS; a.segs = p->segs; a.deg = p->deg;
     a.seg_w = p->seg_w; a.series = p->series.p; a.Kops = p->Kops.p; a.tseen = p->tseen.p; a.seeds = nullptr;
     a.ctl_stride = (long long)a.M * a.KR;
+    a.mat_stride = p->mat_stride;
     return a;
 }
 
@@ -716,14 +725,51 @@ void build_khalf(const double *lops, const double *gammas, int n, int L, double 
     }
 }
 
+bool has_member_data(const qocb_lplan *p) {
+    return !p->h_member_rho0.empty() || std::any_of(p->h_term_members.begin(), p->h_term_members.end(), [](int m) { return m > 1; });
+}
+
+// uploads the cost tables and, with member data, every member's rho0 and cost matrices: member e's matrices of all terms
+// (its own for member terms, copies of the shared ones) form block e of mats, so a member reads them exactly as a one-member
+// plan reads its table
 int upload_lcosts(qocb_lplan *p) {
     if (!p->costs_dirty) return 0;
-    LTRY(p, p->terms.alloc(std::max<size_t>(1, p->h_terms.size())));
-    LTRY(p, p->mats.alloc(std::max<size_t>(1, p->h_mats.size())));
+    LTRY(p, cudaStreamSynchronize(p->stream));                               // no evaluation in flight reads the tables
+    p->mdata = has_member_data(p);
+    std::vector<DTerm> terms = p->h_terms;
+    std::vector<double2> packed;
+    const std::vector<double2> *mats = &p->h_mats;
+    const size_t nn = (size_t)p->pb.hilbert_size * p->pb.hilbert_size, DE = (size_t)p->pb.density_count * nn, E = p->E;
+    p->mat_stride = 0;
+    if (p->mdata) {
+        size_t per = 0;                                                     // matrices of one member over all terms
+        for (auto &t : terms) { t.mat_off = (int)per; per += (size_t)p->pb.density_count * t.fmax; }
+        packed.resize(std::max<size_t>(1, E * per * nn));
+        for (size_t e = 0; e < E; ++e)
+            for (size_t i = 0; i < terms.size(); ++i) {
+                const size_t cnt = (size_t)p->pb.density_count * terms[i].fmax * nn;
+                const double2 *src = p->h_mats.data() + (size_t)p->h_terms[i].mat_off * nn + (p->h_term_members[i] > 1 ? e * cnt : 0);
+                std::copy(src, src + cnt, packed.begin() + (e * per + terms[i].mat_off) * nn);
+            }
+        mats = &packed;
+        p->mat_stride = (long long)(per * nn);
+        std::vector<double2> rho(E * DE);
+        for (size_t e = 0; e < E; ++e) {
+            const double2 *src = p->h_member_rho0.empty() ? p->h_rho0.data() : p->h_member_rho0.data() + e * DE;
+            std::copy(src, src + DE, rho.begin() + e * DE);
+        }
+        LTRY(p, p->rho0.alloc(rho.size()));
+        LTRY(p, cudaMemcpy(p->rho0.p, rho.data(), sizeof(double2) * rho.size(), cudaMemcpyHostToDevice));
+    } else if (p->rho0.n != DE) {                                           // back to shared densities
+        LTRY(p, p->rho0.alloc(DE));
+        LTRY(p, cudaMemcpy(p->rho0.p, p->h_rho0.data(), sizeof(double2) * DE, cudaMemcpyHostToDevice));
+    }
+    LTRY(p, p->terms.alloc(std::max<size_t>(1, terms.size())));
+    LTRY(p, p->mats.alloc(std::max<size_t>(1, mats->size())));
     LTRY(p, p->counts.alloc(std::max<size_t>(1, p->h_counts.size())));
-    if (!p->h_terms.empty()) {
-        LTRY(p, cudaMemcpy(p->terms.p, p->h_terms.data(), sizeof(DTerm) * p->h_terms.size(), cudaMemcpyHostToDevice));
-        LTRY(p, cudaMemcpy(p->mats.p, p->h_mats.data(), sizeof(double2) * p->h_mats.size(), cudaMemcpyHostToDevice));
+    if (!terms.empty()) {
+        LTRY(p, cudaMemcpy(p->terms.p, terms.data(), sizeof(DTerm) * terms.size(), cudaMemcpyHostToDevice));
+        LTRY(p, cudaMemcpy(p->mats.p, mats->data(), sizeof(double2) * mats->size(), cudaMemcpyHostToDevice));
         LTRY(p, cudaMemcpy(p->counts.p, p->h_counts.data(), sizeof(int) * p->h_counts.size(), cudaMemcpyHostToDevice));
     }
     p->costs_dirty = false;
@@ -756,11 +802,14 @@ int launch_forward(qocb_lplan *p, const double *controls, bool keep_tape) {
     const dim3 grid(p->E), block(lindblad_threads(p));
     const int kt = keep_tape ? 1 : 0;
     if (per_start(p)) {
-        if (p->NS > 0) k_lindblad_forward<true, true><<<grid, block, p->smem_fwd, p->stream>>>(a, kt);
-        else k_lindblad_forward<false, true><<<grid, block, p->smem_fwd, p->stream>>>(a, kt);
+        if (p->NS > 0) k_lindblad_forward<true, true, false><<<grid, block, p->smem_fwd, p->stream>>>(a, kt);
+        else k_lindblad_forward<false, true, false><<<grid, block, p->smem_fwd, p->stream>>>(a, kt);
+    } else if (p->mdata) {
+        if (p->NS > 0) k_lindblad_forward<true, false, true><<<grid, block, p->smem_fwd, p->stream>>>(a, kt);
+        else k_lindblad_forward<false, false, true><<<grid, block, p->smem_fwd, p->stream>>>(a, kt);
     } else {
-        if (p->NS > 0) k_lindblad_forward<true, false><<<grid, block, p->smem_fwd, p->stream>>>(a, kt);
-        else k_lindblad_forward<false, false><<<grid, block, p->smem_fwd, p->stream>>>(a, kt);
+        if (p->NS > 0) k_lindblad_forward<true, false, false><<<grid, block, p->smem_fwd, p->stream>>>(a, kt);
+        else k_lindblad_forward<false, false, false><<<grid, block, p->smem_fwd, p->stream>>>(a, kt);
     }
     LTRY(p, cudaGetLastError());
     return 0;
@@ -773,11 +822,14 @@ int launch_backward(qocb_lplan *p, const double2 *seeds) {
     a.seeds = seeds;
     const dim3 grid(p->E), block(lindblad_threads(p));
     if (per_start(p)) {
-        if (p->NS > 0) k_lindblad_backward<true, true><<<grid, block, p->smem_bwd, p->stream>>>(a);
-        else k_lindblad_backward<false, true><<<grid, block, p->smem_bwd, p->stream>>>(a);
+        if (p->NS > 0) k_lindblad_backward<true, true, false><<<grid, block, p->smem_bwd, p->stream>>>(a);
+        else k_lindblad_backward<false, true, false><<<grid, block, p->smem_bwd, p->stream>>>(a);
+    } else if (p->mdata) {
+        if (p->NS > 0) k_lindblad_backward<true, false, true><<<grid, block, p->smem_bwd, p->stream>>>(a);
+        else k_lindblad_backward<false, false, true><<<grid, block, p->smem_bwd, p->stream>>>(a);
     } else {
-        if (p->NS > 0) k_lindblad_backward<true, false><<<grid, block, p->smem_bwd, p->stream>>>(a);
-        else k_lindblad_backward<false, false><<<grid, block, p->smem_bwd, p->stream>>>(a);
+        if (p->NS > 0) k_lindblad_backward<true, false, false><<<grid, block, p->smem_bwd, p->stream>>>(a);
+        else k_lindblad_backward<false, false, false><<<grid, block, p->smem_bwd, p->stream>>>(a);
     }
     LTRY(p, cudaGetLastError());
     return 0;
@@ -888,14 +940,18 @@ int qocb_lindblad_create(const qocb_lindblad_problem *pb, qocb_lplan **out) {
     p->smem_fwd = p->in_smem_fwd ? need_f : fixed; p->smem_bwd = p->in_smem_bwd ? need_b : fixed;
     if (fixed > limit) { g_lerr = "hilbert_size too large for the Lindblad kernels' shared-memory operators"; delete p; return -1; }
     CTRY(p->work.alloc((p->in_smem_fwd && p->in_smem_bwd ? 1 : E) * 24 * DE));   // one slice per member when it is used
-    CTRY(cudaFuncSetAttribute(k_lindblad_forward<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
-    CTRY(cudaFuncSetAttribute(k_lindblad_backward<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
-    CTRY(cudaFuncSetAttribute(k_lindblad_forward<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
-    CTRY(cudaFuncSetAttribute(k_lindblad_backward<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
-    CTRY(cudaFuncSetAttribute(k_lindblad_forward<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
-    CTRY(cudaFuncSetAttribute(k_lindblad_backward<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
-    CTRY(cudaFuncSetAttribute(k_lindblad_forward<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
-    CTRY(cudaFuncSetAttribute(k_lindblad_backward<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
+    CTRY(cudaFuncSetAttribute(k_lindblad_forward<false, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
+    CTRY(cudaFuncSetAttribute(k_lindblad_backward<false, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
+    CTRY(cudaFuncSetAttribute(k_lindblad_forward<true, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
+    CTRY(cudaFuncSetAttribute(k_lindblad_backward<true, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
+    CTRY(cudaFuncSetAttribute(k_lindblad_forward<false, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
+    CTRY(cudaFuncSetAttribute(k_lindblad_backward<false, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
+    CTRY(cudaFuncSetAttribute(k_lindblad_forward<true, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
+    CTRY(cudaFuncSetAttribute(k_lindblad_backward<true, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
+    CTRY(cudaFuncSetAttribute(k_lindblad_forward<false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
+    CTRY(cudaFuncSetAttribute(k_lindblad_backward<false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
+    CTRY(cudaFuncSetAttribute(k_lindblad_forward<true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
+    CTRY(cudaFuncSetAttribute(k_lindblad_backward<true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
 #undef CTRY
     *out = p;
     return 0;
@@ -1031,14 +1087,35 @@ int qocb_lindblad_set_densities(qocb_lplan *p, const double *rho0) {
     if (!p || !rho0) return lfail(p, "null argument", -1);
     LTRY(p, cudaSetDevice(p->pb.device));
     const size_t DE = (size_t)p->pb.density_count * p->pb.hilbert_size * p->pb.hilbert_size;
-    LTRY(p, cudaMemcpy(p->rho0.p, rho0, sizeof(double2) * DE, cudaMemcpyHostToDevice));
+    const double2 *r = reinterpret_cast<const double2 *>(rho0);
+    p->h_rho0.assign(r, r + DE);
+    if (p->mdata || !p->h_member_rho0.empty()) {                            // the tables are rebuilt before the next launch
+        p->h_member_rho0.clear();
+        p->costs_dirty = true;
+    } else {
+        LTRY(p, cudaMemcpy(p->rho0.p, rho0, sizeof(double2) * DE, cudaMemcpyHostToDevice));
+    }
     p->rho_set = true;
     p->tape_ok = false;
     return 0;
 }
 
+/* rho0: [E][D][n][n], every member's own initial densities */
+int qocb_lindblad_set_member_densities(qocb_lplan *p, const double *rho0) {
+    if (!p || !rho0) return lfail(p, "null argument", -1);
+    if (p->batch) return lfail(p, "qocb_lindblad_set_member_densities does not apply to a control batch", -1);
+    const size_t count = (size_t)p->E * p->pb.density_count * p->pb.hilbert_size * p->pb.hilbert_size;
+    const double2 *r = reinterpret_cast<const double2 *>(rho0);
+    p->h_member_rho0.assign(r, r + count);
+    p->rho_set = true;
+    p->costs_dirty = true;
+    p->tape_ok = false;
+    return 0;
+}
+
 /* mats: [D][fmax][n][n] complex; counts: [D] or NULL; kind: QOCB_LCOST_*; weight = cost_multiplier / normalisation */
-int qocb_lindblad_add_cost(qocb_lplan *p, int32_t kind, int32_t step_cost, double weight, const double *mats, const int32_t *counts, int32_t fmax) {
+static int add_lindblad_term(qocb_lplan *p, int32_t kind, int32_t step_cost, double weight, const double *mats, const int32_t *counts,
+                             int32_t fmax, int members) {
     if (!p || !mats) return lfail(p, "null argument", -1);
     if (kind < 0 || kind > 1 || fmax < 1) return lfail(p, "bad cost kind or fmax", -1);
     const int n = p->pb.hilbert_size, nn = n * n, D = p->pb.density_count;
@@ -1051,11 +1128,23 @@ int qocb_lindblad_add_cost(qocb_lplan *p, int32_t kind, int32_t step_cost, doubl
         p->h_counts.push_back(F);
     }
     const double2 *m = reinterpret_cast<const double2 *>(mats);
-    p->h_mats.insert(p->h_mats.end(), m, m + (size_t)D * fmax * nn);
+    p->h_mats.insert(p->h_mats.end(), m, m + (size_t)members * D * fmax * nn);
     p->h_terms.push_back(t);
+    p->h_term_members.push_back(members);
     p->costs_dirty = true;
     p->tape_ok = false;
     return 0;
+}
+
+int qocb_lindblad_add_cost(qocb_lplan *p, int32_t kind, int32_t step_cost, double weight, const double *mats, const int32_t *counts, int32_t fmax) {
+    return add_lindblad_term(p, kind, step_cost, weight, mats, counts, fmax, 1);
+}
+
+/* mats: [E][D][fmax][n][n], member e's matrices; counts: [D] or NULL, shared */
+int qocb_lindblad_add_member_cost(qocb_lplan *p, int32_t kind, int32_t step_cost, double weight, const double *mats,
+                                  const int32_t *counts, int32_t fmax) {
+    if (p && p->batch) return lfail(p, "qocb_lindblad_add_member_cost does not apply to a control batch", -1);
+    return add_lindblad_term(p, kind, step_cost, weight, mats, counts, fmax, p ? p->E : 1);
 }
 
 int qocb_lindblad_cost(qocb_lplan *p, const double *controls, double *cost, double *final_densities) {
@@ -1113,6 +1202,7 @@ int qocb_lindblad_backward(qocb_lplan *p, const double *seeds, double *grad) {
 int qocb_lindblad_set_control_batch(qocb_lplan *p) {
     if (!p) return -1;
     if (p->ops_set) return lfail(p, "qocb_lindblad_set_control_batch must come before qocb_lindblad_set_operators", -1);
+    if (has_member_data(p)) return lfail(p, "the starts of a control batch share their initial densities and cost terms", -1);
     if (!p->pb.have_hamiltonian || p->pb.control_count == 0)
         return lfail(p, "a control batch needs controls (have_hamiltonian = 1 and control_count > 0)", -1);
     LTRY(p, cudaSetDevice(p->pb.device));

@@ -43,6 +43,10 @@ struct SweepArgs {
     double *part;                  // [nchunks][S][2][NP]
     double *cost_part;             // [nchunks]
     const double *psi_in;          // [S][2][NP] state entering the first local slice (psi0 unless time-sharded)
+    int psi_mstride;               // member stride of psi_in in doubles: S*2*NP after qocb_set_member_states, else 0 (shared)
+    long long vecs_mstride;        // member stride of vecs in doubles when some term has member vectors (the table then holds
+                                   // every member's copy of every term, qocb_add_member_cost), else 0: the kernels that
+                                   // evaluate costs offset `vecs` once by e * vecs_mstride
     const double *lam_in;          // [S][2][NP] costate entering the last local state from later shards, or nullptr
     double *b_out;                 // [S][2][NP] k_boundary_bwd also writes the costate at the first local state here
     int j_off, Nglob;              // time sharding: global index of local slice 0; global system_eval_count.
@@ -384,9 +388,10 @@ __global__ void __launch_bounds__(kSwThreads) k_boundary_fwd(SweepArgs a) {
     const int c0 = a.member_chunk0[e], c1 = a.member_chunk0[e + 1];
     MatRegs<NP> cur = {}, nxt = {};
     load_mat_regs<NP, false>(cur, a.chunkP + (size_t)c0 * 2 * NP * NP, S);
-    for (int i = threadIdx.x; i < VS; i += kSwThreads) sm.v0[i] = a.psi_in[off + i];
+    const double *psi_in = a.psi_in + (size_t)e * a.psi_mstride + off;
+    for (int i = threadIdx.x; i < VS; i += kSwThreads) sm.v0[i] = psi_in[i];
     double *psi_e = a.psi + (size_t)e * a.N * VSA + off;
-    for (int i = threadIdx.x; i < VS; i += kSwThreads) psi_e[i] = a.psi_in[off + i];
+    for (int i = threadIdx.x; i < VS; i += kSwThreads) psi_e[i] = psi_in[i];
     BPROF_DECL
     for (int c = c0; c < c1; ++c) {
         const double *gn = c + 1 < c1 ? a.chunkP + (size_t)(c + 1) * 2 * NP * NP : nullptr;   // prefetched inside the mat-vec
@@ -417,6 +422,7 @@ __global__ void __launch_bounds__(kSwThreads) k_sweep_fwd(SweepArgs a) {
     const int wb = a.chunk_begin[c], we = a.chunk_begin[c + 1];
     const int e = wb / (a.N - 1), jb = wb - e * (a.N - 1), je = we - e * (a.N - 1);
     const double *gU = a.U + (size_t)(e * (a.N - 1)) * 2 * NP * NP;
+    a.vecs += (size_t)e * a.vecs_mstride;                            // member e's cost vectors (0: shared)
     double *psi_e = a.psi + (size_t)e * a.N * VS;
     MatRegs<NP> cur = {}, nxt = {};
     load_mat_regs<NP, false>(cur, gU + (size_t)jb * 2 * NP * NP, S);
@@ -456,6 +462,7 @@ __global__ void __launch_bounds__(kSwThreads) k_sweep_bwd(SweepArgs a) {
     const int wb = a.chunk_begin[c], we = a.chunk_begin[c + 1];
     const int e = wb / (a.N - 1), jb = wb - e * (a.N - 1), je = we - e * (a.N - 1);
     const double *gU = a.U + (size_t)(e * (a.N - 1)) * 2 * NP * NP;
+    a.vecs += (size_t)e * a.vecs_mstride;
     const double *psi_e = a.psi + (size_t)e * a.N * VS;
     double *lam_e = a.lam + (size_t)e * a.N * VS;
     const int jstop = PARTICULAR ? jb : jb + 1;
@@ -493,6 +500,7 @@ __global__ void __launch_bounds__(kSwThreads) k_boundary_bwd(SweepArgs a, int ha
     SweepSmem<NP> sm(sm_raw, S);
     const int e = blockIdx.x;
     const int c0 = a.member_chunk0[e], c1 = a.member_chunk0[e + 1];
+    a.vecs += (size_t)e * a.vecs_mstride;
     const double *psi_e = a.psi + (size_t)e * a.N * VSA;
     double *lam_e = a.lam + (size_t)e * a.N * VSA + off;
     MatRegs<NP> cur = {}, nxt = {};
